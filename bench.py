@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- candidate-window scoring throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one pass of the whole post-MSER detection chain (K1 expand/filter, K2 crop+resize, K5 histogram + fold
@@ -364,6 +364,22 @@ def real_mser_run(torch, tsd_b200, dev, ctx_det, stream_det):
             "config": "3 real GTSDB test frames + the boxes cv2.MSER(7,200,2000,0.15) gives for them, tiled to 1024 frames"}
 
 
+def dump_outputs(out_dir, det, counts):
+    """--dump-outputs: what a caller of the timed path receives for its last step (Context.fetch_detections), as float64 .npy files,
+    so that two builds can be compared output for output on the same seeded inputs.  detections.npy [n,7] = frame, x1, y1, x2, y2,
+    id, hundredths in record order; stage_counts.npy [4] = raw, aspect-passing, survivors, detections.  Records beyond 60 MB are
+    cut to a fixed seeded sample (kept in record order), so a dump stays under 64 MB.  With --gpus N > 1 only rank 0 calls this, so
+    the dump holds rank 0's records (its own frames), not the other ranks'."""
+    os.makedirs(out_dir, exist_ok=True)
+    cols = ("frame", "x1", "y1", "x2", "y2", "id", "hundredths")
+    rec = np.stack([det[c] for c in cols], 1).astype(np.float64)
+    cap = (60 << 20) // (8 * len(cols))
+    if len(rec) > cap:
+        rec = rec[np.sort(np.random.default_rng(0).choice(len(rec), cap, replace=False))]
+    np.save(os.path.join(out_dir, "detections.npy"), rec)
+    np.save(os.path.join(out_dir, "stage_counts.npy"), counts.astype(np.float64))
+
+
 def bind_to_gpu_numa_node(local_rank):
     """Pin this process (and so the first-touch placement of its page-locked host frames) to the CPUs of the NUMA node
     the GPU hangs off: the e2e leg reads host memory from the GPU, a remote node costs PCIe/UPI bandwidth.  Best effort."""
@@ -457,6 +473,8 @@ def run_b200(args, rank, world, local_rank):
     n_timed = len(sampler.samples)
     ms = ev0.elapsed_time(ev1)
     launches = ctx.launch_count - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *ctx.fetch_detections(nb))
     ctx.set_profiling(True)                                  # second pass: same K steps, serialised, per-stage CUDA events
     evp0, evp1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     evp0.record(stream)
@@ -601,7 +619,7 @@ def run_b200(args, rank, world, local_rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--frames", type=int, default=4096, help="resident frames per GPU per step")
@@ -612,7 +630,13 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary (recognition chain, real-MSER frames) measurements")
     ap.add_argument("--no-sweep", action="store_true", help="skip the 4K candidate sweep (BASELINE configs[4]) of the secondary measurements")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer leg (used for the ncu launch list of the device-resident step)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the detection records and stage counts of the last timed step (rank 0) "
+                                                         "to DIR/*.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
         return run_reference(args, rank, world)

@@ -1,9 +1,9 @@
 """Generate the golden vectors under tests/golden/ by RUNNING THE UNMODIFIED REFERENCE.
 
-Only runnable where /root/reference exists (the build container).  The GPU box never runs this; it
-consumes the committed fixtures.  Usage:
+Only runnable with TSD_REFERENCE_ROOT set to a checkout of the reference (tests/golden/refload.py).  The
+tests never run this; they consume the committed fixtures.  Usage:
 
-    python tests/golden/make_golden.py det      # detection goldens (about 1 min)
+    TSD_REFERENCE_ROOT=<reference checkout> python tests/golden/make_golden.py det      # detection goldens (about 1 min)
     python tests/golden/make_golden.py rec      # recognition goldens (needs MSERTrain.val: about 7 min first time)
     python tests/golden/make_golden.py crops    # inputs of calculateMeanMasks (class crops, reference order)
     python tests/golden/make_golden.py full     # full-dataset KAT: all 150 frames + 24 frames as JPEG bytes (about 1 min)

@@ -1,4 +1,5 @@
-"""Loader for the UNMODIFIED reference modules (only usable where /root/reference exists).
+"""Loader for the UNMODIFIED reference modules (only usable with TSD_REFERENCE_ROOT set to a checkout of
+cfkr-dev/OpenCV-Traffic-Sign-Detector, which is not part of this repository).
 
 Test infrastructure: used by tests/golden/make_golden.py to generate golden vectors and by the
 optional `-m "not gpu"` tests that re-validate the oracle against the live reference when the
@@ -14,13 +15,13 @@ import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("TSD_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("TSD_REFERENCE_ROOT", "")
 DET_DIR = os.path.join(REF_ROOT, "Deteción de Objetos")
 REC_DIR = os.path.join(REF_ROOT, "Reconocimiento de Objetos")
 
 
 def reference_available():
-    return os.path.isfile(os.path.join(DET_DIR, "source.py")) and os.path.isfile(os.path.join(REC_DIR, "source.py"))
+    return bool(REF_ROOT) and os.path.isfile(os.path.join(DET_DIR, "source.py")) and os.path.isfile(os.path.join(REC_DIR, "source.py"))
 
 
 def _stub_matplotlib():

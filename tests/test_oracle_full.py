@@ -9,6 +9,11 @@ import pytest
 
 from conftest import STORED
 
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+import refload  # noqa: E402
+
+needs_reference = pytest.mark.skipif(not refload.reference_available(), reason="needs the reference's source tree (TSD_REFERENCE_ROOT)")
+
 
 def _lines(files, records):
     """resultado.txt lines (DET/source.py:501-508): file;x1;y1;x2;y2;type;score with str() of the 2-decimal score."""
@@ -77,14 +82,12 @@ def test_ref_port_all_stored_frames(det_full150, jpeg24, templates, resultado150
         assert [d[1:5] for d in dets] == [tuple(c) for c in det_frames[k + "_det_coords"].tolist()]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree not present (GPU box)")
+@needs_reference
 def test_ref_port_vs_live_reference_synthetic(templates, tsd):
-    """Where /root/reference exists: ref_port against the unmodified reference functions on 6 synthetic bench frames
-    (1360x800, 200 candidates: the workload both bench arms time) -- same survivors, same detection tuples -- and its cost
+    """Where the reference's source tree is available: ref_port against the unmodified reference functions on 6 synthetic bench
+    frames (1360x800, 200 candidates: the workload both bench arms time) -- same survivors, same detection tuples -- and its cost
     stays within a factor 1.5 of the reference's (it must cost what the reference costs to be a fair baseline)."""
     import time
-    sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-    import refload
     import cv2
     from oracle import ref_port
     src, _ = refload.load_det()
@@ -129,15 +132,28 @@ def test_gray_descriptor_classifiers_oracle(oracle, rec_golden, rec_gray_golden)
     assert np.max(np.abs(Z - g["knn_Zq"][:300]) / np.maximum(1.0, np.abs(g["knn_Zq"][:300]))) < 1e-9 and np.array_equal(lk, g["pred_knn"][:300])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree not present (GPU box)")
+def test_install_rebinds_exactly_the_patched_names(tsd, monkeypatch):
+    """install() on stand-in modules: every name in _PATCHED is rebound to the mirror's own function and every other attribute is
+    left as it was.  (That the reference's modules define and call those names is checked where the reference tree is available.)"""
+    import types
+    monkeypatch.setattr(tsd.source_det, "_installed_into", None)          # install() records its target; restored afterwards
+    for mirror in (tsd.source_det, tsd.source_rec):
+        mod = types.ModuleType("stand_in_source")
+        before = {name: object() for name in mirror._PATCHED + ("test", "testValidation", "constants", "tqdm")}
+        vars(mod).update(before)
+        assert mirror.install(mod) is mod
+        for name, obj in before.items():
+            assert getattr(mod, name) is (getattr(mirror, name) if name in mirror._PATCHED else obj), name
+        assert set(vars(mod)) == set(before) | set(vars(types.ModuleType("x")))
+
+
+@needs_reference
 def test_install_rebinds_the_reference_modules_call_compatibly():
     """The drop-in boundary on the live reference modules (no GPU needed: nothing is called): every name source_det / source_rec
     patch exists in the reference's own `source` module with the same positional parameters, is really looked up through the module's
     globals by the reference's code (so rebinding it reroutes the reference's own drivers and helpers), and install() rebinds
     exactly those names and nothing else."""
     import inspect
-    sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-    import refload
     import tsd_b200
     for load, mirror in ((refload.load_det, tsd_b200.source_det), (refload.load_rec, tsd_b200.source_rec)):
         ref, _ = load()
@@ -165,16 +181,13 @@ def test_install_rebinds_the_reference_modules_call_compatibly():
             setattr(ref, name, obj)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree not present (GPU box)")
+@needs_reference
 def test_reference_driver_through_install(tmp_path, monkeypatch, resultado150):
-    """The reference's OWN driver `test()` (DET/source.py:611-853) run through source_det.install(), on the 150 test frames, in the
-    container where the reference tree exists -- which has no GPU, so the engine behind the mirrors is a test double answered by
-    the CPU oracle (tests/oracle_context.py).  What this pins is everything between the driver and the engine: the patched
+    """The reference's OWN driver `test()` (DET/source.py:611-853) run through source_det.install(), on the 150 test frames, without
+    a GPU: the engine behind the mirrors is a test double answered by the CPU oracle (tests/oracle_context.py).  What this pins is everything between the driver and the engine: the patched
     names, their argument / return conventions as the driver uses them (Python-int tuples, float scores, [(mask, name)] lists,
     (detections, counts, images) triples), the directory walks.  resultado.txt must equal the reference's own, line for line."""
-    sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
     sys.path.insert(0, os.path.dirname(__file__))
-    import refload
     import tsd_b200
     from oracle_context import OracleContext
     src, _ = refload.load_det()
@@ -200,7 +213,7 @@ def test_reference_driver_through_install(tmp_path, monkeypatch, resultado150):
     assert len(os.listdir(tmp_path / "resultado_imgs")) == 150
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree not present (GPU box)")
+@needs_reference
 @pytest.mark.parametrize("descriptor,classifier", [("HOG", "LDABAYES"), ("HOG", "KNN"), ("GRAY", "LDABAYES"), ("GRAY", "KNN")])
 def test_reference_recognition_driver_through_install(tmp_path, monkeypatch, descriptor, classifier):
     """The reference's own `testValidation()` (REC/source.py:646-809) on a reduced training directory (8 real train frames that
@@ -213,9 +226,7 @@ def test_reference_recognition_driver_through_install(tmp_path, monkeypatch, des
     of REC/constants.py:10-12 (HOG / GRAY descriptor x LDA-Bayes / KNN)."""
     import pickle
     import random
-    sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
     sys.path.insert(0, os.path.dirname(__file__))
-    import refload
     import tsd_b200
     from oracle_context import OracleContext
     src, _ = refload.load_rec()
