@@ -208,7 +208,8 @@ def test_k5_dedup_adversarial(ctx_det, oracle):
 def test_k5_dedup_flat_windows_32(ctx_rec, oracle):
     """32 x 32 windows (1024 pixels: bin counts up to 1024) with a few flat or two-tone windows per frame: the tensor-core pair
     kernel keeps counts modulo 256 and corrects the pairs of such windows exactly -- also when BOTH windows of a pair exceed 255 in
-    the same bin -- for 2 .. 128 windows per frame; frames with more than 16 such windows, or more than 128 windows, go to k5_pairs."""
+    the same bin -- for 2 .. 128 windows per frame; frames with more than 16 such windows go to k5_pairs, frames of more than 128
+    windows to k5_gram_big (the same correction per pair of 128-row blocks)."""
     rng = np.random.default_rng(33)
     tones = rng.integers(0, 256, (5, 3), dtype=np.uint8)
     wins, coords, off = [], [], [0]
