@@ -105,11 +105,13 @@ TSD_API int tsd_set_templates(tsd_ctx *ctx, const uint8_t *red6, const uint8_t *
  * (DET/source.py:459-462).  By default the library fills it with libm pow(); the Python wrapper passes the
  * values numpy computes so that the in-process reference and the GPU path use bit-identical f. */
 TSD_API int tsd_set_similarity_table(tsd_ctx *ctx, const double *f, int n);
-/* Six binary LDA classifiers: W f64 [324][6] (column c = classifiers[c].coef_[0]), b f64 [6] (intercept_),
- * REC/source.py:551-562 fit on the host with scikit-learn. */
+/* Six binary LDA classifiers: W f64 [nfeat][6] (column c = classifiers[c].coef_[0]), b f64 [6] (intercept_),
+ * REC/source.py:551-562 fit on the host with scikit-learn.  nfeat = 1..4096 (324 for HOG, 1024 for raw grey pixels; the
+ * chain needs 324).  K8 keeps W in shared memory, nfeat * 48 B: 192 KB at 4096 features; TSD_E_INVALID if the device
+ * cannot give a block that much. */
 TSD_API int tsd_set_lda(tsd_ctx *ctx, const double *W, const double *b, int nfeat);
 /* 7-class LDA reducer + KNN training set: xbar f64 [nfeat], scalings f64 [nfeat][6], Ztrain f64 [ntrain][6],
- * ytrain int32 [ntrain] (REC/source.py:586-589). */
+ * ytrain int32 [ntrain] (REC/source.py:586-589).  k = 1..8, labels 0..15 (TSD_E_INVALID otherwise). */
 TSD_API int tsd_set_knn(tsd_ctx *ctx, const double *xbar, const double *scalings, int nfeat, const double *Ztrain,
                         const int32_t *ytrain, int ntrain, int k);
 
@@ -202,10 +204,15 @@ TSD_API int tsd_recognize(tsd_ctx *ctx, const uint8_t *windows, int n, double to
 
 /* EVALUATION ONLY (BASELINE.json north_star: the LDA projection on tensor cores vs FMA): the same decision from mma.sync TF32 logits,
  * split = 1 (plain TF32) or 3 (3xTF32 with FP32 accumulation).  logits float32 [n][6] (may be NULL), *ms (may be NULL) = device time of
- * the kernel alone.  The chain and tsd_lda_predict use the f64 FMA kernel (the reference computes in float64).  Host pointers. */
+ * the kernel alone.  The chain and tsd_lda_predict use the f64 FMA kernel (the reference computes in float64).  Host pointers.
+ * The kernel keeps W as TF32 tiles in shared memory, 64 B per feature rounded up to 8 features: TSD_E_INVALID when they do not fit
+ * in one block (above 3 632 features on the B200). */
 TSD_API int tsd_lda_predict_tf32(tsd_ctx *ctx, const float *X, int n, double tol, int split, float *logits, int32_t *labels, float *ms, int mem);
 
-/* K8b predictProbabilityKNNClassifiers (REC/source.py:592-596): Z f64 [n][6] (may be NULL), labels int32 [n]. */
+/* K8b predictProbabilityKNNClassifiers (REC/source.py:592-596): Z f64 [n][6] (may be NULL), labels int32 [n].
+ * Brute force over the training set; training rows at equal distance are ranked by index (the smaller one is nearer), then a
+ * uniform vote with ties to the smallest label.  scikit-learn's kd-tree orders exact distance ties its own way, so labels can
+ * differ from it when a tie straddles the k-th neighbour (SURVEY A.8). */
 TSD_API int tsd_knn_predict(tsd_ctx *ctx, const float *X, int n, double *Z, int32_t *labels, int mem);
 
 /* ---- whole path -------------------------------------------------------------------------------------------- */

@@ -142,6 +142,20 @@ static int check_launch(tsd_ctx* c, const char* what) {
     return TSD_OK;
 }
 
+// Lets kernel fn launch with `bytes` of dynamic shared memory: fails with TSD_E_INVALID when the device's per-block opt-in limit
+// is smaller (227 KB on the B200), else raises the function's limit.  Never lowers it: the attribute belongs to the device, and
+// another context on it may need a larger value.
+static int allow_dynamic_smem(tsd_ctx* c, const void* fn, size_t bytes, const char* what) {
+    int optin = 0;
+    CU(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device));
+    cudaFuncAttributes fa;
+    CU(cudaFuncGetAttributes(&fa, fn));
+    if (bytes + fa.sharedSizeBytes > (size_t)optin)
+        return fail(TSD_E_INVALID, "%s needs %zu B of shared memory per block, the device allows %d B", what, bytes + fa.sharedSizeBytes, optin);
+    if (bytes > (size_t)fa.maxDynamicSharedSizeBytes) CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    return TSD_OK;
+}
+
 // Event record / wait on c->cur that also works while the stream is being captured into a CUDA graph (external event nodes).
 static int ev_record(tsd_ctx* c, cudaEvent_t ev) {
     cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
@@ -501,6 +515,8 @@ int tsd_set_similarity_table(tsd_ctx* c, const double* f, int n) {
 int tsd_set_lda(tsd_ctx* c, const double* W, const double* b, int nfeat) {
     if (!c || !W || !b || nfeat < 1 || nfeat > 4096) return fail(TSD_E_INVALID, "bad argument");
     CU(cudaSetDevice(c->device));
+    // k8_lda_kernel stages W in dynamic shared memory: nfeat * 48 B, 192 KB at 4096 features (above 48 KB it needs the opt-in)
+    TRY(allow_dynamic_smem(c, (const void*)k8_lda_kernel, (size_t)nfeat * 6 * sizeof(double), "k8_lda"));
     TRY(join_pending(c));
     CU(cudaStreamSynchronize(c->stream));
     if (c->d_ldaW) cudaFree(c->d_ldaW);
@@ -518,6 +534,9 @@ int tsd_set_knn(tsd_ctx* c, const double* xbar, const double* scalings, int nfea
                 int ntrain, int k) {
     if (!c || !xbar || !scalings || !Ztrain || !ytrain || nfeat < 1 || ntrain < 1 || k < 1 || k > kKnnMaxK)
         return fail(TSD_E_INVALID, "bad argument (k must be 1..%d)", kKnnMaxK);
+    for (int t = 0; t < ntrain; t++)                         // k8_knn_kernel votes into 16 label counters
+        if (ytrain[t] < 0 || ytrain[t] >= kKnnMaxLabels)
+            return fail(TSD_E_INVALID, "ytrain[%d] = %d, labels must be 0..%d", t, ytrain[t], kKnnMaxLabels - 1);
     CU(cudaSetDevice(c->device));
     TRY(join_pending(c));
     CU(cudaStreamSynchronize(c->stream));
@@ -1251,14 +1270,16 @@ int tsd_lda_predict_tf32(tsd_ctx* c, const float* X, int n, double tol, int spli
     if (mem != TSD_MEM_HOST) return fail(TSD_E_INVALID, "host pointers only");
     if (!c->d_ldaW) return fail(TSD_E_STATE, "LDA weights not set (tsd_set_lda)");
     CU(cudaSetDevice(c->device));
+    // the hi and lo TF32 tiles of W, [2][kpad][8] floats = 64 B per padded feature: up to 3 632 features on the B200
+    const int kpad = (c->lda_nfeat + 7) & ~7;
+    const size_t smem = (size_t)2 * kpad * 8 * sizeof(float);
+    TRY(allow_dynamic_smem(c, split == 1 ? (const void*)k8_lda_tf32_kernel<1> : (const void*)k8_lda_tf32_kernel<3>, smem, "k8_lda_tf32"));
     if (n == 0) return TSD_OK;
     Stage s(c);
     void *dx, *dl, *dy;
     TRY(s.in(X, (size_t)n * c->lda_nfeat * 4, &dx));
     TRY(s.alloc(&dl, (size_t)n * 6 * 4));
     TRY(s.alloc(&dy, (size_t)n * 4));
-    const int kpad = (c->lda_nfeat + 7) & ~7;
-    const size_t smem = (size_t)2 * kpad * 8 * sizeof(float);
     int grid = cdiv(cdiv(n, 16), 4);
     if (grid > c->sm_count * 8) grid = c->sm_count * 8;
     cudaEvent_t e0, e1;

@@ -1579,6 +1579,7 @@ __global__ void __launch_bounds__(128) k8_lda_tf32_kernel(const float* __restric
 // K8b  reducer.transform + KNeighborsClassifier(k).predict  (REC:592-596).  One warp per query: Z = (x - xbar) S in
 // f64, then every lane keeps its k best of the training rows it visits; the warp merges by (distance, index).
 constexpr int kKnnMaxK = 8;
+constexpr int kKnnMaxLabels = 16;                   // training labels 0..15 (tsd_set_knn checks)
 __global__ void __launch_bounds__(128) k8_knn_kernel(const float* __restrict__ X, int n, int nfeat, const double* __restrict__ xbar,
                                                      const double* __restrict__ S, const double* __restrict__ Zt,
                                                      const int32_t* __restrict__ yt, int ntrain, int k,
@@ -1610,9 +1611,9 @@ __global__ void __launch_bounds__(128) k8_knn_kernel(const float* __restrict__ X
         }
     }
     // k rounds of warp arg-min over the lanes' current heads
-    int votes[16];
+    int votes[kKnnMaxLabels];
 #pragma unroll
-    for (int j = 0; j < 16; j++) votes[j] = 0;
+    for (int j = 0; j < kKnnMaxLabels; j++) votes[j] = 0;
     int head = 0;
     for (int r = 0; r < k; r++) {
         double d = head < k ? bd[head] : INFINITY; int idx = head < k ? bi[head] : 0x7fffffff;
@@ -1623,11 +1624,11 @@ __global__ void __launch_bounds__(128) k8_knn_kernel(const float* __restrict__ X
             if (od < bdv || (od == bdv && oi < bidx)) { bdv = od; bidx = oi; }
         }
         if (idx == bidx && d == bdv) head++;
-        if (bidx != 0x7fffffff) { int y = yt[bidx]; if (y >= 0 && y < 16) votes[y]++; }
+        if (bidx != 0x7fffffff) { int y = yt[bidx]; if (y >= 0 && y < kKnnMaxLabels) votes[y]++; }
     }
     if (lane == 0) {
         int lab = 0, bv = -1;
-        for (int y = 0; y < 16; y++) if (votes[y] > bv) { bv = votes[y]; lab = y; }   // ties -> smallest label
+        for (int y = 0; y < kKnnMaxLabels; y++) if (votes[y] > bv) { bv = votes[y]; lab = y; }   // ties -> smallest label
         labels[w] = lab;
     }
 }
