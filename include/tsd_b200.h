@@ -90,7 +90,9 @@ TSD_API int tsd_flush(tsd_ctx *ctx);
  * frames IN PLACE over PCIe (only the 32-byte sectors the candidate ROIs touch are transferred, each once per batch, into a
  * device-resident mirror of the frames; batches of 512 frames or more run as up to four chunks whose transfers overlap the
  * previous chunk's kernels, TSD_STAGE_CHUNK=0 turns the chunking off); pageable frames are copied whole, in chunks that overlap
- * the kernels.  Buffers from cudaHostAlloc / torch pin_memory() are already page-locked. */
+ * the kernels.  Buffers from cudaHostAlloc / torch pin_memory() are already page-locked.
+ * Staging needs a 16-byte aligned frames pointer, row_stride and frame_stride multiples of 16 and 3 * W a multiple of 16; any other
+ * page-locked layout is read by K2 itself, tap by tap over PCIe (as with TSD_STAGE=0).  Either way the records are the same. */
 TSD_API int tsd_host_register(void *p, int64_t bytes);
 TSD_API int tsd_host_unregister(void *p);
 /* Number of kernels this library launched on the context since creation (bench.py's gpu_launches). */

@@ -1013,12 +1013,18 @@ int tsd_preprocess(tsd_ctx* c, const uint8_t* frames, int nframes, int H, int W,
         CU(cudaMemcpyAsync(c->b_pin.p, frames, in_bytes, cudaMemcpyHostToDevice, c->stream));
         d_in = (const uint8_t*)c->b_pin.p; d_out = (uint8_t*)c->b_pout.p;
     }
-    pre_gray_lut_kernel<<<dim3(tiles_x * tiles_y, nframes), 256, 0, c->cur>>>(d_in, H, W, row_stride, frame_stride, tiles_x, tiles_y, tw, th, clip, lut_scale,
-                                                                               (uint8_t*)c->b_pgray.p, (uint8_t*)c->b_pluts.p);
-    TRY(check_launch(c, "pre_gray_lut"));
-    pre_clahe_blur_kernel<<<dim3(cdiv(W, kPreTW), cdiv(H, kPreTH), nframes), 256, 0, c->cur>>>((uint8_t*)c->b_pgray.p, (uint8_t*)c->b_pluts.p, H, W, tiles_x, tiles_y,
-                                                                                                  1.0f / (float)tw, 1.0f / (float)th, c->d_gamma, d_out);
-    TRY(check_launch(c, "pre_clahe_blur"));
+    // both kernels take the frame from gridDim.y / gridDim.z (at most 65 535): larger batches are launched in frame ranges
+    for (int f0 = 0; f0 < nframes; f0 += 65535) {
+        const int nf = nframes - f0 < 65535 ? nframes - f0 : 65535;
+        uint8_t* gray = (uint8_t*)c->b_pgray.p + (size_t)f0 * H * W;
+        uint8_t* luts = (uint8_t*)c->b_pluts.p + (size_t)f0 * tiles_x * tiles_y * 256;
+        pre_gray_lut_kernel<<<dim3(tiles_x * tiles_y, nf), 256, 0, c->cur>>>(d_in + (size_t)f0 * frame_stride, H, W, row_stride, frame_stride, tiles_x, tiles_y,
+                                                                         tw, th, clip, lut_scale, gray, luts);
+        TRY(check_launch(c, "pre_gray_lut"));
+        pre_clahe_blur_kernel<<<dim3(cdiv(W, kPreTW), cdiv(H, kPreTH), nf), 256, 0, c->cur>>>(gray, luts, H, W, tiles_x, tiles_y, 1.0f / (float)tw,
+                                                                                             1.0f / (float)th, c->d_gamma, d_out + (size_t)f0 * H * W);
+        TRY(check_launch(c, "pre_clahe_blur"));
+    }
     if (mem == TSD_MEM_HOST) {
         CU(cudaMemcpyAsync(out, d_out, npix, cudaMemcpyDeviceToHost, c->stream));
         CU(cudaStreamSynchronize(c->stream));

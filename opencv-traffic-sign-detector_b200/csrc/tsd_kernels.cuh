@@ -241,8 +241,11 @@ __global__ void __launch_bounds__(128) k2_crop_resize_kernel(
     const uint8_t* __restrict__ src = frames + (int64_t)win_frame[w] * frame_stride + (int64_t)cy * row_stride + (int64_t)cx * C;
     uint8_t* __restrict__ dst = windows + (int64_t)w * out_stride;
     const int rowlen = D * C, total = D * rowlen;
-    if (cw <= 0 || ch <= 0) return;
-    for (int i = total + lane; i < out_stride; i += 32) dst[i] = 0;     // pad bytes of the internal layout are zero                         // filtered out by K1 (cv2.resize would raise)
+    if (cw <= 0 || ch <= 0) {                                // empty crop (cv2.resize would raise; K1 never emits one): a defined, all-zero window
+        for (int i = lane; i < out_stride; i += 32) dst[i] = 0;
+        return;
+    }
+    for (int i = total + lane; i < out_stride; i += 32) dst[i] = 0;     // pad bytes of the internal layout are zero
     if (cw == D && ch == D) {                               // same size: copy
         for (int i = lane; i < total; i += 32) { int y = i / rowlen, r = i - y * rowlen; dst[i] = src[(int64_t)y * row_stride + r]; }
         return;
