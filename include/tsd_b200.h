@@ -46,7 +46,10 @@ extern "C" {
 
 typedef struct tsd_ctx tsd_ctx;
 
-/* All hard-coded constants of the reference path, one POD (SURVEY.md section 5 "config / flags"). */
+/* All hard-coded constants of the reference path, one POD (SURVEY.md section 5 "config / flags").  tsd_create refuses (TSD_E_INVALID)
+ * a window outside 2..32 and a coord_tol * merge_factor that is not above sqrt(f(65535)) = 0.3913: pairs whose corners are further
+ * apart than the 65 536-entry corner-similarity table reaches (255 px) take no action, which equals the reference only while their
+ * similarity, at most sqrt(f(65535)), is below the lowest similarity that acts. */
 typedef struct tsd_config {
     double enlarge;            /* 1.30 DET/source.py:119 ; 1.15 REC/source.py:54 */
     double aspect_lo;          /* 0.8  DET/source.py:164 (strict) */
@@ -105,7 +108,8 @@ TSD_API int64_t tsd_launch_count(tsd_ctx *ctx);
 TSD_API int tsd_set_templates(tsd_ctx *ctx, const uint8_t *red6, const uint8_t *blue6);
 /* Optional override of the corner-similarity table f(d2) = EuclDSimilarity at squared distance d2 = 0..n-1
  * (DET/source.py:459-462).  By default the library fills it with libm pow(); the Python wrapper passes the
- * values numpy computes so that the in-process reference and the GPU path use bit-identical f. */
+ * values numpy computes so that the in-process reference and the GPU path use bit-identical f.  TSD_E_INVALID unless
+ * sqrt(f(n-1)) < coord_tol * merge_factor (pairs beyond the table take no action). */
 TSD_API int tsd_set_similarity_table(tsd_ctx *ctx, const double *f, int n);
 /* Six binary LDA classifiers: W f64 [nfeat][6] (column c = classifiers[c].coef_[0]), b f64 [6] (intercept_),
  * REC/source.py:551-562 fit on the host with scikit-learn.  nfeat = 1..4096 (324 for HOG, 1024 for raw grey pixels; the
@@ -138,7 +142,8 @@ TSD_API int tsd_windows(tsd_ctx *ctx, const uint8_t *frames, int nframes, int H,
 
 /* K5  cleanDuplicatedDetections(list, by_coords, tol) per frame (DET/source.py:177-223; helpers :459-477,575-586).
  * In: windows/coords/offsets (CSR per frame).  Out: survivors, compacted per frame in the fold's list order.
- * *total_out receives out_offsets[nframes]. */
+ * *total_out receives out_offsets[nframes].  D = 2..32.  by_coords: TSD_E_INVALID unless tol * merge_factor (of the config) is
+ * above sqrt(f(n-1)) of the similarity table, 0.3913 for the default one. */
 TSD_API int tsd_dedup(tsd_ctx *ctx, const uint8_t *windows, const int32_t *coords, const int32_t *offsets, int nframes,
                       int D, int by_coords, double tol, uint8_t *out_windows, int32_t *out_coords, int32_t *out_offsets,
                       int32_t *total_out, int mem);
@@ -167,7 +172,8 @@ TSD_API int tsd_mean_windows(tsd_ctx *ctx, const uint8_t *windows, const int32_t
  * (DET/source.py:401-450) for all files and types at once: det / gt int32 [n][6] = (frame, x1, y1, x2, y2, type bucket 0..5), gt grouped
  * by frame (gt_offsets int32 [nframes+1]); status int32 [ndet] (1 = "correct": best same-type ground truth by
  * sqrt(f(d_TL) f(d_BR)) exceeds tol = 0.85), match int32 [ndet] (its gt row or -1), tally int32 [nframes][6][4] =
- * (correct, incorrect, not detected, expected).  Needs tsd_set_similarity_table. */
+ * (correct, incorrect, not detected, expected).  Needs tsd_set_similarity_table.  TSD_E_INVALID unless tol is above sqrt(f(n-1)) of
+ * the table (0.3913 for 65 536 entries): ground truths beyond the table are skipped. */
 TSD_API int tsd_match_detections(tsd_ctx *ctx, const int32_t *det, int ndet, const int32_t *gt, const int32_t *gt_offsets, int nframes,
                                  double tol, int32_t *status, int32_t *match, int32_t *tally);
 /* tsd_match_iou = the loop of precision_recall_curve (Reconocimiento de Objetos/evaluar_resultados.py:224-262) with bboxes_overlap

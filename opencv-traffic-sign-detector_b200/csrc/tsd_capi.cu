@@ -217,6 +217,15 @@ static double eucl_similarity_d2(long long d2) {             // DET:459-462 with
     return 1.0 / (1.0 + pow(M_E, ((0.154 * pow(d, 1.2)) - 31.8) / (0.2 * d)));
 }
 
+// Pairs whose squared corner distance is at or beyond the similarity table take no action (coord_sim, eval_match).  That equals
+// the reference only while every such pair's similarity stays below the lowest one that acts, `lo`: f is decreasing, so the table
+// must reach a distance where sqrt(f(n-1)) < lo.  (The default table reaches 255 px: sqrt(f(65535)) = 0.3913.)
+static int check_simtab(const tsd_ctx* c, double lo, const char* what) {
+    const double s = sqrt(c->h_simtab[c->simtab_n - 1]);
+    if (s >= lo) return fail(TSD_E_INVALID, "%s %.6g is not above sqrt(f(%d)) = %.6g: the corner-similarity table is too short", what, lo, c->simtab_n - 1, s);
+    return TSD_OK;
+}
+
 static int create_impl(tsd_ctx* c, int device) {
     CU(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
     CU(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
@@ -306,6 +315,7 @@ static int create_impl(tsd_ctx* c, int device) {
     CU(cudaMemcpy(c->d_simtab, f.data(), sizeof(double) * n, cudaMemcpyHostToDevice));
     c->simtab_n = n;
     c->h_simtab = f;
+    TRY(check_simtab(c, c->cfg.coord_tol * c->cfg.merge_factor, "coord_tol * merge_factor ="));
     {   // HOG Gaussian window, sigma = (16+16)/8 = 4  (OpenCV HOGCache::init)
         float sigma = 4.f, sc = 1.f / (sigma * sigma * 2);
         for (int i = 0; i < 16; i++) {
@@ -735,6 +745,7 @@ static int dev_fold(tsd_ctx* c, uint8_t* windows, int ws, int32_t* coords, uint3
     P.E_T = E_T; P.e_stride = e_stride;
     P.hist_tol = hist_tol; P.hist_lo = hist_tol * c->cfg.merge_factor;      // tolerance * 0.8823 in f64 (DET:217)
     P.coord_tol = coord_tol; P.coord_lo = coord_tol * c->cfg.merge_factor;
+    if (do_coords) TRY(check_simtab(c, P.coord_lo, "tol * merge_factor ="));
     if (nframes == 0) { if (surv_offsets) CU(cudaMemsetAsync(surv_offsets, 0, 4, c->cur)); return TSD_OK; }
     // max_n is only an upper bound (raw boxes per frame); frames with more than 1024 aspect-passing windows are flagged by
     // the warp-per-frame fold (out_count = -1) and redone by the general block-synchronous fold below
@@ -1057,6 +1068,7 @@ int tsd_match_detections(tsd_ctx* c, const int32_t* det, int ndet, const int32_t
                          int32_t* status, int32_t* match, int32_t* tally) {
     if (!c || ndet < 0 || nframes < 0 || !gt_offsets || (ndet && (!det || !status || !match)) || (nframes && !tally)) return fail(TSD_E_INVALID, "bad argument");
     if (!c->d_simtab) return fail(TSD_E_STATE, "similarity table not set (tsd_set_similarity_table)");
+    TRY(check_simtab(c, tol, "tol ="));                      // eval_match skips ground truths beyond the table
     const int ngt = gt_offsets[nframes];
     if (ngt < 0 || (ngt && !gt)) return fail(TSD_E_INVALID, "bad ground truth");
     for (int i = 0; i < ndet; i++) if (det[6 * i + 5] < 0 || det[6 * i + 5] > 5) return fail(TSD_E_INVALID, "detection %d: type bucket %d not in 0..5", i, det[6 * i + 5]);
@@ -1398,11 +1410,13 @@ static int enqueue_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, i
         uint32_t* bits = (uint32_t*)c->b_bits.p + wo * 2 * NW;
         int grid = cdiv((int64_t)cap * 32, 256);
         if (grid > c->sm_count * TSD_K3_GRID) grid = c->sm_count * TSD_K3_GRID;
-        // inside the chain only the bit-packed masks are consumed (K4); the byte masks (the bit-exact artefact tsd_color_masks returns)
-        // are written only when TSD_KEEP_MASKS=1 asks for them
+        // K4 reads the bit-packed masks at NW = 20 / 32 words (D = 25, 29..32) and the byte masks at every other D.  K3 v3 writes the
+        // byte masks only when K4 reads them or TSD_KEEP_MASKS=1 asks for them (the generic kernel always writes both)
+        const bool k4_bits = NW == 20 || NW == 32;
+        const bool want_bytes = c->keep_masks || !k4_bits;
         if (ws <= 4 * 32 * 16)
-            k3_masks_v3_kernel<4><<<grid, 256, 0, c->cur>>>(windows, slots, d_nsurv, nb, npx, ws, c->d_tab, c->d_mlut, c->keep_masks ? red : nullptr,
-                                                            c->keep_masks ? blue : nullptr, ms, bits);
+            k3_masks_v3_kernel<4><<<grid, 256, 0, c->cur>>>(windows, slots, d_nsurv, nb, npx, ws, c->d_tab, c->d_mlut, want_bytes ? red : nullptr,
+                                                            want_bytes ? blue : nullptr, ms, bits);
         else
             k3_masks_generic_kernel<<<grid, 256, 0, c->cur>>>(windows, slots, d_nsurv, nb, npx, ws, c->d_tab, bounds_of(c->cfg), red, blue, ms, bits);
         TRY(check_launch(c, "k3_masks"));

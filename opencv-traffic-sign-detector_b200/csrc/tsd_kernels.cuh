@@ -979,7 +979,9 @@ __device__ __forceinline__ double coord_sim(int4 a, int4 b, const double* __rest
     const int dx = a.x - b.x, dy = a.y - b.y, ex = a.z - b.z, ey = a.w - b.w;
     if (max(max(abs(dx), abs(dy)), max(abs(ex), abs(ey))) > 32767) return 0.0;
     const int d1 = dx * dx + dy * dy, d2 = ex * ex + ey * ey;
-    if (d1 >= simtab_n || d2 >= simtab_n) return 0.0;      // f < 0.16 beyond the table: sqrt(f1 f2) < 0.4 < tol*0.8823
+    // beyond the table f(d) <= f(simtab_n - 1), and the host refuses a tolerance unless sqrt(f(simtab_n - 1)) < tol * merge_factor
+    // (check_simtab): such a pair takes no action, as in the reference
+    if (d1 >= simtab_n || d2 >= simtab_n) return 0.0;
     return __dsqrt_rn(__dmul_rn(simtab[d1], simtab[d2]));
 }
 
@@ -1690,8 +1692,8 @@ __global__ void label_emit_kernel(const int32_t* __restrict__ lab, const int32_t
 // N4  the evaluators' matching loops (reporting only).
 // eval_match: checkIfDetectionByTypeOnFileIsCorrectIncorrectDuplicated (DET:425-450) for every detection at once -- best ground
 // truth of the same frame and type bucket by sqrt(f(d_TL) f(d_BR)) (first strict maximum), "correct" when it exceeds tol.  A
-// ground truth beyond the similarity table (a corner further than 255 px: f < 0.16, similarity < 0.4) can never be the match of a
-// correct detection and is skipped.  eval_tally_*: the per (frame, type) counts of getCorrectsAndWrongByTypeOnFile (DET:401-422).
+// ground truth beyond the similarity table (similarity below sqrt(f(simtab_n - 1)), which the host requires to be below tol) can
+// never be the match of a correct detection and is skipped.  eval_tally_*: the per (frame, type) counts of getCorrectsAndWrongByTypeOnFile (DET:401-422).
 // =====================================================================================================
 struct EvalBox { int32_t frame, x1, y1, x2, y2, type; };     // type = bucket 0..5 (DET:371-386: anything that is not 1..5 lands in the sixth)
 

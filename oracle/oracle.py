@@ -39,18 +39,18 @@ def lib():
     if _lib is None:
         build()
         L = C.CDLL(_SO)
-        L.orc_expand_box.argtypes = [C.c_int32] * 4 + [C.c_double, _i32p]
+        L.orc_expand_box.argtypes = [C.c_int32] * 4 + [C.c_double, C.c_double, C.c_double, _i32p]
         L.orc_expand_box.restype = C.c_int
         L.orc_resize_linear_u8.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, _u8p, C.c_int]
         L.orc_resize_linear_u8.restype = None
         L.orc_crop_resize.argtypes = [_u8p, C.c_int, C.c_int, C.c_int, _i32p, _u8p, C.c_int]
         L.orc_crop_resize.restype = C.c_int
         L.orc_bgr2hsv.argtypes = [_u8p, C.c_int, _u8p]
-        L.orc_color_masks.argtypes = [_u8p, C.c_int, _u8p, _u8p]
+        L.orc_color_masks.argtypes = [_u8p, C.c_int, _u8p, _u8p, _u8p, _u8p]
         L.orc_score_hundredths.argtypes = [_u8p, _u8p, C.c_int, _i32p]
         L.orc_score_hundredths.restype = C.c_int
         L.orc_best_template.argtypes = [_u8p, _u8p, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]
-        L.orc_score_window.argtypes = [_u8p, C.c_int, _u8p, _u8p, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]
+        L.orc_score_window.argtypes = [_u8p, C.c_int, _u8p, _u8p, C.c_int, _u8p, _u8p, C.POINTER(C.c_int), C.POINTER(C.c_int)]
         L.orc_score_window.restype = C.c_int
         L.orc_hist_normalized.argtypes = [_u8p, C.c_int, _f32p]
         L.orc_hist_correl.argtypes = [_f32p, _f32p]
@@ -69,29 +69,57 @@ def lib():
         L.orc_lda_predict.argtypes = [_f32p, C.c_int, C.c_int, _f64p, _f64p, C.c_double, _f64p, _i32p]
         L.orc_knn_predict.argtypes = [_f32p, C.c_int, C.c_int, _f64p, _f64p, _f64p, _i32p, C.c_int, C.c_int, _f64p, _i32p]
         L.orc_detect_frame.argtypes = [_u8p, C.c_int, C.c_int, _i32p, C.c_int, C.c_double, C.c_int, _u8p, _u8p, C.c_int,
+                                       C.c_double, C.c_double, _u8p, _u8p, C.c_double, C.c_double, C.c_double,
                                        _i32p, _i32p, _i32p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.orc_detect_frame.restype = C.c_int
         _lib = L
     return _lib
 
 
+# ---- the tsd_config fields the oracle takes ------------------------------------------------------------------------
+# The reference's constants (DET:119-129,164,70-87,712); `cfg` below is a tsd_config (ctypes) or any object with these field names.
+DEFAULTS = dict(aspect_lo=0.8, aspect_hi=1.20, hist_tol=0.85, coord_tol=0.95, merge_factor=0.8823,
+                red_lo=((0, 50, 10), (160, 50, 10)), red_hi=((10, 255, 255), (179, 255, 255)), blue_lo=(90, 70, 10),
+                blue_hi=(128, 255, 255))
+
+
+def _config(cfg, kw, names):
+    """-> {name: value} for `names`: keyword argument, else cfg's field, else the reference's constant."""
+    unknown = set(kw) - set(DEFAULTS)
+    if unknown:
+        raise TypeError("unknown config fields %s" % sorted(unknown))
+    return {k: kw[k] if k in kw else getattr(cfg, k) if cfg is not None else DEFAULTS[k] for k in names}
+
+
+def _hsv_bounds(cfg, kw):
+    """-> (lo, hi) uint8 [3][3] (red band 0, red band 1, blue) x (H, S, V)."""
+    v = _config(cfg, kw, ("red_lo", "red_hi", "blue_lo", "blue_hi"))
+    lo = np.array([list(v["red_lo"][0]), list(v["red_lo"][1]), list(v["blue_lo"])], np.uint8)
+    hi = np.array([list(v["red_hi"][0]), list(v["red_hi"][1]), list(v["blue_hi"])], np.uint8)
+    return lo.reshape(-1), hi.reshape(-1)
+
+
 # ---- A.1  DET:155-174 / REC:88-107 -------------------------------------------------------------------------------
-def expand_box(box, percentage):
-    """(x,y,w,h) int32 -> (x1,y1,x2,y2) tuple or None."""
+def expand_box(box, percentage, cfg=None, **kw):
+    """(x,y,w,h) int32 -> (x1,y1,x2,y2) tuple or None.  Aspect bounds: aspect_lo / aspect_hi (cfg or keywords)."""
+    a = _config(cfg, kw, ("aspect_lo", "aspect_hi"))
     out = np.zeros(4, np.int32)
-    ok = lib().orc_expand_box(int(box[0]), int(box[1]), int(box[2]), int(box[3]), float(percentage), out)
+    ok = lib().orc_expand_box(int(box[0]), int(box[1]), int(box[2]), int(box[3]), float(percentage), float(a["aspect_lo"]),
+                              float(a["aspect_hi"]), out)
     return tuple(int(v) for v in out) if ok else None
 
 
-def expand_boxes(boxes, percentage):
+def expand_boxes(boxes, percentage, cfg=None, **kw):
     """boxes int32[n,4] -> (coords int32[n,4], valid bool[n])."""
+    a = _config(cfg, kw, ("aspect_lo", "aspect_hi"))
     boxes = np.ascontiguousarray(boxes, np.int32).reshape(-1, 4)
     coords = np.zeros_like(boxes)
     valid = np.zeros(len(boxes), bool)
     out = np.zeros(4, np.int32)
     L = lib()
     for i, b in enumerate(boxes):
-        if L.orc_expand_box(int(b[0]), int(b[1]), int(b[2]), int(b[3]), float(percentage), out):
+        if L.orc_expand_box(int(b[0]), int(b[1]), int(b[2]), int(b[3]), float(percentage), float(a["aspect_lo"]),
+                            float(a["aspect_hi"]), out):
             coords[i] = out
             valid[i] = True
     return coords, valid
@@ -131,13 +159,15 @@ def bgr2hsv(bgr):
     return out
 
 
-def color_masks(window):
-    """-> (red uint8[D,D], blue uint8[D,D]) in {0,255}; getColorMaskRedOrBlue(img,'r'/'b')."""
+def color_masks(window, cfg=None, **kw):
+    """-> (red uint8[D,D], blue uint8[D,D]) in {0,255}; getColorMaskRedOrBlue(img,'r'/'b').  HSV bounds: red_lo, red_hi
+    [2][3], blue_lo, blue_hi [3] (cfg or keywords)."""
     window = np.ascontiguousarray(window, np.uint8)
     shp = window.shape[:-1]
     red = np.empty(shp, np.uint8)
     blue = np.empty(shp, np.uint8)
-    lib().orc_color_masks(window.reshape(-1), window.size // 3, red.reshape(-1), blue.reshape(-1))
+    lo, hi = _hsv_bounds(cfg, kw)
+    lib().orc_color_masks(window.reshape(-1), window.size // 3, lo, hi, red.reshape(-1), blue.reshape(-1))
     return red, blue
 
 
@@ -150,13 +180,14 @@ def score_hundredths(mask, templ):
     return s, tuple(int(c) for c in counts)
 
 
-def score_window(window, red6, blue6, tol_hundredths=55):
-    """detectionsMaskCorrelation -> (emitted, id, hundredths)."""
+def score_window(window, red6, blue6, tol_hundredths=55, cfg=None, **kw):
+    """detectionsMaskCorrelation -> (emitted, id, hundredths).  HSV bounds as in color_masks."""
     D = window.shape[0]
     i, h = C.c_int(), C.c_int()
+    lo, hi = _hsv_bounds(cfg, kw)
     ok = lib().orc_score_window(np.ascontiguousarray(window, np.uint8).reshape(-1), D,
                                 np.ascontiguousarray(red6, np.uint8).reshape(-1),
-                                np.ascontiguousarray(blue6, np.uint8).reshape(-1), tol_hundredths, C.byref(i), C.byref(h))
+                                np.ascontiguousarray(blue6, np.uint8).reshape(-1), int(tol_hundredths), lo, hi, C.byref(i), C.byref(h))
     return bool(ok), i.value, h.value
 
 
@@ -284,8 +315,11 @@ def knn_predict(X, xbar, S, Ztrain, ytrain, k=4):
 
 
 # ---- whole frame: DET:116-131 + 708-716 --------------------------------------------------------------------------
-def detect_frame(frame, boxes, red6, blue6, percentage=1.30, D=25, tol_hundredths=55, want_survivors=False):
-    """-> dict(coords int32[nd,4], ids, hundredths, stage_counts[4] [, surv_windows, surv_coords])."""
+def detect_frame(frame, boxes, red6, blue6, percentage=1.30, D=25, tol_hundredths=55, want_survivors=False, cfg=None, **kw):
+    """-> dict(coords int32[nd,4], ids, hundredths, stage_counts[4] [, surv_windows, surv_coords]).
+    cfg (or keywords): aspect_lo / aspect_hi, the HSV bounds, hist_tol, coord_tol, merge_factor."""
+    a = _config(cfg, kw, ("aspect_lo", "aspect_hi", "hist_tol", "coord_tol", "merge_factor"))
+    lo, hi = _hsv_bounds(cfg, kw)
     frame = np.ascontiguousarray(frame, np.uint8)
     boxes = np.ascontiguousarray(boxes, np.int32).reshape(-1, 4)
     n = len(boxes)
@@ -299,8 +333,9 @@ def detect_frame(frame, boxes, red6, blue6, percentage=1.30, D=25, tol_hundredth
     sco = np.zeros((cap, 4), np.int32) if want_survivors else None
     nd = lib().orc_detect_frame(frame.reshape(-1), H, W, boxes.reshape(-1), n, float(percentage), D,
                                 np.ascontiguousarray(red6, np.uint8).reshape(-1),
-                                np.ascontiguousarray(blue6, np.uint8).reshape(-1), tol_hundredths,
-                                dc.reshape(-1), di, dh,
+                                np.ascontiguousarray(blue6, np.uint8).reshape(-1), int(tol_hundredths),
+                                float(a["aspect_lo"]), float(a["aspect_hi"]), lo, hi, float(a["hist_tol"]), float(a["coord_tol"]),
+                                float(a["merge_factor"]), dc.reshape(-1), di, dh,
                                 sw.ctypes.data if sw is not None else None,
                                 sco.ctypes.data if sco is not None else None, sc.ctypes.data)
     out = dict(coords=dc[:nd].copy(), ids=di[:nd].copy(), hundredths=dh[:nd].copy(), stage_counts=sc)

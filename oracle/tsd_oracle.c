@@ -30,15 +30,16 @@
 /* ------------------------------------------------------------------------------------------------
  * A.1  makeWindowBiggerOrDiscardFakeDetections  -- DET/source.py:155-174 (= REC/source.py:88-107)
  * box = numpy int32 (x, y, w, h); percentage = Python float literal (1.30 det / 1.15 rec).
- * Returns 1 and writes (x1,y1,x2,y2) when 0.8 < w/h < 1.2 (strict), else 0.
+ * Returns 1 and writes (x1,y1,x2,y2) when aspect_lo < w/h < aspect_hi (strict; the reference's 0.8 and 1.20), else 0.
  * ---------------------------------------------------------------------------------------------- */
-ORC_API int orc_expand_box(int32_t x, int32_t y, int32_t w, int32_t h, double percentage, int32_t out[4])
+ORC_API int orc_expand_box(int32_t x, int32_t y, int32_t w, int32_t h, double percentage, double aspect_lo, double aspect_hi,
+                           int32_t out[4])
 {
     double pm1 = percentage - 1.0;                 /* (percentage - 1) evaluated in f64, :161 */
     double dw = ((double)w * pm1) * 0.5;           /* w * (p-1) * 0.5, left to right          */
     double dh = ((double)h * pm1) * 0.5;
     double ratio = (double)w / (double)h;          /* numpy int32 / int32 -> float64 (:164); h==0 -> inf/nan -> reject */
-    if (!(0.8 < ratio && ratio < 1.20)) return 0;
+    if (!(aspect_lo < ratio && ratio < aspect_hi)) return 0;
     double x1 = (double)x - dw, y1 = (double)y - dh;
     double x2 = (double)(x + w) + dw, y2 = (double)(y + h) + dh;
     x1 = x1 > 0 ? x1 : 0;  y1 = y1 > 0 ? y1 : 0;   /* only the low side is clamped (:167-168) */
@@ -175,17 +176,27 @@ ORC_API void orc_bgr2hsv(const uint8_t *bgr, int npx, uint8_t *hsv)
     }
 }
 
-/* red: H in [0,10] u [160,179], S>=50, V>=10 (:70-79); blue: H in [90,128], S>=70, V>=10 (:85-87) */
-ORC_API void orc_color_masks(const uint8_t *bgr, int npx, uint8_t *red, uint8_t *blue)
+/* cv2.inRange bounds of the three bands [red band 0, red band 1, blue][H, S, V], inclusive (DET:70-87):
+ * red: H in [0,10] u [160,179], S>=50, V>=10 (:70-79); blue: H in [90,128], S>=70, V>=10 (:85-87). */
+static const uint8_t k_hsv_lo[9] = {0, 50, 10, 160, 50, 10, 90, 70, 10};
+static const uint8_t k_hsv_hi[9] = {10, 255, 255, 179, 255, 255, 128, 255, 255};
+
+static inline int in_band(int H, int S, int V, const uint8_t *lo, const uint8_t *hi)
+{
+    return H >= lo[0] && H <= hi[0] && S >= lo[1] && S <= hi[1] && V >= lo[2] && V <= hi[2];
+}
+
+/* hsv_lo / hsv_hi: uint8 [3][3] as above, or NULL for the reference's bounds */
+ORC_API void orc_color_masks(const uint8_t *bgr, int npx, const uint8_t *hsv_lo, const uint8_t *hsv_hi, uint8_t *red, uint8_t *blue)
 {
     hsv_tables();
+    const uint8_t *lo = hsv_lo ? hsv_lo : k_hsv_lo, *hi = hsv_hi ? hsv_hi : k_hsv_hi;
     for (int i = 0; i < npx; i++) {
         int H, S, V;
         bgr2hsv_px(bgr[3 * i], bgr[3 * i + 1], bgr[3 * i + 2], &H, &S, &V);
-        int lo = (H <= 10) && S >= 50 && V >= 10;
-        int hi = (H >= 160 && H <= 179) && S >= 50 && V >= 10;
-        red[i] = (uint8_t)((lo || hi) ? 255 : 0);           /* cv2.add saturates 255+255 -> 255 */
-        blue[i] = (uint8_t)((H >= 90 && H <= 128 && S >= 70 && V >= 10) ? 255 : 0);
+        int r0 = in_band(H, S, V, lo, hi), r1 = in_band(H, S, V, lo + 3, hi + 3);
+        red[i] = (uint8_t)((r0 || r1) ? 255 : 0);           /* cv2.add saturates 255+255 -> 255 */
+        blue[i] = (uint8_t)(in_band(H, S, V, lo + 6, hi + 6) ? 255 : 0);
     }
 }
 
@@ -235,11 +246,11 @@ ORC_API void orc_best_template(const uint8_t *mask, const uint8_t *templates6, i
 /* detectionsMaskCorrelation (:229-245): red wins only if strictly greater; emit iff winner > tol.
  * Returns 1 and fills (id, hundredths) if emitted. tol_hundredths = 55 for 0.55. */
 ORC_API int orc_score_window(const uint8_t *bgr, int D, const uint8_t *red6, const uint8_t *blue6,
-                             int tol_hundredths, int *id, int *hundredths)
+                             int tol_hundredths, const uint8_t *hsv_lo, const uint8_t *hsv_hi, int *id, int *hundredths)
 {
     int npx = D * D;
     uint8_t *r = (uint8_t *)malloc((size_t)npx), *b = (uint8_t *)malloc((size_t)npx);
-    orc_color_masks(bgr, npx, r, b);
+    orc_color_masks(bgr, npx, hsv_lo, hsv_hi, r, b);
     int sr, ir, sb, ib;
     orc_best_template(r, red6, npx, &sr, &ir);
     orc_best_template(b, blue6, npx, &sb, &ib);
@@ -656,10 +667,13 @@ ORC_API void orc_knn_predict(const float *X, int n, int nfeat, const double *xba
  * Whole-frame restatement of MSERTrafficSignDetector's post-MSER part (DET/source.py:116-131) followed by
  * the mask-correlation filter (:708-716); used as the bounded CPU sample in bench.py and in parity tests.
  * boxes: n x 4 (x,y,w,h).  Outputs (capacity n): det_coords [.,4], det_id, det_hundredths.
+ * The tsd_config fields: aspect bounds (0.8, 1.20), HSV bounds (NULL = the reference's), hist_tol 0.85, coord_tol 0.95,
+ * merge_factor 0.8823.
  * stage_counts (optional int[4]) = {raw, aspect-passing, survivors after both passes, detections}.
  * ---------------------------------------------------------------------------------------------- */
 ORC_API int orc_detect_frame(const uint8_t *frame, int H, int W, const int32_t *boxes, int n, double percentage, int D,
-                             const uint8_t *red6, const uint8_t *blue6, int tol_hundredths,
+                             const uint8_t *red6, const uint8_t *blue6, int tol_hundredths, double aspect_lo, double aspect_hi,
+                             const uint8_t *hsv_lo, const uint8_t *hsv_hi, double hist_tol, double coord_tol, double merge_factor,
                              int32_t *det_coords, int32_t *det_id, int32_t *det_hundredths,
                              uint8_t *surv_windows /* optional, n*D*D*3 */, int32_t *surv_coords /* optional n*4 */,
                              int32_t *stage_counts)
@@ -670,20 +684,20 @@ ORC_API int orc_detect_frame(const uint8_t *frame, int H, int W, const int32_t *
     int m = 0;
     for (int i = 0; i < n; i++) {
         int32_t c[4];
-        if (!orc_expand_box(boxes[4 * i], boxes[4 * i + 1], boxes[4 * i + 2], boxes[4 * i + 3], percentage, c)) continue;
+        if (!orc_expand_box(boxes[4 * i], boxes[4 * i + 1], boxes[4 * i + 2], boxes[4 * i + 3], percentage, aspect_lo, aspect_hi, c)) continue;
         if (!orc_crop_resize(frame, H, W, 3, c, win + wb * m, D)) continue;   /* cv2.resize would raise on an empty crop */
         memcpy(co + 4 * m, c, sizeof c);
         m++;
     }
     int passing = m;
-    m = orc_dedup(win, co, m, D, 0, 0.85, 0.8823, NULL);
-    m = orc_dedup(win, co, m, D, 1, 0.95, 0.8823, NULL);
+    m = orc_dedup(win, co, m, D, 0, hist_tol, merge_factor, NULL);
+    m = orc_dedup(win, co, m, D, 1, coord_tol, merge_factor, NULL);
     if (surv_windows) memcpy(surv_windows, win, wb * (size_t)m);
     if (surv_coords) memcpy(surv_coords, co, sizeof(int32_t) * 4 * (size_t)m);
     int nd = 0;
     for (int i = 0; i < m; i++) {
         int id, hs;
-        if (orc_score_window(win + wb * i, D, red6, blue6, tol_hundredths, &id, &hs)) {
+        if (orc_score_window(win + wb * i, D, red6, blue6, tol_hundredths, hsv_lo, hsv_hi, &id, &hs)) {
             memcpy(det_coords + 4 * nd, co + 4 * i, sizeof(int32_t) * 4);
             det_id[nd] = id; det_hundredths[nd] = hs; nd++;
         }
