@@ -86,8 +86,11 @@ TSD_API int tsd_synchronize(tsd_ctx *ctx);
  * context's stream therefore waits for a batch only when the NEXT batch is enqueued, or when tsd_flush / tsd_synchronize /
  * tsd_fetch_detections is called: tsd_flush makes tsd_stream() wait for everything enqueued so far without blocking the host.
  * The front half of a batch (K1, K2, histograms, pair classes) starts only when the previous batch's has ended, which keeps the
- * two streams half a period apart (TSD_STAGGER=0 turns that off); the kernel sequence of a batch shape is replayed as a CUDA
- * graph from its third sighting on (TSD_GRAPH=0: eager launches). */
+ * two streams half a period apart (TSD_STAGGER=0 turns that off).  The kernel sequence of a batch runs eagerly the first time,
+ * is captured into a CUDA graph the second time and replayed from then on (TSD_GRAPH=0: eager launches; none while profiling).
+ * A batch's key includes its scratch slot, so a batch shape repeated in overlap mode runs eagerly on calls 1 and 2, is captured
+ * on calls 3 and 4 and is replayed from call 5 on.  Up to 8 graphs are kept; a cycle of more than 8 keys runs eagerly.
+ * tsd_stat_graphs counts captures and replays. */
 TSD_API int tsd_flush(tsd_ctx *ctx);
 /* Page-lock a caller-owned host buffer (cudaHostRegister, mapped).  tsd_detect_frames with TSD_MEM_HOST reads page-locked
  * frames IN PLACE over PCIe (only the 32-byte sectors the candidate ROIs touch are transferred, each once per batch, into a
@@ -98,8 +101,12 @@ TSD_API int tsd_flush(tsd_ctx *ctx);
  * page-locked layout is read by K2 itself, tap by tap over PCIe (as with TSD_STAGE=0).  Either way the records are the same. */
 TSD_API int tsd_host_register(void *p, int64_t bytes);
 TSD_API int tsd_host_unregister(void *p);
-/* Number of kernels this library launched on the context since creation (bench.py's gpu_launches). */
+/* Number of kernels this library launched on the context since creation (bench.py's gpu_launches).  A replayed CUDA graph
+ * counts the kernels it holds. */
 TSD_API int64_t tsd_launch_count(tsd_ctx *ctx);
+/* Measurement helper: CUDA graphs of the chain instantiated (*captured) and cached graphs launched again (*replayed) on the
+ * context since its creation.  Host-side counters: does not synchronise. */
+TSD_API int tsd_stat_graphs(tsd_ctx *ctx, int64_t *captured, int64_t *replayed);
 
 /* ---- model / template state (host pointers) --------------------------------------------------------------- */
 /* 6 red + 6 blue template masks, uint8 [6][D*D] in {0,255}: output of calculateMeanMasks (DET/source.py:24-59),
@@ -262,8 +269,9 @@ TSD_API int tsd_fetch_detections(tsd_ctx *ctx, tsd_detection *det, int det_cap, 
  * frames over PCIe under batch k's GPU-bound kernels.  TSD_E_STATE if there is no such batch. */
 TSD_API int tsd_fetch_previous(tsd_ctx *ctx, tsd_detection *det, int det_cap, int32_t *ndet, int32_t *counts /* [4] or NULL */);
 
-/* Measurement helper: total number of non-zero histogram bins over the windows of the last tsd_enqueue_frames call
- * (the bytes k5_pairs has to read at least once).  Synchronises. */
+/* Measurement helper: total number of non-zero histogram bins over the windows of the last tsd_enqueue_frames call, each
+ * window as the first duplicate-removal pass leaves it: an item that absorbed a near duplicate counts the histogram of its
+ * merged pixels (the fold rebuilds it in place).  It approximates the bytes k5_pairs has to read at least once.  Synchronises. */
 TSD_API int tsd_stat_hist_entries(tsd_ctx *ctx, int64_t *total);
 
 /* Measurement helper: number of window pairs (since process start, this device) whose class could not be decided from the exact

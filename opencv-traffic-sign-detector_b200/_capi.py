@@ -65,6 +65,7 @@ _SIGNATURES = {
     "tsd_stat_hist_entries": (_i, [_vp, C.POINTER(C.c_int64)]),
     "tsd_stat_unsure_pairs": (_i, [_vp, C.POINTER(C.c_int64), _i]),
     "tsd_stat_staged_bytes": (_i, [_vp, C.POINTER(C.c_int64), _i]),
+    "tsd_stat_graphs": (_i, [_vp, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "tsd_host_unregister": (_i, [_vp]),
     "tsd_set_templates": (_i, [_vp, _vp, _vp]),
     "tsd_set_similarity_table": (_i, [_vp, _vp, _i]),

@@ -113,13 +113,17 @@ struct tsd_ctx {
     std::vector<cudaEvent_t> ev;
     std::vector<std::string> ev_names;
     int ev_used = 0;
-    // CUDA graphs of the chain (TSD_GRAPH=0 turns them off): a batch shape seen twice in a row is captured once and replayed from then
-    // on -- the chains of small batches (real MSER frames) are bound by launch latency.  `gen` counts every event that changes a
-    // pointer baked into a captured kernel argument (scratch reallocation, slot layout, model state) and is part of the key.
+    // CUDA graphs of the chain (TSD_GRAPH=0 turns them off): a batch key met again while it is among the last kGraphCap keys run
+    // eagerly is captured once and replayed from then on -- the chains of small batches (real MSER frames) are bound by launch
+    // latency.  The key holds the slot's scratch pointers, so in overlap mode each slot has its own key: a repeated batch is
+    // eager on calls 1-2, captured on calls 3-4 and replayed from call 5 on.  `gen` counts every event that changes a pointer
+    // baked into a captured kernel argument (scratch reallocation, slot layout, model state) and is part of the key.
+    static constexpr size_t kGraphCap = 8;   // graphs kept (least recently used goes first) = keys remembered from eager runs
     struct GraphEntry { std::vector<uint64_t> key; cudaGraphExec_t exec = nullptr; int64_t launches = 0; uint64_t stamp = 0; };
     std::vector<GraphEntry> graphs;
-    std::vector<uint64_t> seen_key;
+    std::vector<std::vector<uint64_t>> seen_keys;   // keys of the last eager runs, oldest first
     uint64_t gen = 0, graph_clock = 0;
+    int64_t graphs_captured = 0, graphs_replayed = 0;   // tsd_stat_graphs
     int use_graph = 1;
 };
 
@@ -156,17 +160,11 @@ static int allow_dynamic_smem(tsd_ctx* c, const void* fn, size_t bytes, const ch
     return TSD_OK;
 }
 
-// Event record / wait on c->cur that also works while the stream is being captured into a CUDA graph (external event nodes).
+// Event record on c->cur that also works while the stream is being captured into a CUDA graph (external event node).
 static int ev_record(tsd_ctx* c, cudaEvent_t ev) {
     cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
     CU(cudaStreamIsCapturing(c->cur, &st));
     CU(cudaEventRecordWithFlags(ev, c->cur, st == cudaStreamCaptureStatusActive ? cudaEventRecordExternal : cudaEventRecordDefault));
-    return TSD_OK;
-}
-static int ev_wait(tsd_ctx* c, cudaEvent_t ev) {
-    cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
-    CU(cudaStreamIsCapturing(c->cur, &st));
-    CU(cudaStreamWaitEvent(c->cur, ev, st == cudaStreamCaptureStatusActive ? cudaEventWaitExternal : cudaEventWaitDefault));
     return TSD_OK;
 }
 
@@ -415,6 +413,13 @@ int tsd_synchronize(tsd_ctx* c) {
 }
 
 int64_t tsd_launch_count(tsd_ctx* c) { return c ? c->launches : 0; }
+
+int tsd_stat_graphs(tsd_ctx* c, int64_t* captured, int64_t* replayed) {
+    if (!c || !captured || !replayed) return fail(TSD_E_INVALID, "bad argument");
+    *captured = c->graphs_captured;
+    *replayed = c->graphs_replayed;
+    return TSD_OK;
+}
 
 int tsd_set_profiling(tsd_ctx* c, int on) {
     if (!c) return fail(TSD_E_INVALID, "ctx is NULL");
@@ -1368,8 +1373,8 @@ static int enqueue_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, i
     // front half (K1, K2, histograms, pair classes) of the next.  Left alone the two streams share the GPU evenly, drift into
     // phase and end up folding at the same time (3.24 ms per 4096-frame step against 2.6 ms of kernel work); making the front
     // half of a batch wait for the previous batch's keeps them a half period apart.
+    // (the wait for the previous batch's front half is issued by enqueue_impl before this sequence, outside any capture)
     const bool stagger = B.in_slot && c->stagger;
-    if (stagger) TRY(ev_wait(c, c->ev_w1[B.sidx ^ 1]));
     mark(c, "start");
     // K1: candidate loop of MSERTrafficSignDetector (DET:116-120)
     TRY(dev_windows_index(c, d_boxes, d_box_offsets, cf, H, W, c->cfg.enlarge, cnt, winoff, coords, winframe));
@@ -1460,8 +1465,9 @@ static int enqueue_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, i
     return TSD_OK;
 }
 
-// One batch through the chain on c->cur: eagerly the first time a batch shape is seen, captured into a CUDA graph the second time,
-// replayed from then on (at most 8 graphs are kept, least recently used goes first).
+// One batch through the chain on c->cur: eagerly the first time a batch key is seen, captured into a CUDA graph when it comes back
+// while it is among the last kGraphCap eagerly run keys, replayed from then on (at most kGraphCap graphs are kept, least recently
+// used goes first).  A cycle of more than kGraphCap keys therefore always runs eagerly instead of capturing on every call.
 static int run_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, int W, int64_t row_stride, int64_t frame_stride,
                      const int32_t* d_boxes, const int32_t* d_box_offsets, int maxb, const tsd_ctx::Batch& B, uint32_t* M, int32_t* todo,
                      const uint8_t* host_src) {
@@ -1477,13 +1483,16 @@ static int run_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, int W
             CU(cudaGraphLaunch(g.exec, c->cur));
             g.stamp = c->graph_clock;
             c->launches += g.launches;
+            c->graphs_replayed++;
             return TSD_OK;
         }
-    if (c->seen_key != key) {                                // first sighting: run it eagerly (one-off calls never pay for an instantiation)
-        c->seen_key = key;
+    const auto seen = std::find(c->seen_keys.begin(), c->seen_keys.end(), key);
+    if (seen == c->seen_keys.end()) {                        // first sighting: run it eagerly (one-off calls never pay for an instantiation)
+        if (c->seen_keys.size() >= tsd_ctx::kGraphCap) c->seen_keys.erase(c->seen_keys.begin());
+        c->seen_keys.push_back(key);
         return enqueue_chain(c, mode, d_frames, H, W, row_stride, frame_stride, d_boxes, d_box_offsets, maxb, B, M, todo, host_src);
     }
-    c->seen_key.clear();
+    c->seen_keys.erase(seen);
     const int64_t l0 = c->launches;
     CU(cudaStreamBeginCapture(c->cur, cudaStreamCaptureModeThreadLocal));
     const int rc = enqueue_chain(c, mode, d_frames, H, W, row_stride, frame_stride, d_boxes, d_box_offsets, maxb, B, M, todo, host_src);
@@ -1496,7 +1505,8 @@ static int run_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, int W
     const cudaError_t ei = cudaGraphInstantiate(&g.exec, graph, 0);
     cudaGraphDestroy(graph);
     if (ei != cudaSuccess) return fail(TSD_E_CUDA, "cudaGraphInstantiate: %s", cudaGetErrorString(ei));
-    if (c->graphs.size() >= 8) {
+    c->graphs_captured++;
+    if (c->graphs.size() >= tsd_ctx::kGraphCap) {
         size_t lru = 0;
         for (size_t i = 1; i < c->graphs.size(); i++) if (c->graphs[i].stamp < c->graphs[lru].stamp) lru = i;
         cudaGraphExecDestroy(c->graphs[lru].exec);
@@ -1611,6 +1621,9 @@ static int enqueue_impl(tsd_ctx* c, int mode, const uint8_t* d_frames, int nfram
         TRY(join_pending(c));                                // the PREVIOUS batch: the context's stream waits for it only now, after this batch's fork
         c->cur = c->os[sl];
         c->ticket_base = 8 * sl;
+        // TSD_STAGGER: the front half of this batch starts when the previous batch's has ended (the event enqueue_chain records).
+        // Waited here, on the stream, for a captured graph as well: the graph then holds only the record, as an external event node.
+        if (c->stagger) CU(cudaStreamWaitEvent(c->cur, c->ev_w1[sl ^ 1], 0));
         rc = run_chain(c, mode, d_frames, H, W, row_stride, frame_stride, d_boxes, d_box_offsets, max_boxes_per_frame, B, M, todo, host_src);
         CU(cudaEventRecord(c->ev_join[sl], c->os[sl]));
         c->pending_join = sl;

@@ -319,6 +319,13 @@ class Context:
         check(self._L.tsd_stat_staged_bytes(self._h, C.byref(t), int(bool(reset))))
         return int(t.value)
 
+    def stat_graphs(self):
+        """(captured, replayed): CUDA graphs of the chain instantiated, and cached graphs launched again, since the context was
+        created (host-side counters, no synchronisation)."""
+        cap, rep = C.c_int64(), C.c_int64()
+        check(self._L.tsd_stat_graphs(self._h, C.byref(cap), C.byref(rep)))
+        return int(cap.value), int(rep.value)
+
     def preprocess(self, frames, clip_limit=2.0, tiles=(8, 8), gamma=2):
         """grayAndEnhanceContrast (DET:135-152) for a batch: BGR2GRAY -> CLAHE -> GaussianBlur 3x3 -> gamma LUT.
         frames uint8 [F,H,W,3] or [H,W,3] -> uint8 [F,H,W] (or [H,W])."""

@@ -306,8 +306,9 @@ def test_timeline_and_stagger_switch(tsd, oracle, templates, monkeypatch):
         with tsd.Context(0, "det") as ctx:
             ctx.set_templates(red6, blue6)
             one = lambda: ctx.enqueue_frames(d_frames.data_ptr(), F, 800, 1360, d_boxes.data_ptr(), d_off.data_ptr(), int(off[-1]), max_boxes_per_frame=N)
-            for _ in range(4):                               # eager, captured, replayed, replayed (CUDA graph with external event nodes)
-                one()
+            for _ in range(4):                               # one key per slot: eager, eager, captured, captured (CUDA graphs holding
+                one()                                        # the stagger's event record as an external event node)
+            assert ctx.stat_graphs() == (2, 0)
             prev, _ = ctx.fetch_detections(int(off[-1]), previous=True)
             last, _ = ctx.fetch_detections(int(off[-1]))
             assert rec(prev) == exp and rec(last) == exp, (stagger, cap)
