@@ -4,7 +4,6 @@
 #include "../../include/tsd_b200.h"
 #include "tsd_kernels.cuh"
 #include "tsd_k5.cuh"
-#include "tsd_k2_tma.cuh"
 
 #include <math.h>
 #include <stdarg.h>
@@ -75,7 +74,6 @@ struct tsd_ctx {
     DevBuf b_mirror[2], b_stagemap[2];       // per scratch slot (consecutive batches of a chunked tsd_detect_frames call overlap)
     int stage_chunk = 256;                   // TSD_STAGE_CHUNK: frames per chunk of tsd_detect_frames on page-locked host frames (0 = one batch)
     int stage_ctas = 2;                      // TSD_STAGE_CTAS: CTAs per SM of the staging copy (PCIe-bound: 2 keep the link as busy as 8 and leave the SMs to the other chunk's chain)
-    int stage_gran = 1;                      // TSD_STAGE_GRAN = 32 | 64 | 128 bytes: unit the marked spans are widened to (sectors: 1, 2, 4)
     unsigned long long* d_staged = nullptr;  // bytes the staging copy moved over PCIe (tsd_stat_staged_bytes)
     int chunk_frames = 32;                   // TSD_CHUNK_FRAMES: frames per H2D chunk of the host-buffer path
     tsd_config cfg;
@@ -105,11 +103,9 @@ struct tsd_ctx {
     int use_gram = 1;                        // TSD_GRAM=0: pair classes of every frame from the CUDA-core kernel (k5_pairs)
     int k2_grid = 256;                       // TSD_K2_GRID: CTAs per SM of K2 (0 = one window per warp, no loop).  4096 frames, ms: 12: .830, 24: .784, 48: .741, 96: .718, 128: .715, 192: .708, 256: .709, 384: .704, 640: .709, unlimited (1384): .757
     int fold_per_sm_cap = 2;                 // TSD_FOLD_PER_SM: cap of resident k5_fold_warp CTAs per SM (0 = as many as fit; measured with the staggered overlap at 4096 frames: 0: 3.22, 1: 3.20, 2: 3.09, 3: 3.18 ms per step)
-    int fold_cta_cost = 0;                   // TSD_FOLD_CTA_COST: frames with at least this many merge-band pairs go to the CTA fold (0 = by size only)
     // function attributes (dynamic shared memory opt-in) are set once per context: per-context flags, no process-wide statics
     int fold_per_sm[4] = {0, 0, 0, 0};       // resident CTAs per SM of the four k5_fold_warp instantiations (0 = not queried yet)
-    bool attr_gram = false, attr_pairs = false, attr_k2tma = false;
-    int k2_tma = 0;                          // TSD_K2=tma: the TMA-staged resize kernel (tsd_k2_tma.cuh) instead of the direct gather
+    bool attr_gram = false, attr_pairs = false;
     std::vector<cudaEvent_t> ev;
     std::vector<std::string> ev_names;
     int ev_used = 0;
@@ -239,15 +235,12 @@ static int create_impl(tsd_ctx* c, int device) {
     { const char* e = getenv("TSD_OVERLAP"); if (e) c->overlap = atoi(e) != 0; }
     { const char* e = getenv("TSD_ZEROCOPY"); if (e) c->zero_copy = e[0] != '0'; }
     { const char* e = getenv("TSD_STAGE"); if (e) c->stage_rois = e[0] != '0'; }
-    { const char* e = getenv("TSD_STAGE_GRAN"); if (e) { const int g = atoi(e); c->stage_gran = g >= 128 ? 4 : g >= 64 ? 2 : 1; } }
     { const char* e = getenv("TSD_CHUNK_FRAMES"); if (e && atoi(e) > 0) c->chunk_frames = atoi(e); }
     { const char* e = getenv("TSD_STAGE_CHUNK"); if (e) c->stage_chunk = atoi(e); }
     { const char* e = getenv("TSD_STAGE_CTAS"); if (e && atoi(e) > 0) c->stage_ctas = atoi(e); }
     { const char* e = getenv("TSD_KEEP_MASKS"); if (e) c->keep_masks = atoi(e); }
     { const char* e = getenv("TSD_GRAM"); if (e) c->use_gram = atoi(e) != 0; }
     { const char* e = getenv("TSD_GRAPH"); if (e) c->use_graph = atoi(e) != 0; }
-    { const char* e = getenv("TSD_K2"); if (e) c->k2_tma = strcmp(e, "tma") == 0; }
-    { const char* e = getenv("TSD_FOLD_CTA_COST"); if (e) c->fold_cta_cost = atoi(e); }
     { const char* e = getenv("TSD_FOLD_PER_SM"); if (e) c->fold_per_sm_cap = atoi(e); }
     { const char* e = getenv("TSD_STAGGER"); if (e) c->stagger = atoi(e); }
     { const char* e = getenv("TSD_K2_GRID"); if (e) c->k2_grid = atoi(e); }
@@ -609,41 +602,21 @@ static int dev_expand(tsd_ctx* c, const int32_t* boxes, int n, double enlarge, i
 }
 
 // out_stride = bytes between output windows: D*D*ch (public packed layout) or win_stride() (internal, zero padded).
-// nframes = frames behind `frames` (the TMA variant's tensor map needs the extent; 0 = unknown: direct gather).
+// nframes = frames behind `frames` (0 = unknown: byte loads throughout).
 static int dev_crop_resize(tsd_ctx* c, const uint8_t* frames, int H, int W, int64_t rs, int64_t fs, int ch, const int32_t* coords,
                            const int32_t* win_frame, const int32_t* n_ptr, int n_max, int D, uint8_t* windows, int out_stride, int nframes = 0) {
     if (n_max == 0) return TSD_OK;
     if (rs * (int64_t)H >= ((int64_t)1 << 31)) return fail(TSD_E_INVALID, "a frame must span less than 2 GiB (row offsets are 32-bit)");
     const int g4_all = cdiv(n_max, 4);                       // one window per warp (the generic kernel does not loop)
     int g4 = g4_all;
-    if (c->k2_grid > 0 && g4 > c->k2_grid * c->sm_count) g4 = c->k2_grid * c->sm_count;     // persistent warps (the v2 / TMA kernels stride over the windows)
-    int skip_tma = 0;
+    if (c->k2_grid > 0 && g4 > c->k2_grid * c->sm_count) g4 = c->k2_grid * c->sm_count;     // persistent warps (the v2 kernel strides over the windows)
 #define K2_ARGS frames, H, W, rs, fs, (const int4*)coords, win_frame, n_ptr, n_max
-    // TSD_K2=tma: ROI staged by the Tensor Memory Accelerator (internal 16-byte window layout, BGR, D = 25 / 32, TMA-legal frame layout)
-    if (c->k2_tma && ch == 3 && (D == 25 || D == 32) && nframes > 0 && out_stride % 16 == 0 && ((uintptr_t)windows % 16) == 0) {
-        K2TensorMaps maps;
-        if (k2_build_tensor_maps(&maps, frames, nframes, H, W, rs, fs)) {
-            const size_t smem = (size_t)kTmaWarps * tma_warp_bytes(D) + 128;
-            if (!c->attr_k2tma) {
-                CU(cudaFuncSetAttribute(k2_crop_resize_tma_kernel<25>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kTmaWarps * tma_warp_bytes(25) + 128)));
-                CU(cudaFuncSetAttribute(k2_crop_resize_tma_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kTmaWarps * tma_warp_bytes(32) + 128)));
-                CU(cudaFuncSetAttribute(k2_crop_resize_tma_kernel<25>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-                CU(cudaFuncSetAttribute(k2_crop_resize_tma_kernel<32>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-                c->attr_k2tma = true;
-            }
-            // one window per warp; the crops that do not fit the staging buffer are left to the gather kernel launched right after
-            if (D == 25) k2_crop_resize_tma_kernel<25><<<g4, kTmaWarps * 32, smem, c->cur>>>(maps, K2_ARGS, windows, out_stride);
-            else k2_crop_resize_tma_kernel<32><<<g4, kTmaWarps * 32, smem, c->cur>>>(maps, K2_ARGS, windows, out_stride);
-            TRY(check_launch(c, "k2_crop_resize_tma"));
-            skip_tma = 1;
-        }
-    }
     // aligned 32-bit tap loads need 4-byte aligned frames and strides and the number of frames (the last row of the last frame keeps byte loads)
     const int wide_last = (nframes > 0 && ((uintptr_t)frames % 4) == 0 && rs % 4 == 0 && fs % 4 == 0) ? nframes - 1 : -2;
-    if (ch == 3 && D == 25) k2_crop_resize_v2_kernel<3, 25><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, skip_tma, wide_last);
-    else if (ch == 3 && D == 32) k2_crop_resize_v2_kernel<3, 32><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, skip_tma, wide_last);
-    else if (ch == 1 && D == 25) k2_crop_resize_v2_kernel<1, 25><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, 0, -2);
-    else if (ch == 1 && D == 32) k2_crop_resize_v2_kernel<1, 32><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, 0, -2);
+    if (ch == 3 && D == 25) k2_crop_resize_v2_kernel<3, 25><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, wide_last);
+    else if (ch == 3 && D == 32) k2_crop_resize_v2_kernel<3, 32><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, wide_last);
+    else if (ch == 1 && D == 25) k2_crop_resize_v2_kernel<1, 25><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, -2);
+    else if (ch == 1 && D == 32) k2_crop_resize_v2_kernel<1, 32><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, -2);
     else if (ch == 3) k2_crop_resize_kernel<3><<<g4_all, 128, 0, c->cur>>>(K2_ARGS, D, windows, out_stride);      // other window sizes: generic kernel
     else k2_crop_resize_kernel<1><<<g4_all, 128, 0, c->cur>>>(K2_ARGS, D, windows, out_stride);
 #undef K2_ARGS
@@ -708,26 +681,22 @@ static int launch_folds(tsd_ctx* c, int variant, const FoldParams& P, int nframe
         if (per_sm_cta < 1) per_sm_cta = 1;
         if (getenv("TSD_DEBUG")) fprintf(stderr, "[tsd] k5_fold_warp<256,%d>: %zu B shared memory per CTA, %d CTAs per SM; k5_fold_cta: %zu B, %d per SM\n", CAP, smem, per_sm, smem_cta, per_sm_cta);
     }
-    // longest-first frame order + the two work counters + the costs in that order (context scratch: [nframes] order, [2] counters,
-    // [nframes] costs)
-    int32_t* order = (int32_t*)c->b_order.p + 2 * c->order_off;
+    // longest-first frame order + the two work counters (context scratch: [nframes] order, [2] counters)
+    int32_t* order = (int32_t*)c->b_order.p + c->order_off;
     int32_t* counter = order + nframes;
-    int32_t* cost_sorted = counter + 2;
-    k5_order_kernel<<<1, 1024, 0, c->cur>>>(cost, P.offsets, nframes, order, counter, cost_sorted);
+    k5_order_kernel<<<1, 1024, 0, c->cur>>>(cost, P.offsets, nframes, order, counter);
     TRY(check_launch(c, "k5_order"));
-    // frames predicted to merge often go to the CTA fold too (batches large enough for a straggler to matter)
-    const int cost_min = (cost && nframes >= 256) ? c->fold_cta_cost : 0;
     int grid = cdiv(nframes, warps);
     // Resident fold CTAs per SM: each holds 16 K registers and ~56 KB of shared memory, so the four that fit take the WHOLE SM and the
     // kernels of the other batch (two-slot overlap) cannot run beside them; a cap leaves room (the fold is bound by latency, not by
     // the number of its warps: one batch needs ~1100 warp-milliseconds spread over the ~2.6 ms the other batch's kernels take).
     const int cap_sm = (c->fold_per_sm_cap > 0 && c->fold_per_sm_cap < per_sm) ? c->fold_per_sm_cap : per_sm;
     if (grid > cap_sm * c->sm_count) grid = cap_sm * c->sm_count;
-    k5_fold_warp_kernel<256, CAP><<<grid, warps * 32, smem, c->cur>>>(P, nframes, M, RW, cut, order, counter, kFoldCtaMin, cost_sorted, cost_min);
+    k5_fold_warp_kernel<256, CAP><<<grid, warps * 32, smem, c->cur>>>(P, nframes, M, RW, cut, order, counter, kFoldCtaMin);
     TRY(check_launch(c, "k5_fold_warp"));
-    if (max_n > kFoldCtaMin || cost_min > 0) {
+    if (max_n > kFoldCtaMin) {
         grid = nframes < per_sm_cta * c->sm_count ? nframes : per_sm_cta * c->sm_count;
-        k5_fold_cta_kernel<CAP><<<grid, kFoldCtaWarps * 32, smem_cta, c->cur>>>(P, nframes, M, RW, cut, order, counter + 1, kFoldCtaMin, cost_sorted, cost_min);
+        k5_fold_cta_kernel<CAP><<<grid, kFoldCtaWarps * 32, smem_cta, c->cur>>>(P, nframes, M, RW, cut, order, counter + 1, kFoldCtaMin);
         TRY(check_launch(c, "k5_fold_cta"));
     }
     return TSD_OK;
@@ -940,7 +909,7 @@ int tsd_dedup(tsd_ctx* c, const uint8_t* windows, const int32_t* coords, const i
     c->order_off = 0;
     TRY(ensure(c, c->b_pairs, (size_t)(n > 0 ? n : 1) * 2 * pair_row_words(max_n) * sizeof(uint32_t)));
     TRY(ensure(c, c->b_gramdone, 2 * todo_capacity(nframes, max_n) * 4));
-    TRY(ensure(c, c->b_order, (size_t)(2 * nframes + 4) * 4));
+    TRY(ensure(c, c->b_order, (size_t)(nframes + 2) * 4));
     TRY(dev_fold(c, (uint8_t*)dw, ws, (int32_t*)dc, (uint32_t*)dent, (WinMeta*)dmeta, (int32_t*)doff, nframes, npx, !by_coords, by_coords,
                  tol, tol, (int32_t*)dlist, (uint8_t*)dflags, (int32_t*)dcnt, max_n, (uint32_t*)c->b_pairs.p, (int32_t*)c->b_gramdone.p, (float*)den, n, (int32_t*)dooff));
     if (nframes) {
@@ -1385,7 +1354,7 @@ static int enqueue_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, i
         uint32_t* stagemap = (uint32_t*)c->b_stagemap[B.sidx].p;
         CU(cudaMemsetAsync(stagemap, 0, (size_t)nwords * 4, c->cur));
         if (nb > 0) {
-            stage_mark_kernel<<<cdiv((int64_t)nb * 32, 128), 128, 0, c->cur>>>((const int4*)coords, winframe, d_nwin, nb, H, W, D, wpr, c->stage_gran, stagemap);
+            stage_mark_kernel<<<cdiv((int64_t)nb * 32, 128), 128, 0, c->cur>>>((const int4*)coords, winframe, d_nwin, nb, H, W, D, wpr, stagemap);
             TRY(check_launch(c, "stage_mark"));
             int g = cdiv(nwords, 256);
             if (g > c->sm_count * c->stage_ctas) g = c->sm_count * c->stage_ctas;
@@ -1476,7 +1445,7 @@ static int run_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, int W
     const std::vector<uint64_t> key = {(uint64_t)mode, (uint64_t)(uintptr_t)d_frames, (uint64_t)B.nframes, (uint64_t)H, (uint64_t)W, (uint64_t)row_stride,
                                        (uint64_t)frame_stride, (uint64_t)(uintptr_t)d_boxes, (uint64_t)(uintptr_t)d_box_offsets, (uint64_t)B.nbcap, (uint64_t)maxb,
                                        (uint64_t)B.wo, (uint64_t)B.fo, (uint64_t)B.sidx, (uint64_t)(uintptr_t)M, (uint64_t)(uintptr_t)todo,
-                                       (uint64_t)c->ticket_base, c->gen, (uint64_t)c->keep_masks, (uint64_t)c->use_gram, (uint64_t)(uintptr_t)host_src, (uint64_t)c->fold_cta_cost, (uint64_t)c->fold_per_sm_cap, (uint64_t)c->k2_grid, (uint64_t)c->stagger, (uint64_t)c->stage_ctas, (uint64_t)c->stage_gran, (uint64_t)c->k2_tma};
+                                       (uint64_t)c->ticket_base, c->gen, (uint64_t)c->keep_masks, (uint64_t)c->use_gram, (uint64_t)(uintptr_t)host_src, (uint64_t)c->fold_per_sm_cap, (uint64_t)c->k2_grid, (uint64_t)c->stagger, (uint64_t)c->stage_ctas};
     c->graph_clock++;
     for (auto& g : c->graphs)
         if (g.key == key) {
@@ -1580,7 +1549,7 @@ static int enqueue_impl(tsd_ctx* c, int mode, const uint8_t* d_frames, int nfram
     TRY(ensure(c, c->b_detcnt, fcap * 4));
     TRY(ensure(c, c->b_detoff, fcap * 4));
     TRY(ensure(c, c->b_summary, 2 * 16));
-    TRY(ensure(c, c->b_order, (2 * fcap + 4) * 4));
+    TRY(ensure(c, c->b_order, fcap * 4));
     TRY(ensure(c, c->b_gramdone, todo_words * 4));
     TRY(ensure(c, c->b_coords, cap * 16));
     TRY(ensure(c, c->b_winframe, cap * 4));

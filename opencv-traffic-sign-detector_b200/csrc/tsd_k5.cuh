@@ -1103,9 +1103,8 @@ __global__ void __launch_bounds__(kBigWarps * 32, 1) k5_gram_big_kernel(const ui
 
 // Longest-processing-time-first order of the frames for the fold: key = 32 * (merge-band pairs) + windows, counting sort,
 // descending.  One CTA.  Also resets the fold's work counter.
-// cost_sorted[k] = frame_cost of order[k]: the folds route on it (frame_cost itself aliases the survivor counts they write).
 __global__ void __launch_bounds__(1024) k5_order_kernel(const int32_t* __restrict__ frame_cost, const int32_t* __restrict__ offsets, int nframes,
-                                                        int32_t* __restrict__ order, int32_t* __restrict__ counter, int32_t* __restrict__ cost_sorted) {
+                                                        int32_t* __restrict__ order, int32_t* __restrict__ counter) {
     constexpr int NB = 2048;
     __shared__ int32_t hist[NB];
     for (int i = threadIdx.x; i < NB; i += blockDim.x) hist[i] = 0;
@@ -1140,7 +1139,6 @@ __global__ void __launch_bounds__(1024) k5_order_kernel(const int32_t* __restric
         const int key = min(NB - 1, 32 * (frame_cost ? frame_cost[f] : 0) + (offsets[f + 1] - offsets[f]));
         const int pos = atomicAdd(&hist[NB - 1 - key], 1);
         order[pos] = f;
-        cost_sorted[pos] = frame_cost ? frame_cost[f] : 0;
     }
 }
 
@@ -1428,18 +1426,10 @@ __device__ __forceinline__ void fold_emit_survivors(unsigned A, const FoldParams
     __syncwarp();
 }
 
-// Which fold takes a frame: k5_fold_cta (one CTA) the frames of more than n_skip windows and -- cost_min > 0 -- the frames whose
-// merge-band pair count (frame_cost, the fold's cost predictor) reaches cost_min: a frame that merges a dozen times keeps one
-// warp busy for ~0.7 ms while the rest of the batch is long done; k5_fold_warp (one warp) everything else.
-__device__ __forceinline__ bool fold_goes_to_cta(int n, int cost, int n_skip, int cost_min) {
-    return n > n_skip || (cost_min > 0 && cost >= cost_min && n > 32);
-}
-
-// n_skip / cost_min: see fold_goes_to_cta (k5_fold_cta is launched beside this kernel on the same order list).
+// Frames of more than n_skip windows (up to 1024) are k5_fold_cta's: it is launched beside this kernel on the same order list.
 template <int RMAX, int CAP>
 __global__ void __launch_bounds__(kFoldWarps * 32, TSD_FOLD_MINB) k5_fold_warp_kernel(FoldParams P, int nframes, uint32_t* M, int RW, int sim_cut,
-                                                                       const int32_t* __restrict__ order, int32_t* counter, int n_skip,
-                                                                       const int32_t* __restrict__ frame_cost_sorted, int cost_min) {
+                                                                       const int32_t* __restrict__ order, int32_t* counter, int n_skip) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     HsvLut& lut = *reinterpret_cast<HsvLut*>(smem_raw);
     const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -1457,7 +1447,7 @@ __global__ void __launch_bounds__(kFoldWarps * 32, TSD_FOLD_MINB) k5_fold_warp_k
         if (idx >= nframes) break;
         const int f = order[idx];
         const int base = P.offsets[f], n = P.offsets[f + 1] - base;
-        if (n <= RW * 32 && n <= 1024 && fold_goes_to_cta(n, frame_cost_sorted ? frame_cost_sorted[idx] : 0, n_skip, cost_min)) continue;   // k5_fold_cta's frame
+        if (n <= RW * 32 && n <= 1024 && n > n_skip) continue;     // k5_fold_cta's frame
         if (n > RMAX || n > RW * 32) { if (lane == 0) P.out_count[f] = -1; continue; }    // host picks RMAX / RW large enough
         for (int p = lane; p < n; p += 32) sm.hash[p] = P.meta[base + p].hash;
         bool dense_clean = false;                            // the previous frame's pass 2 overlaid the dense scratch: wiped at the first merge
@@ -1782,8 +1772,7 @@ __device__ __forceinline__ unsigned fold_cta_coord_pass(FoldCtaSmem<CAP>& S, con
 
 template <int CAP>
 __global__ void __launch_bounds__(kFoldCtaWarps * 32) k5_fold_cta_kernel(FoldParams P, int nframes, uint32_t* M, int RW, int sim_cut,
-                                                                          const int32_t* __restrict__ order, int32_t* counter, int n_skip,
-                                                                          const int32_t* __restrict__ frame_cost_sorted, int cost_min) {
+                                                                          const int32_t* __restrict__ order, int32_t* counter, int n_skip) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     FoldCtaSmem<CAP>& S = *reinterpret_cast<FoldCtaSmem<CAP>*>(smem_raw);
     FoldWarpSmem<1024, CAP>& sm = S.w;
@@ -1798,7 +1787,7 @@ __global__ void __launch_bounds__(kFoldCtaWarps * 32) k5_fold_cta_kernel(FoldPar
                 const int idx = atomicAdd(counter, 1);
                 if (idx >= nframes) break;
                 const int fc = order[idx], nc = P.offsets[fc + 1] - P.offsets[fc];
-                if (nc <= 1024 && nc <= RW * 32 && fold_goes_to_cta(nc, frame_cost_sorted ? frame_cost_sorted[idx] : 0, n_skip, cost_min)) { f = fc; break; }
+                if (nc <= 1024 && nc <= RW * 32 && nc > n_skip) { f = fc; break; }
             }
             S.frame = f;
         }

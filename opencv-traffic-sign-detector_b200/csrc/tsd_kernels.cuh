@@ -38,9 +38,6 @@
 #ifndef TSD_K2_MINB
 #define TSD_K2_MINB 12           // min resident CTAs per SM of k2_crop_resize_v2 (12 -> 40 registers)
 #endif
-#ifndef TSD_K2_WIDE
-#define TSD_K2_WIDE 1            // K2 general path: aligned 32-bit tap loads + IDP.2A horizontal pass (0: byte loads)
-#endif
 #ifndef TSD_HIST_GROUP_UNROLL
 #define TSD_HIST_GROUP_UNROLL 2  // groups of 4 pixels per lane in flight in the aligned histogram passes (measured at 4096 frames: 1: .922, 2: .921, 3: .934, 4: .953 ms)
 #endif
@@ -300,14 +297,6 @@ __global__ void __launch_bounds__(128) k2_crop_resize_kernel(
 // BGR frames with 4-byte aligned rows (k2_rows_wide), as byte loads otherwise (k2_rows).  Persistent warps stride over the windows.
 // (Variants that lost on B200 -- crop staged in shared memory with cp.async or by TMA, row reuse + staged output, one CTA per
 // frame, L2 prefetch of the ROI -- are documented with their measurements in DESIGN.md section 8.)
-// Which windows the TMA-staged resize kernel takes (tsd_k2_tma.cuh): crops whose byte span, widened to whole 16-byte units in front
-// and 64-byte units in total, and whose rows, in boxes of 8, fit the per-warp staging buffer.  cx = clipped x1, cw / ch = clipped size.
-constexpr int kTmaStageBytes = 10240;
-constexpr int kTmaBoxRows = 8;
-__device__ __forceinline__ bool k2_tma_takes(int cx, int cw, int ch) {
-    const int P = ((cw * 3 + ((cx * 3) & 15) + 63) >> 6) << 6, nops = (ch + kTmaBoxRows - 1) / kTmaBoxRows;
-    return cw > 0 && ch > 0 && P <= 256 && ch <= 64 && P * kTmaBoxRows * nops <= kTmaStageBytes;
-}
 
 // The D destination rows of one window in the general (two-pass 11-bit fixed point) case.  XDC: the second tap sits C bytes after the
 // first in every column (xd1 == C, true for every crop wider than D).  (v0 >> 16) + (v1 >> 16) + 2 is folded into one multiply-add:
@@ -391,8 +380,7 @@ __device__ __forceinline__ void k2_rows_wide(const uint8_t* __restrict__ px, con
     }
 }
 
-// One window by one warp, taps gathered straight from the frame (the body of k2_crop_resize_v2; also the path k2_crop_resize_tma
-// takes for crops that do not fit its staging buffer).  s_y = the warp's 32 x int4 scratch.
+// One window by one warp, taps gathered straight from the frame (the body of k2_crop_resize_v2).  s_y = the warp's 32 x int4 scratch.
 template <int C, int D>
 __device__ __forceinline__ void k2_window_gather(const uint8_t* __restrict__ frames, int H, int W, int64_t row_stride, int64_t frame_stride,
                                                  const int4* __restrict__ coords, const int32_t* __restrict__ win_frame, int w,
@@ -469,7 +457,7 @@ __device__ __forceinline__ void k2_window_gather(const uint8_t* __restrict__ fra
     s_y[lane] = make_int4(yr0 * (int)row_stride, yr1 * (int)row_stride, yb0, yb1);
     __syncwarp();
     // every down-scale (cw > D) has its second tap exactly one pixel to the right in every column: the tap offsets are immediates
-    if (C == 3 && TSD_K2_WIDE && wide_last >= -1 && !(win_frame[w] == wide_last && cy + ch == H)) k2_rows_wide<D>(px, s_y, xa0, xa1, dst, act);
+    if (C == 3 && wide_last >= -1 && !(win_frame[w] == wide_last && cy + ch == H)) k2_rows_wide<D>(px, s_y, xa0, xa1, dst, act);
     else if (__all_sync(0xffffffffu, xd1 == C)) k2_rows<C, D, true>(px, s_y, C, xa0, xa1, dst, act);
     else k2_rows<C, D, false>(px, s_y, xd1, xa0, xa1, dst, act);
 }
@@ -478,19 +466,13 @@ template <int C, int D>
 __global__ void __launch_bounds__(128, TSD_K2_MINB) k2_crop_resize_v2_kernel(
     const uint8_t* __restrict__ frames, int H, int W, int64_t row_stride, int64_t frame_stride,
     const int4* __restrict__ coords, const int32_t* __restrict__ win_frame, const int32_t* __restrict__ n_ptr, int n_max,
-    uint8_t* __restrict__ windows, int out_stride, int skip_tma, int wide_last) {
+    uint8_t* __restrict__ windows, int out_stride, int wide_last) {
     __shared__ int4 s_y[4][32];                              // per warp: (row0, row1, weight0, weight1) of every destination row
     const int wl = threadIdx.x >> 5;
     const int n = n_ptr ? min(*n_ptr, n_max) : n_max;
     const int nwarps = (gridDim.x * blockDim.x) >> 5;
-    for (int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < n; w += nwarps) {     // (the grid normally covers all windows: one trip)
-        if (skip_tma) {                                      // the TMA-staged kernel, launched beside this one, takes the crops that fit its buffer
-            const int4 c = coords[w];
-            const int cx = min(c.x, W), cy = min(c.y, H);
-            if (k2_tma_takes(cx, min(c.z, W) - cx, min(c.w, H) - cy)) continue;
-        }
+    for (int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < n; w += nwarps)     // (the grid normally covers all windows: one trip)
         k2_window_gather<C, D>(frames, H, W, row_stride, frame_stride, coords, win_frame, w, windows, out_stride, s_y[wl], wide_last);
-    }
 }
 
 // =====================================================================================================
@@ -505,10 +487,8 @@ __global__ void __launch_bounds__(128, TSD_K2_MINB) k2_crop_resize_v2_kernel(
 //                device-resident mirror with the frame's own layout, which K2 then reads at HBM speed.
 // The mirror is never cleared: K2 only reads sectors that were marked (and therefore copied) in the same batch.
 // =====================================================================================================
-// gran = sectors per PCIe request unit (1, 2 or 4): the span is widened to whole units of 32 * gran bytes (a read request that
-// fills a whole 128-byte line moves more payload per PCIe packet than four 32-byte ones).
 __global__ void __launch_bounds__(128) stage_mark_kernel(const int4* __restrict__ coords, const int32_t* __restrict__ win_frame,
-                                                         const int32_t* __restrict__ n_ptr, int n_max, int H, int W, int D, int wpr, int gran,
+                                                         const int32_t* __restrict__ n_ptr, int n_max, int H, int W, int D, int wpr,
                                                          uint32_t* __restrict__ bitmap) {
     const int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     const int n = n_ptr ? min(*n_ptr, n_max) : n_max;
@@ -517,7 +497,7 @@ __global__ void __launch_bounds__(128) stage_mark_kernel(const int4* __restrict_
     const int cx = min(c.x, W), cy = min(c.y, H);
     const int cw = min(c.z, W) - cx, ch = min(c.w, H) - cy;
     if (cw <= 0 || ch <= 0) return;
-    const int s0 = ((3 * cx) >> 5) & ~(gran - 1), s1 = min(((3 * (cx + cw) - 1) >> 5) | (gran - 1), ((3 * W + 31) >> 5) - 1);   // first / last 32-byte sector of the row span
+    const int s0 = (3 * cx) >> 5, s1 = (3 * (cx + cw) - 1) >> 5;          // first / last 32-byte sector of the row span
     uint32_t* fb = bitmap + (int64_t)win_frame[w] * H * wpr;
     int rows[2], nrows = 0;
     if (ch <= 2 * D) {                                       // every row of the crop (copy / 2x2 AREA / down-scales up to 2)
@@ -533,8 +513,8 @@ __global__ void __launch_bounds__(128) stage_mark_kernel(const int4* __restrict_
     for (int k = 0; k < nrows; k++) {
         uint32_t* rb = fb + (int64_t)rows[k] * wpr;
         for (int wd = s0 >> 5; wd <= (s1 >> 5); wd++) {
-            const int lo = max(s0, 32 * wd) & 31, hi = min(s1, 32 * wd + 31) & 31;
-            const uint32_t m = (hi == 31 ? 0xffffffffu : ((2u << hi) - 1u)) & ~((1u << lo) - 1u);
+            const int lo = wd == (s0 >> 5) ? s0 & 31 : 0, hi = wd == (s1 >> 5) ? s1 & 31 : 31;     // first / last sector of the span in this word
+            const uint32_t m = (0xffffffffu << lo) & (0xffffffffu >> (31 - hi));
             if ((rb[wd] & m) != m) atomicOr(rb + wd, m);     // (most windows re-mark sectors an overlapping window already set)
         }
     }

@@ -3,15 +3,15 @@
 tsd_create takes a whole tsd_config, and the kernels dispatch on several of its values.  Per window size D = 2 .. 32
 (npx = D * D, ws = 3 npx rounded up to 16 bytes, NW = ceil(npx / 32) mask words):
 
-  K2    k2_crop_resize_v2<3, D> at D = 25 / 32 (and TSD_K2=tma there), the generic kernel at every other D
+  K2    k2_crop_resize_v2<3, D> at D = 25 / 32, the generic kernel at every other D
   K5    k5_hist / launch_folds <640> for npx <= 640 (D <= 25), <1024> above
   K3    k3_masks_v3 (flag tables built in create_impl) for ws <= 2048 (D <= 26), the generic kernel (HsvBounds) above
   K4    k4_score_bits<20> / <32> at NW = 20 / 32 (D = 25, 29 .. 32), k4_score_kernel on the byte masks at every other D
 
   window sizes  per D: tsd_windows, tsd_hist, both tsd_dedup passes, tsd_color_masks, tsd_score_masks (with scores) and tsd_score;
                 the chain on host pointers (score_tol_hundredths = -1: every survivor is a record), on device pointers, with
-                TSD_KEEP_MASKS=1, with TSD_GRAM=0 and (D = 25 / 32) with TSD_K2=tma.  Seeded random templates, one of them
-                degenerate (at most 1 % of the pixels set) and one all set.
+                TSD_KEEP_MASKS=1 and with TSD_GRAM=0.  Seeded random templates, one of them degenerate (at most 1 % of the
+                pixels set) and one all set.
   HSV bounds    an empty band, a band of everything, hue bounds above 179, single values, identical red bands, a blue band
                 overlapping a red one: tsd_color_masks over all 2^24 colours, and the chain at D = 25 / 32 on windows made of
                 colours whose H, S or V is one below, on and one above each bound.
@@ -454,7 +454,7 @@ def test_config_inputs_are_in_their_regimes(oracle):
 
 
 # ---- GPU --------------------------------------------------------------------------------------------------------------
-ENV_KEYS = ("TSD_KEEP_MASKS", "TSD_GRAM", "TSD_K2")
+ENV_KEYS = ("TSD_KEEP_MASKS", "TSD_GRAM")
 
 
 @pytest.fixture
@@ -519,8 +519,8 @@ def test_window_size_stages(oracle, make_ctx, D):
 @pytest.mark.gpu
 @pytest.mark.parametrize("D", DS)
 def test_window_size_chain(oracle, make_ctx, D):
-    """The detection chain at window size D: host pointers (every survivor reported), device pointers, TSD_KEEP_MASKS=1,
-    TSD_GRAM=0 and at D = 25 / 32 TSD_K2=tma.  The stage-by-stage expectation is the oracle's whole-frame restatement."""
+    """The detection chain at window size D: host pointers (every survivor reported), device pointers, TSD_KEEP_MASKS=1 and
+    TSD_GRAM=0.  The stage-by-stage expectation is the oracle's whole-frame restatement."""
     red6, blue6 = templates_for(D)
     frames, boxes, off = sweep_inputs(D)
     all_cfg, tol_cfg = ns(window=D, score_tol_hundredths=-1), ns(window=D)
@@ -529,13 +529,11 @@ def test_window_size_chain(oracle, make_ctx, D):
     assert exp_all[1][2] == exp_all[1][3] > 0 and exp_tol[1][3] < exp_all[1][3]
     runs = [("host", all_cfg, {}, exp_all), ("device", tol_cfg, {}, exp_tol), ("keep_masks", all_cfg, {"TSD_KEEP_MASKS": "1"}, exp_all),
             ("gram0", all_cfg, {"TSD_GRAM": "0"}, exp_all)]
-    if D in (25, 32):
-        runs.append(("device_tma", all_cfg, {"TSD_K2": "tma"}, exp_all))
     bad = []
     for name, cfg, env, (rec, counts) in runs:
         ctx = make_ctx(cfg, env)
         ctx.set_templates(red6, blue6)
-        if name.startswith("device"):
+        if name == "device":
             got = run_device(ctx, frames, boxes, off)
         else:
             det, c = ctx.detect_frames(frames, boxes, off)

@@ -2,12 +2,11 @@
 
 Which kernels handle a frame depends on its window count, on its "big rows" (windows with a histogram bin holding more than 255
 pixels: the tensor-core tiles keep count & 255 and those pairs are corrected exactly from the sparse lists), on the window size and
-on the TSD_GRAM / TSD_FOLD_CTA_COST switches:
+on the TSD_GRAM switch:
 
   producers  k5_pairs (<= 24 windows; frames k5_gram leaves; block pairs k5_gram_big hands over; everything with TSD_GRAM=0)
              k5_gram (25 .. 128 windows, <= 16 big rows), k5_gram_big (129 .. 1024 windows, 128-row block pairs, <= 32 big rows each)
-  folds      k5_fold_warp (<= 256 windows), k5_fold_cta (257 .. 1024; smaller frames by merge cost with TSD_FOLD_CTA_COST),
-             k5_fold (more than 1024 windows)
+  folds      k5_fold_warp (<= 256 windows), k5_fold_cta (257 .. 1024), k5_fold (more than 1024 windows)
 
 The input generator is seeded numpy plus the oracle's BGR -> HSV (no GPU); test_route_inputs_are_in_their_regimes checks on the
 CPU that every case really is in the regime it names, so none of the GPU cases can pass vacuously.  Every GPU case compares
@@ -38,8 +37,7 @@ C_FRAMES = (
 CASES = {"a": tuple((n, {}) for n in A_SIZES), "b": B_FRAMES, "c": C_FRAMES}
 HIST_TOLS = (0.85, 0.6, 0.4)         # histogram pass (long merge chains, merges of merged items at the lower ones)
 CORNER_TOLS = (0.95, 0.6)            # corner pass
-COST_FRAMES = (256, 33, 120)         # (f) frames, windows per frame between: small frames sent to k5_fold_cta by merge cost
-SEEDS = {"a": 101, "b": 102, "c": 103, "cost": 104}
+SEEDS = {"a": 101, "b": 102, "c": 103}
 ROUTE_CLASSES = ((2, 24), (25, 128), (129, 256), (257, 1024), (1025, 1 << 30))     # producer / fold size classes of case a
 BLOCK = 128                          # rows per block of k5_gram_big
 BIG_MAX = 32                         # big rows per block pair k5_gram_big keeps on the tensor cores
@@ -143,18 +141,12 @@ def make_frames(oracle, frames, D, seed):
     return dict(windows=np.stack(wins), coords=np.array(coords, np.int32), offsets=np.array(off, np.int32), big=bigs, D=D)
 
 
-def make_cost_frames(oracle, D):
-    F, lo, hi = COST_FRAMES
-    rng = np.random.default_rng(SEEDS["cost"] * 100 + D)
-    return make_frames(oracle, [(int(rng.integers(lo, hi + 1)), {}) for _ in range(F)], D, SEEDS["cost"])
-
-
 _CASES, _EXPECT = {}, {}
 
 
 def case(oracle, name, D):
     if (name, D) not in _CASES:
-        _CASES[name, D] = make_cost_frames(oracle, D) if name == "cost" else make_frames(oracle, CASES[name], D, SEEDS[name])
+        _CASES[name, D] = make_frames(oracle, CASES[name], D, SEEDS[name])
     return _CASES[name, D]
 
 
@@ -264,17 +256,6 @@ def test_route_inputs_are_in_their_regimes(oracle):
                 h = oracle.hist_normalized(c["windows"][i]).ravel()
                 assert np.array_equal(np.flatnonzero(h), np.flatnonzero(counts[i])), (name, D, i)
                 assert np.argmax(h) == np.argmax(counts[i])
-        # (f) >= 256 frames of 33 .. 120 windows, most of them with merge-band pairs (the cost the CTA-fold routing reads)
-        c = case(oracle, "cost", D)
-        sizes = np.diff(c["offsets"])
-        F, lo, hi = COST_FRAMES
-        assert len(sizes) >= 256 and sizes.min() >= lo and sizes.max() <= hi and sizes.min() > 32
-        merging = 0
-        for s in frame_slices(c):
-            st = np.zeros(3, np.int64)
-            oracle.dedup(c["windows"][s], c["coords"][s], False, 0.85, stats=st)
-            merging += st[2] > 0
-        assert merging >= len(sizes) // 2, merging
 
 
 # ---- GPU: every route against the oracle ----------------------------------------------------------------------------------
@@ -313,19 +294,6 @@ def test_k5_routes_gram_off(tsd, oracle, monkeypatch, D):
             c = case(oracle, name, D)
             for tol in HIST_TOLS:
                 check(_dedup(ctx, c, False, tol), expect(oracle, c, False, tol, name), (name, D, "TSD_GRAM=0", tol))
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("D", (25, 32))
-def test_k5_fold_cta_by_cost(tsd, oracle, monkeypatch, D):
-    """TSD_FOLD_CTA_COST=1 / 4 with 256 frames of 33 .. 120 windows: the frames with that many merge-band pairs go to k5_fold_cta
-    instead of the warp fold; the survivors do not change."""
-    c = case(oracle, "cost", D)
-    for cost in ("1", "4"):
-        monkeypatch.setenv("TSD_FOLD_CTA_COST", cost)
-        with tsd.Context(0, "det" if D == 25 else "rec") as ctx:
-            for tol in (0.85, 0.6):
-                check(_dedup(ctx, c, False, tol), expect(oracle, c, False, tol, "cost"), (D, "TSD_FOLD_CTA_COST", cost, tol))
 
 
 @pytest.mark.gpu

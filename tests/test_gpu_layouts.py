@@ -5,7 +5,6 @@ frame_stride and base pointer, and the layout picks the kernel variant that read
 
   K2 wide       aligned 32-bit tap loads: BGR, base, row_stride, frame_stride all multiples of 4 (D = 25 / 32)
   K2 bytes      byte loads: any other layout, and grey
-  K2 tma        TSD_K2=tma: base and both strides multiples of 16
   K2 generic    any D other than 25 / 32
   staged        page-locked frames, 16-byte legal (base, strides, 3 W): stage_mark -> stage_copy -> device mirror
   gather        page-locked frames otherwise (or TSD_STAGE=0): K2 reads host memory over PCIe
@@ -19,17 +18,17 @@ and tiny ones (1, 5, 16, 21, D - 1, D, D + 1); heights 800, 1, 7, 9 and D +- 1. 
 right or bottom edge, lie wholly outside, end on the last row of the last frame, give exact D x D and 2D x 2D crops at an
 edge, 1-px crops, crops of 33 .. 2D rows and crops taller than 2D.
 
-  per stage   tsd_crop_resize (host / device, C = 3 / 1, D = 25 / 32 / 20, plus TSD_K2=tma) and tsd_windows, bit-exact against
+  per stage   tsd_crop_resize (host / device, C = 3 / 1, D = 25 / 32 / 20) and tsd_windows, bit-exact against
               oracle.crop_resize / expand_boxes; strides below the minimum refused by every entry point.
-  chain       RUN_DETECT and RUN_RECOGNIZE through device pointers (and tma), pageable chunks, staging at TSD_STAGE_GRAN =
-              32 / 64 / 128 and in chunks, TSD_STAGE=0 and TSD_ZEROCOPY=0: records and stage counts equal the oracle's, the
-              staged byte count equals the marking rule restated in numpy, and the mirrors hold other pixels first (poison).
+  chain       RUN_DETECT and RUN_RECOGNIZE through device pointers, pageable chunks, staging in one batch and in chunks,
+              TSD_STAGE=0 and TSD_ZEROCOPY=0: records and stage counts equal the oracle's, the staged byte count equals the
+              marking rule restated in numpy, and the mirrors hold other pixels first (poison).
   det_cap     TSD_E_NOMEM with *ndet and the counts filled on the unchunked, pageable-chunked and staged-chunked routes.
   preprocess  host / device, contiguous / strided, tiles (1,1) (8,8) (3,5) (16,2) and larger than the image, H or W = 1, 2,
               3, (3, 300), 4K, clip 0 / 0.01 / 2 / 40, gamma 1 / 2 / 0.5 and a caller's table; more than 65 535 frames.
 
 test_layout_inputs_are_in_their_regimes checks on the CPU that every route row is reached at both D, that every box class
-occurs and that the staged-byte model marks half sectors and granules clamped at the row end.
+occurs and that the staged-byte model marks half sectors.
 """
 import ctypes as C
 import functools
@@ -47,18 +46,18 @@ MODES = {"det": 25, "rec": 32}
 
 # name: (H, W, row_stride, frame_stride, base offset).  (frame_stride None = the minimum, row_stride * (H - 1) + 3 W.)
 LAYOUTS = {
-    "1360_contiguous":  (800, 1360, 4080, 4080 * 800, 0),          # all %16: staged, tma, wide; half last sector
+    "1360_contiguous":  (800, 1360, 4080, 4080 * 800, 0),          # all %16: staged, wide; half last sector
     "1360_padded":      (800, 1360, 4096, 4096 * 800 + 32, 16),    # all %16 with padding
     "1366_odd":         (800, 1366, 4101, 4101 * 800 + 3, 1),      # nothing %4: bytes, gather
     "1366_contiguous":  (800, 1366, 4098, 4098 * 800, 0),          # 3 W % 4 = 2: bytes
-    "1376_rs4":         (7, 1376, 4132, 4132 * 7, 4),              # rs, fs, base %4 only: wide, no tma, gather
+    "1376_rs4":         (7, 1376, 4132, 4132 * 7, 4),              # rs, fs, base %4 only: wide, gather
     "1376_minimal":     (7, 1376, 4160, None, 16),                 # 3 W % 32 = 0, minimal frame_stride (29 088, %16 = 0): staged
     "1360_rs16x4":      (9, 1360, 4084, 4084 * 9 + 12, 16),        # only rs %16 = 4
     "1360_fs16x8":      (9, 1360, 4096, 4096 * 9 + 8, 16),         # only fs %16 = 8
     "1360_base4":       (9, 1360, 4096, 4096 * 9, 4),              # only base %16 = 4
     "1360_base1":       (9, 1360, 4096, 4096 * 9, 1),              # only base %4 = 1
     "1360_h1":          (1, 1360, 4083, 4085, 0),                  # one row; rs %4 = 3
-    "w1_h26":           (26, 1, 16, 16 * 26, 16),                  # %16 everywhere but 3 W = 3: tma, wide, gather
+    "w1_h26":           (26, 1, 16, 16 * 26, 16),                  # %16 everywhere but 3 W = 3: wide, gather
     "w5_h24":           (24, 5, 20, None, 4),                      # fs = 475
     "w16_h33":          (33, 16, 48, 48 * 33, 0),                  # 3 W = 48: staged
     "w21_h31":          (31, 21, 63, 63 * 31, 1),
@@ -71,13 +70,9 @@ LAYOUTS = {
 }
 ROUTES = {                            # name: (memory, environment)
     "device":        ("device", {}),
-    "device_tma":    ("device", {"TSD_K2": "tma"}),
     "pageable":      ("pageable", {"TSD_CHUNK_FRAMES": "2"}),
-    "staged32":      ("pinned", {"TSD_STAGE_GRAN": "32", "TSD_STAGE_CHUNK": "0"}),
-    "staged64":      ("pinned", {"TSD_STAGE_GRAN": "64", "TSD_STAGE_CHUNK": "0"}),
-    "staged128":     ("pinned", {"TSD_STAGE_GRAN": "128", "TSD_STAGE_CHUNK": "0"}),
+    "staged":        ("pinned", {"TSD_STAGE_CHUNK": "0"}),
     "staged_chunks": ("pinned", {"TSD_STAGE_CHUNK": "2"}),
-    "staged_tma":    ("pinned", {"TSD_K2": "tma", "TSD_STAGE_CHUNK": "0"}),
     "gather":        ("pinned", {"TSD_STAGE": "0"}),
     "zerocopy_off":  ("pinned", {"TSD_ZEROCOPY": "0"}),
 }
@@ -240,18 +235,13 @@ def windows_of(name, D):
 
 
 # ---- the staged-byte model: stage_mark + stage_copy restated ----------------------------------------------------------
-def staged_bytes(name, D, gran):
-    """-> (bytes one batch stages, number of half sectors copied, number of spans clamped at the row end)."""
+def staged_bytes(name, D):
+    """-> (bytes one batch stages, number of half sectors copied)."""
     H, W = LAYOUTS[name][:2]
     _, fr, cl = windows_of(name, D)
-    g = gran // 32
-    last = (3 * W + 31) // 32 - 1
-    sectors, clamped = set(), 0
+    sectors = set()
     for f, (cx, cy, cw, ch) in zip(fr.tolist(), cl.tolist()):
-        s0 = ((3 * cx) >> 5) & ~(g - 1)
-        s1u = ((3 * (cx + cw) - 1) >> 5) | (g - 1)
-        s1 = min(s1u, last)
-        clamped += s1u > last
+        s0, s1 = (3 * cx) >> 5, (3 * (cx + cw) - 1) >> 5
         if ch <= 2 * D:
             rows = range(cy, cy + ch)
         else:
@@ -267,7 +257,7 @@ def staged_bytes(name, D, gran):
         b = min(32, 3 * W - 32 * s) & ~15
         nbytes += b
         half += b == 16
-    return nbytes, half, clamped
+    return nbytes, half
 
 
 def stages(name, route):
@@ -297,8 +287,6 @@ def k2_rows(name, route, D):
         else:
             rows.add("pageable_chunked" if int(env.get("TSD_CHUNK_FRAMES", "32")) < F else "pageable")
     rows.add("wide" if b % 4 == 0 and rs % 4 == 0 and fs % 4 == 0 else "bytes")
-    if env.get("TSD_K2") == "tma" and b % 16 == 0 and rs % 16 == 0 and fs % 16 == 0:
-        rows.add("tma")
     return rows
 
 
@@ -391,7 +379,7 @@ def test_layout_inputs_are_in_their_regimes(oracle, det_expected):
         for route in ROUTES:
             for name in LAYOUTS:
                 rows |= k2_rows(name, route, D)
-        assert rows >= {"wide", "bytes", "tma", "staged", "staged_chunks", "gather_unaligned", "gather_stage0",
+        assert rows >= {"wide", "bytes", "staged", "staged_chunks", "gather_unaligned", "gather_stage0",
                         "pageable_chunked"}, (D, rows)
     # every box class, at both D
     for D in FLAVOURS:
@@ -401,15 +389,13 @@ def test_layout_inputs_are_in_their_regimes(oracle, det_expected):
                 tot[k] += v
         assert all(v > 0 for v in tot.values()), (D, tot)
         assert sum(box_classes(name, D)["last_row_last_frame"] > 0 for name in LAYOUTS) >= len(LAYOUTS) - 2
-    # the staged-byte model: half sectors and granules clamped at the row end both occur on staged layouts
-    staged = [n for n in LAYOUTS if stages(n, "staged32")]
+    # the staged-byte model: half sectors occur on staged layouts
+    staged = [n for n in LAYOUTS if stages(n, "staged")]
     assert len(staged) >= 5
     for D in FLAVOURS:
-        assert sum(staged_bytes(n, D, 32)[1] for n in staged) > 0
-        assert sum(staged_bytes(n, D, g)[2] for n in staged for g in (64, 128)) > 0
+        assert sum(staged_bytes(n, D)[1] for n in staged) > 0
         for n in staged:
-            b32, b64, b128 = (staged_bytes(n, D, g)[0] for g in (32, 64, 128))
-            assert 0 < b32 <= b64 <= b128, n
+            assert staged_bytes(n, D)[0] > 0, n
     # the chain's expectations have detections on big frames and every recognition label
     det = det_expected
     assert sum(len(det[n][0]) for n in LAYOUTS) > 20
@@ -479,7 +465,7 @@ def make_ctx(tsd, monkeypatch):
     made = []
 
     def mk(flavour="det", env=None):
-        for k in ("TSD_K2", "TSD_STAGE", "TSD_STAGE_GRAN", "TSD_STAGE_CHUNK", "TSD_CHUNK_FRAMES", "TSD_ZEROCOPY"):
+        for k in ("TSD_STAGE", "TSD_STAGE_CHUNK", "TSD_CHUNK_FRAMES", "TSD_ZEROCOPY"):
             monkeypatch.delenv(k, raising=False)
         for k, v in (env or {}).items():
             monkeypatch.setenv(k, v)
@@ -506,14 +492,11 @@ def _crop_expect(oracle, name, C, D):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("tma", (False, True))
-def test_crop_resize_layouts(oracle, make_ctx, tma):
+def test_crop_resize_layouts(oracle, make_ctx):
     """tsd_crop_resize on every layout, host and device pointers, C = 3 / 1, D = 25 / 32 / 20, against oracle.crop_resize on the
-    contiguous frame.  Device calls add crops that are empty after clipping: their windows must be all zero.  With TSD_K2=tma the
-    TMA kernel runs only at D = 32 here: tsd_crop_resize writes packed windows, and the 1 875-byte stride of D = 25 is not a
-    multiple of 16.  The chain routes (internal 16-byte window stride) run it at D = 25."""
+    contiguous frame.  Device calls add crops that are empty after clipping: their windows must be all zero."""
     A = _lib()
-    ctx = make_ctx("det", {"TSD_K2": "tma"} if tma else {})
+    ctx = make_ctx("det")
     bad = []
     for name in LAYOUTS:
         for Cn in (3, 1):
@@ -637,7 +620,6 @@ def test_chain_layouts(oracle, templates, det_expected, make_ctx, mode, route):
         Wl, bl, exp_all = expected_rec(oracle)
         ctx.set_lda(Wl, bl)
         run_mode = A.RUN_RECOGNIZE
-    gran = int(env.get("TSD_STAGE_GRAN", "32"))
     bad = []
     for name in LAYOUTS:
         boxes, off = boxes_for(name, D)
@@ -673,7 +655,7 @@ def test_chain_layouts(oracle, templates, det_expected, make_ctx, mode, route):
             finally:
                 ctx.unpin(canvas)
             got = _records(det)
-            want = staged_bytes(name, D, gran)[0] if stages(name, route) else 0
+            want = staged_bytes(name, D)[0] if stages(name, route) else 0
             if staged != want:
                 bad.append((name, "staged bytes", staged, want))
         if got != exp or gcounts != list(ecounts):
@@ -683,7 +665,7 @@ def test_chain_layouts(oracle, templates, det_expected, make_ctx, mode, route):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("route", ("staged32", "staged_chunks", "pageable", "device"))
+@pytest.mark.parametrize("route", ("staged", "staged_chunks", "pageable", "device"))
 def test_det_cap(oracle, make_ctx, route):
     """det_cap = 0 and n - 1: TSD_E_NOMEM with *ndet = n and the counts filled in (summed over chunks); det_cap = n: the oracle's
     records; the next call on the same context is still right."""

@@ -14,12 +14,3 @@ for lib in "" build/libtsd_*.so; do
   [ -n "$REC" ] && TSD_LIB=${lib:+$PWD/$lib} python tools/prof_step.py --mode rec --frames 1024 --steps 5 --times 2>&1 | tail -2 | head -1 >> gpurun_out/$N.log
 done
 cat gpurun_out/$N.tests.log gpurun_out/$N.log 2>/dev/null
-if [ -n "$FOLDCOST" ]; then
-  for cst in $FOLDCOST; do
-    echo "== default lib, TSD_FOLD_CTA_COST=$cst" >> gpurun_out/$N.log
-    TSD_FOLD_CTA_COST=$cst python tools/prof_step.py --frames 4096 --steps 5 --times 2>&1 | tail -2 | head -1 >> gpurun_out/$N.log
-    TSD_FOLD_CTA_COST=$cst python tools/prof_step.py --frames 4096 --steps 10 --wall 2>&1 | head -1 >> gpurun_out/$N.log
-    TSD_FOLD_CTA_COST=$cst python tools/prof_step.py --mode rec --frames 1024 --steps 5 --times 2>&1 | tail -2 | head -1 >> gpurun_out/$N.log
-  done
-  tail -n $((4 * $(echo $FOLDCOST | wc -w))) gpurun_out/$N.log
-fi

@@ -1,5 +1,5 @@
 """e2e timing of Context.detect_frames (host pinned frames -> H2D -> chain -> D2H records).
-Environment: TSD_STAGE (0 = K2 gathers from host memory itself), TSD_STAGE_GRAN (32 | 64 | 128), TSD_ZEROCOPY, TSD_CHUNK_FRAMES."""
+Environment: TSD_STAGE (0 = K2 gathers from host memory itself), TSD_STAGE_CHUNK, TSD_STAGE_CTAS, TSD_ZEROCOPY, TSD_CHUNK_FRAMES."""
 import argparse, os, sys, time
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -29,6 +29,6 @@ ctx.set_profiling(True)
 ctx.detect_frames(hf, boxes, off)
 print({k: round(v, 3) for k, v in ctx.stage_times()})
 ctx.set_profiling(False)
-print("stage=%s gran=%s zerocopy=%s frames=%d ms=%.2f windows/s=%.2fM staged=%.1f MB (%.1f GB/s) counts=%s" % (
-    os.environ.get("TSD_STAGE", "1"), os.environ.get("TSD_STAGE_GRAN", "32"), os.environ.get("TSD_ZEROCOPY", "1"), a.frames, dt * 1e3,
+print("stage=%s zerocopy=%s frames=%d ms=%.2f windows/s=%.2fM staged=%.1f MB (%.1f GB/s) counts=%s" % (
+    os.environ.get("TSD_STAGE", "1"), os.environ.get("TSD_ZEROCOPY", "1"), a.frames, dt * 1e3,
     a.frames * 200 / dt / 1e6, staged / 1e6, staged / dt / 1e9, counts.tolist()))
