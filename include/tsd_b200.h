@@ -20,6 +20,10 @@
  *     bytes between rows; boxes int32 [n][4] = (x, y, w, h) as produced by cv2.MSER.detectRegions()[1];
  *     coords int32 [n][4] = (x1, y1, x2, y2); windows uint8 [n][D][D][3]; *_offsets int32 [nframes+1]
  *     (CSR: items of frame f are offsets[f] .. offsets[f+1]-1, in the reference's list order).
+ *   - size limits: counts of frames, boxes, windows and items are int32 (byte sizes and offsets past 4 GiB are fine).  One frame
+ *     must span less than 2 GiB (row_stride * H < 2^31; TSD_E_INVALID otherwise).  A batch of tsd_detect_frames /
+ *     tsd_enqueue_frames / tsd_dedup has fewer than 2^23 frames (TSD_E_INVALID otherwise, before any device work; pageable host
+ *     frames run in chunks, so only each chunk counts).  tsd_bgr2gray and tsd_bgr2hsv take any int64 pixel count.
  */
 #ifndef TSD_B200_H
 #define TSD_B200_H

@@ -873,6 +873,7 @@ int tsd_dedup(tsd_ctx* c, const uint8_t* windows, const int32_t* coords, const i
               double tol, uint8_t* out_windows, int32_t* out_coords, int32_t* out_offsets, int32_t* total_out, int mem) {
     if (!c || !offsets || !out_offsets || nframes < 0 || D < 2 || D > kMaxD) return fail(TSD_E_INVALID, "bad argument");
     if (mem != TSD_MEM_HOST) return fail(TSD_E_INVALID, "tsd_dedup takes host pointers; use tsd_enqueue_frames for device-resident batches");
+    if (nframes >= kMaxBatchFrames) return fail(TSD_E_INVALID, "%d frames: a batch holds fewer than 2^23 (the K5 work lists keep frame << 8 in an int32)", nframes);
     CU(cudaSetDevice(c->device));
     const int n = offsets[nframes], npx = D * D, nbytes = npx * 3, ws = win_stride(npx, 3), es = ent_stride(npx);
     if (n && (!windows || !coords)) return fail(TSD_E_INVALID, "NULL argument");
@@ -1169,16 +1170,20 @@ int tsd_score(tsd_ctx* c, const uint8_t* windows, int n, int D, int32_t* id, int
 }
 
 int tsd_bgr2gray(tsd_ctx* c, const uint8_t* bgr, int64_t npx, uint8_t* gray, int mem) {
-    if (!c || npx < 0 || npx > 0x7fffffffLL || (npx && (!bgr || !gray))) return fail(TSD_E_INVALID, "bad argument");
+    if (!c || npx < 0 || (npx && (!bgr || !gray))) return fail(TSD_E_INVALID, "bad argument");
     CU(cudaSetDevice(c->device));
     if (npx == 0) return TSD_OK;
     Stage s(c);
     void *di = (void*)bgr, *dout = gray;
     if (mem == TSD_MEM_HOST) { TRY(s.in(bgr, (size_t)npx * 3, &di)); TRY(s.alloc(&dout, (size_t)npx)); }
-    int grid = cdiv(npx, 256);
-    if (grid > c->sm_count * 32) grid = c->sm_count * 32;
-    k6_gray_kernel<<<grid, 256, 0, c->cur>>>((uint8_t*)di, nullptr, nullptr, 1, (int)npx, 0, (uint8_t*)dout);
-    TRY(check_launch(c, "k6_gray"));
+    // K6 counts pixels in int (the chain's windows): one launch per range of at most 2^30 pixels, from offset pointers
+    for (int64_t p0 = 0; p0 < npx; p0 += (int64_t)1 << 30) {
+        const int m = (int)std::min<int64_t>(npx - p0, (int64_t)1 << 30);
+        int grid = cdiv(m, 256);
+        if (grid > c->sm_count * 32) grid = c->sm_count * 32;
+        k6_gray_kernel<<<grid, 256, 0, c->cur>>>((uint8_t*)di + p0 * 3, nullptr, nullptr, 1, m, 0, (uint8_t*)dout + p0);
+        TRY(check_launch(c, "k6_gray"));
+    }
     if (mem == TSD_MEM_HOST) { TRY(s.out(gray, dout, (size_t)npx)); CU(cudaStreamSynchronize(c->stream)); }
     return TSD_OK;
 }
@@ -1242,7 +1247,7 @@ int tsd_recognize(tsd_ctx* c, const uint8_t* windows, int n, double tol, int32_t
     TRY(s.alloc(&dg, (size_t)n * 1024)); TRY(s.alloc(&dh, (size_t)n * TSD_HOG_LEN * 4)); TRY(s.alloc(&dl, (size_t)n * 4));
     int grid = cdiv((int64_t)n * 1024, 256);
     if (grid > c->sm_count * 32) grid = c->sm_count * 32;
-    k6_gray_kernel<<<grid, 256, 0, c->cur>>>((uint8_t*)dw, nullptr, nullptr, 1, n * 1024, 0, (uint8_t*)dg);
+    k6_gray_kernel<<<grid, 256, 0, c->cur>>>((uint8_t*)dw, nullptr, nullptr, n, 1024, 3072, (uint8_t*)dg);      // as in the chain: n windows of 1024 px
     TRY(check_launch(c, "k6_gray"));
     int hgrid = cdiv(n, kHogWarps);
     if (hgrid > c->sm_count * 8) hgrid = c->sm_count * 8;
@@ -1494,6 +1499,7 @@ static int enqueue_impl(tsd_ctx* c, int mode, const uint8_t* d_frames, int nfram
     if (!c || !d_frames || !d_box_offsets || nframes < 1 || nb < 0 || H < 1 || W < 1) return fail(TSD_E_INVALID, "bad argument");
     if (mode != TSD_RUN_DETECT && mode != TSD_RUN_RECOGNIZE) return fail(TSD_E_INVALID, "bad mode %d", mode);
     if (row_stride < (int64_t)W * 3 || frame_stride < row_stride * (H - 1) + (int64_t)W * 3) return fail(TSD_E_INVALID, "bad strides");
+    if (nframes >= kMaxBatchFrames) return fail(TSD_E_INVALID, "%d frames: a batch holds fewer than 2^23 (the K5 work lists keep frame << 8 in an int32)", nframes);
     const int D = c->cfg.window, npx = D * D, ws = win_stride(npx, 3), es = ent_stride(npx);
     const int ms = (npx + 15) & ~15, NW = (npx + 31) >> 5;
     if (mode == TSD_RUN_DETECT && (!c->have_templates || c->tmpl_D != D)) return fail(TSD_E_STATE, "templates not set for D=%d", D);

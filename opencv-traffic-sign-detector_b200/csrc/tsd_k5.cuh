@@ -35,6 +35,9 @@ constexpr int kGramCbWords = (kGramChunks + 1) / 2;
 constexpr int kEnergyRows = kHistGroups + kGramCbWords;   // rows of the [rows][windows] energy block
 static_assert(kGramKC % 32 == 0 && kEnergyRows <= 32, "chunk boundaries");
 constexpr int kClsUnsure = 3;
+// The todo work lists of k5_gram / k5_gram_big / k5_pairs keep (frame << 8) | (I << 4) | J in an int32: the batch entry points
+// (tsd_enqueue_frames and the chains behind it, tsd_dedup) refuse batches of kMaxBatchFrames frames or more.
+constexpr int kMaxBatchFrames = 1 << 23;
 constexpr int kGramBM = 128;                           // windows per frame k5_gram handles / rows per block of k5_gram_big
 // Statistics: pairs whose integer-dot classification came within 2e-6 of a threshold and were decided by the exact f64 evaluation
 // (tsd_stat_unsure_pairs; the tests use it to prove that path is exercised).  Rare, so the atomic costs nothing.
