@@ -124,7 +124,7 @@ TSD_API int tsd_set_templates(tsd_ctx *ctx, const uint8_t *red6, const uint8_t *
 TSD_API int tsd_set_similarity_table(tsd_ctx *ctx, const double *f, int n);
 /* Six binary LDA classifiers: W f64 [nfeat][6] (column c = classifiers[c].coef_[0]), b f64 [6] (intercept_),
  * REC/source.py:551-562 fit on the host with scikit-learn.  nfeat = 1..4096 (324 for HOG, 1024 for raw grey pixels; the
- * chain needs 324).  K8 keeps W in shared memory, nfeat * 48 B: 192 KB at 4096 features; TSD_E_INVALID if the device
+ * chain takes 324 or, with TSD_REC_GRAY, 1 024).  K8 keeps W in shared memory, nfeat * 48 B: 192 KB at 4096 features; TSD_E_INVALID if the device
  * cannot give a block that much. */
 TSD_API int tsd_set_lda(tsd_ctx *ctx, const double *W, const double *b, int nfeat);
 /* 7-class LDA reducer + KNN training set: xbar f64 [nfeat], scalings f64 [nfeat][6], Ztrain f64 [ntrain][6],
@@ -229,8 +229,9 @@ TSD_API int tsd_recognize(tsd_ctx *ctx, const uint8_t *windows, int n, double to
 TSD_API int tsd_lda_predict_tf32(tsd_ctx *ctx, const float *X, int n, double tol, int split, float *logits, int32_t *labels, float *ms, int mem);
 
 /* K8b predictProbabilityKNNClassifiers (REC/source.py:592-596): Z f64 [n][6] (may be NULL), labels int32 [n].
- * Brute force over the training set; training rows at equal distance are ranked by index (the smaller one is nearer), then a
- * uniform vote with ties to the smallest label.  scikit-learn's kd-tree orders exact distance ties its own way, so labels can
+ * Brute force over the training set (tiles of it in shared memory, one thread per query; below about one 128-query block per SM the
+ * training set is also split across blocks and the partial lists merged); training rows at equal distance are ranked by index
+ * (the smaller one is nearer), then a uniform vote with ties to the smallest label.  scikit-learn's kd-tree orders exact distance ties its own way, so labels can
  * differ from it when a tie straddles the k-th neighbour (SURVEY A.8). */
 TSD_API int tsd_knn_predict(tsd_ctx *ctx, const float *X, int n, double *Z, int32_t *labels, int mem);
 
@@ -246,11 +247,22 @@ typedef struct tsd_detection {
 
 #define TSD_RUN_DETECT 1       /* K1 K2 K5 K5 K3 K4  (DET main.py path) */
 #define TSD_RUN_RECOGNIZE 2    /* K1 K2 K5 K5 K6 K7 K8 on the recognition flavour (x1.15, 32x32) */
+/* Classifier modifiers, OR-ed into TSD_RUN_RECOGNIZE (REC/constants.py:10-12: HOG or GRAY descriptors, LDABAYES or KNN).
+ * TSD_RUN_RECOGNIZE alone is HOG + LDA.
+ *   TSD_REC_GRAY  the descriptor is the 1 024 raw grey pixels of the 32x32 window (REC/source.py:520-521): K7 is skipped.
+ *   TSD_REC_KNN   the label comes from the tsd_set_knn model (its reducer, training set and k): projection, k nearest
+ *                 neighbours and a uniform vote (REC/source.py:592-596); proba_tol is not used.  Training rows at equal
+ *                 distance rank by index, the smaller one nearer, and vote ties go to the smallest label (SURVEY.md A.8).
+ * A survivor becomes a record when its label is not 0, with hundredths = 0.  State (TSD_E_STATE, before any device work):
+ * D = 32; LDA needs tsd_set_lda weights of 324 features (HOG) or 1 024 (GRAY), KNN a tsd_set_knn reducer of the same size.
+ * A modifier with TSD_RUN_DETECT, or any other bit, is TSD_E_INVALID. */
+#define TSD_REC_GRAY 4
+#define TSD_REC_KNN 8
 
 /* The whole post-MSER chain for a batch of frames (SURVEY.md section 3.4):
  * MSERTrafficSignDetector's candidate loop + both cleanDuplicatedDetections passes (DET/source.py:116-131), then
  * detectionsMaskCorrelation for every survivor (DET/source.py:708-716)  [TSD_RUN_DETECT], or
- * BGR2GRAY + HOG + LDA decision [TSD_RUN_RECOGNIZE].
+ * BGR2GRAY + HOG or GRAY descriptors + LDA or KNN decision [TSD_RUN_RECOGNIZE | TSD_REC_*].
  * det [det_cap] receives the records in frame order then list order; counts int32 [4] (may be NULL) receives
  * {raw boxes, aspect-passing windows, survivors, detections}.  Returns TSD_E_NOMEM if det_cap is too small.
  * With TSD_MEM_DEVICE the frames/boxes are device memory, `det`/`counts` are still HOST pointers and the call
@@ -289,7 +301,8 @@ TSD_API int tsd_stat_staged_bytes(tsd_ctx *ctx, int64_t *total, int reset);
 
 /* Device-side stage timing: CUDA events are recorded between the stages of every tsd_enqueue_frames call made after
  * tsd_set_profiling(ctx, 1); tsd_stage_times synchronises and returns, per stage name, the time summed over those
- * calls (names[i] / ms[i] for i < returned count). */
+ * calls (names[i] / ms[i] for i < returned count).  Recognition stages: k6_gray, k7_hog (absent with TSD_REC_GRAY), then k8_lda
+ * or, with TSD_REC_KNN, k8_knn (projection + top-k + vote). */
 TSD_API int tsd_set_profiling(tsd_ctx *ctx, int on);
 TSD_API int tsd_stage_times(tsd_ctx *ctx, const char **names, float *ms, int cap);
 /* tsd_set_profiling(ctx, 2) keeps consecutive tsd_enqueue_frames calls overlapped (two scratch slots, two streams) and

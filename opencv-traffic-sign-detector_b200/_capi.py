@@ -14,6 +14,7 @@ LIB_PATH = os.environ.get("TSD_LIB") or os.path.join(_PKG, "libtsd_b200.so")    
 
 MEM_HOST, MEM_DEVICE = 0, 1
 RUN_DETECT, RUN_RECOGNIZE = 1, 2
+REC_GRAY, REC_KNN = 4, 8              # classifier modifiers OR-ed into RUN_RECOGNIZE (HOG + LDA without them)
 HOG_LEN = 324
 
 

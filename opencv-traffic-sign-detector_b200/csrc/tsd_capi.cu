@@ -96,7 +96,8 @@ struct tsd_ctx {
     HogConst hog;
     // grow-only scratch
     DevBuf b_coords, b_winframe, b_windows, b_entries, b_meta, b_list, b_flags, b_cnt, b_winoff, b_survcnt, b_survoff,
-        b_slots, b_pairs, b_energy, b_red, b_blue, b_bits, b_id, b_hund, b_emit, b_detcnt, b_detoff, b_det, b_gray, b_hog, b_labels, b_scores;
+        b_slots, b_pairs, b_energy, b_red, b_blue, b_bits, b_id, b_hund, b_emit, b_detcnt, b_detoff, b_det, b_gray, b_hog, b_labels, b_scores,
+        b_knnz, b_knnpd, b_knnpi;
     int last_mode = 0;
     int profiling = 0;
     int keep_masks = 0;                      // TSD_KEEP_MASKS=1: the chain also writes K3's byte masks (nobody reads them there)
@@ -350,7 +351,7 @@ int tsd_destroy(tsd_ctx* c) {
     for (int i = 0; i < 2; i++) if (c->os[i]) cudaStreamSynchronize(c->os[i]);
     DevBuf* bufs[] = {&c->b_coords, &c->b_winframe, &c->b_windows, &c->b_entries, &c->b_meta, &c->b_list, &c->b_flags, &c->b_cnt,
                       &c->b_winoff, &c->b_survcnt, &c->b_survoff, &c->b_slots, &c->b_pairs, &c->b_energy, &c->b_red, &c->b_blue, &c->b_bits, &c->b_id, &c->b_hund,
-                      &c->b_emit, &c->b_detcnt, &c->b_detoff, &c->b_det, &c->b_gray, &c->b_hog, &c->b_labels, &c->b_scores,
+                      &c->b_emit, &c->b_detcnt, &c->b_detoff, &c->b_det, &c->b_gray, &c->b_hog, &c->b_labels, &c->b_scores, &c->b_knnz, &c->b_knnpd, &c->b_knnpi,
                       &c->b_stage[0], &c->b_stage[1], &c->b_hboxes, &c->b_hoff, &c->b_summary, &c->b_order, &c->b_gramdone, &c->b_mirror[0], &c->b_mirror[1], &c->b_stagemap[0], &c->b_stagemap[1], &c->b_pgray, &c->b_pluts, &c->b_pin, &c->b_pout};
     for (DevBuf* b : bufs) if (b->p) cudaFree(b->p);
     for (int i = 0; i < 2; i++) {
@@ -524,7 +525,8 @@ int tsd_set_lda(tsd_ctx* c, const double* W, const double* b, int nfeat) {
     if (!c || !W || !b || nfeat < 1 || nfeat > 4096) return fail(TSD_E_INVALID, "bad argument");
     CU(cudaSetDevice(c->device));
     // k8_lda_kernel stages W in dynamic shared memory: nfeat * 48 B, 192 KB at 4096 features (above 48 KB it needs the opt-in)
-    TRY(allow_dynamic_smem(c, (const void*)k8_lda_kernel, (size_t)nfeat * 6 * sizeof(double), "k8_lda"));
+    TRY(allow_dynamic_smem(c, (const void*)k8_lda_kernel<float>, (size_t)nfeat * 6 * sizeof(double), "k8_lda"));
+    TRY(allow_dynamic_smem(c, (const void*)k8_lda_kernel<uint8_t>, (size_t)nfeat * 6 * sizeof(double), "k8_lda"));
     TRY(join_pending(c));
     CU(cudaStreamSynchronize(c->stream));
     if (c->d_ldaW) cudaFree(c->d_ldaW);
@@ -542,7 +544,7 @@ int tsd_set_knn(tsd_ctx* c, const double* xbar, const double* scalings, int nfea
                 int ntrain, int k) {
     if (!c || !xbar || !scalings || !Ztrain || !ytrain || nfeat < 1 || ntrain < 1 || k < 1 || k > kKnnMaxK)
         return fail(TSD_E_INVALID, "bad argument (k must be 1..%d)", kKnnMaxK);
-    for (int t = 0; t < ntrain; t++)                         // k8_knn_kernel votes into 16 label counters
+    for (int t = 0; t < ntrain; t++)                         // the k-NN vote counts into 16 label counters
         if (ytrain[t] < 0 || ytrain[t] >= kKnnMaxLabels)
             return fail(TSD_E_INVALID, "ytrain[%d] = %d, labels must be 0..%d", t, ytrain[t], kKnnMaxLabels - 1);
     CU(cudaSetDevice(c->device));
@@ -1205,12 +1207,17 @@ int tsd_hog(tsd_ctx* c, const uint8_t* gray, int n, float* desc, int mem) {
     return TSD_OK;
 }
 
-static int dev_lda(tsd_ctx* c, const float* X, const int32_t* n_ptr, int n_max, double tol, double* logits, int32_t* labels) {
+}  // extern "C"
+
+template <typename T>
+static int dev_lda(tsd_ctx* c, const T* X, const int32_t* n_ptr, int n_max, double tol, double* logits, int32_t* labels) {
     int grid = cdiv((int64_t)n_max * 32, 256);
     if (grid > c->sm_count * 8) grid = c->sm_count * 8;
-    k8_lda_kernel<<<grid, 256, (size_t)c->lda_nfeat * 6 * sizeof(double), c->cur>>>(X, n_ptr, n_max, c->lda_nfeat, c->d_ldaW, c->d_ldab, tol, logits, labels);
+    k8_lda_kernel<T><<<grid, 256, (size_t)c->lda_nfeat * 6 * sizeof(double), c->cur>>>(X, n_ptr, n_max, c->lda_nfeat, c->d_ldaW, c->d_ldab, tol, logits, labels);
     return check_launch(c, "k8_lda");
 }
+
+extern "C" {
 
 int tsd_lda_predict(tsd_ctx* c, const float* X, int n, double tol, double* logits, int32_t* labels, int mem) {
     if (!c || n < 0 || (n && (!X || !labels))) return fail(TSD_E_INVALID, "bad argument");
@@ -1296,21 +1303,72 @@ int tsd_lda_predict_tf32(tsd_ctx* c, const float* X, int n, double tol, int spli
     return TSD_OK;
 }
 
+}  // extern "C"
+
+// K8b's split of the training set: a batch of fewer than one kKnnThreads-query CTA per SM also splits the training rows across about
+// 2 * sm_count / (query CTAs) CTAs, in whole tiles.  Decided from the host-side query bound n_max.  Then nsplit * n_max stays below
+// 3 * sm_count * kKnnThreads, which bounds the partial lists (knn_part_entries).
+static int knn_splits(const tsd_ctx* c, int n_max, int* rows_per_split) {
+    const int qblocks = cdiv(n_max, kKnnThreads), ntiles = cdiv(c->knn_ntrain, kKnnTile);
+    int nsplit = qblocks >= c->sm_count ? 1 : std::min(ntiles, cdiv(2 * c->sm_count, std::max(qblocks, 1)));
+    const int tiles = cdiv(ntiles, nsplit);
+    *rows_per_split = tiles * kKnnTile;
+    return cdiv(ntiles, tiles);
+}
+static size_t knn_part_entries(const tsd_ctx* c) { return (size_t)3 * c->sm_count * kKnnThreads * kKnnMaxK; }
+
+template <int K>
+static int launch_knn_topk(tsd_ctx* c, const double* Z, const int32_t* n_ptr, int n_max, int nsplit, int rows_per_split,
+                           double* part_d, int32_t* part_i, int32_t* labels) {
+    k8_knn_topk_kernel<K><<<dim3(std::max(1, cdiv(n_max, kKnnThreads)), nsplit), kKnnThreads, 0, c->cur>>>(
+        Z, n_ptr, n_max, c->d_Zt, c->d_yt, c->knn_ntrain, rows_per_split, part_d, part_i, labels);
+    TRY(check_launch(c, "k8_knn_topk"));
+    if (nsplit > 1) {
+        k8_knn_merge_kernel<K><<<std::max(1, cdiv(n_max, 256)), 256, 0, c->cur>>>(part_d, part_i, nsplit, n_ptr, n_max, c->d_yt, labels);
+        TRY(check_launch(c, "k8_knn_merge"));
+    }
+    return TSD_OK;
+}
+
+// K8b for X [n_max][knn_nfeat] (n = *n_ptr when n_ptr is set): Z [n_max][6] f64 out, part_d / part_i: knn_part_entries(c) each.
+template <typename T>
+static int dev_knn(tsd_ctx* c, const T* X, const int32_t* n_ptr, int n_max, double* Z, double* part_d, int32_t* part_i, int32_t* labels) {
+    int grid = std::max(1, cdiv((int64_t)n_max * 32, 256));
+    if (grid > c->sm_count * 8) grid = c->sm_count * 8;
+    k8_knn_project_kernel<T><<<grid, 256, 0, c->cur>>>(X, n_ptr, n_max, c->knn_nfeat, c->d_xbar, c->d_scal, Z);
+    TRY(check_launch(c, "k8_knn_project"));
+    int rps = 0;
+    const int nsplit = knn_splits(c, n_max, &rps);
+    switch (c->knn_k) {
+        case 1: return launch_knn_topk<1>(c, Z, n_ptr, n_max, nsplit, rps, part_d, part_i, labels);
+        case 2: return launch_knn_topk<2>(c, Z, n_ptr, n_max, nsplit, rps, part_d, part_i, labels);
+        case 3: return launch_knn_topk<3>(c, Z, n_ptr, n_max, nsplit, rps, part_d, part_i, labels);
+        case 4: return launch_knn_topk<4>(c, Z, n_ptr, n_max, nsplit, rps, part_d, part_i, labels);
+        case 5: return launch_knn_topk<5>(c, Z, n_ptr, n_max, nsplit, rps, part_d, part_i, labels);
+        case 6: return launch_knn_topk<6>(c, Z, n_ptr, n_max, nsplit, rps, part_d, part_i, labels);
+        case 7: return launch_knn_topk<7>(c, Z, n_ptr, n_max, nsplit, rps, part_d, part_i, labels);
+        case 8: return launch_knn_topk<8>(c, Z, n_ptr, n_max, nsplit, rps, part_d, part_i, labels);
+    }
+    return fail(TSD_E_STATE, "k = %d outside 1..%d", c->knn_k, kKnnMaxK);
+}
+
+extern "C" {
+
 int tsd_knn_predict(tsd_ctx* c, const float* X, int n, double* Z, int32_t* labels, int mem) {
     if (!c || n < 0 || (n && (!X || !labels))) return fail(TSD_E_INVALID, "bad argument");
     if (!c->d_Zt) return fail(TSD_E_STATE, "KNN model not set (tsd_set_knn)");
     CU(cudaSetDevice(c->device));
     if (n == 0) return TSD_OK;
     Stage s(c);
-    void *dx = (void*)X, *dz = Z, *dy = labels;
+    void *dx = (void*)X, *dz = Z, *dy = labels, *pd, *pi;
     if (mem == TSD_MEM_HOST) {
         TRY(s.in(X, (size_t)n * c->knn_nfeat * 4, &dx));
-        if (Z) TRY(s.alloc(&dz, (size_t)n * 6 * 8));
         TRY(s.alloc(&dy, (size_t)n * 4));
     }
-    k8_knn_kernel<<<cdiv((int64_t)n * 32, 128), 128, 0, c->cur>>>((float*)dx, n, c->knn_nfeat, c->d_xbar, c->d_scal, c->d_Zt, c->d_yt,
-                                                                      c->knn_ntrain, c->knn_k, (double*)dz, (int32_t*)dy);
-    TRY(check_launch(c, "k8_knn"));
+    if (mem == TSD_MEM_HOST || !Z) TRY(s.alloc(&dz, (size_t)n * 6 * 8));
+    TRY(s.alloc(&pd, knn_part_entries(c) * 8));
+    TRY(s.alloc(&pi, knn_part_entries(c) * 4));
+    TRY(dev_knn(c, (const float*)dx, nullptr, n, (double*)dz, (double*)pd, (int32_t*)pi, (int32_t*)dy));
     if (mem == TSD_MEM_HOST) {
         if (Z) TRY(s.out(Z, dz, (size_t)n * 6 * 8));
         TRY(s.out(labels, dy, (size_t)n * 4));
@@ -1409,22 +1467,33 @@ static int enqueue_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, i
         TRY(check_launch(c, "k4_score"));
         mark(c, "k4_score");
     } else {
+        // the descriptor (REC:517-521): HOG of the grey window, or with TSD_REC_GRAY its 1 024 grey bytes; then LDA or KNN
         uint8_t* gray = (uint8_t*)c->b_gray.p + wo * npx;
-        float* hog = (float*)c->b_hog.p + wo * TSD_HOG_LEN;
         int grid = cdiv((int64_t)cap * npx, 256);
         if (grid > c->sm_count * 16) grid = c->sm_count * 16;
         k6_gray_kernel<<<grid, 256, 0, c->cur>>>(windows, slots, d_nsurv, nb, npx, ws, gray);
         TRY(check_launch(c, "k6_gray"));
         mark(c, "k6_gray");
-        {
+        float* hog = nullptr;
+        if (!(mode & TSD_REC_GRAY)) {
+            hog = (float*)c->b_hog.p + wo * TSD_HOG_LEN;
             int hgrid = cdiv(cap, kHogWarps);
             if (hgrid > c->sm_count * 8) hgrid = c->sm_count * 8;
             k7_hog_kernel<<<hgrid, kHogWarps * 32, 0, c->cur>>>(gray, d_nsurv, nb, c->hog, hog);
+            TRY(check_launch(c, "k7_hog"));
+            mark(c, "k7_hog");
         }
-        TRY(check_launch(c, "k7_hog"));
-        mark(c, "k7_hog");
-        TRY(dev_lda(c, hog, d_nsurv, nb, c->cfg.proba_tol, nullptr, id));
-        mark(c, "k8_lda");
+        if (mode & TSD_REC_KNN) {
+            double* Z = (double*)c->b_knnz.p + wo * 6;
+            const size_t po = (size_t)B.sidx * knn_part_entries(c);
+            double* pd = (double*)c->b_knnpd.p + po;
+            int32_t* pi = (int32_t*)c->b_knnpi.p + po;
+            TRY(hog ? dev_knn(c, hog, d_nsurv, nb, Z, pd, pi, id) : dev_knn(c, gray, d_nsurv, nb, Z, pd, pi, id));
+            mark(c, "k8_knn");
+        } else {
+            TRY(hog ? dev_lda(c, hog, d_nsurv, nb, c->cfg.proba_tol, nullptr, id) : dev_lda(c, gray, d_nsurv, nb, c->cfg.proba_tol, nullptr, id));
+            mark(c, "k8_lda");
+        }
         // a survivor becomes a record when the classifier says "sign" (label != 0); no score in this flavour
         CU(cudaMemsetAsync(hund, 0, cap * 4, c->cur));
         label_emit_kernel<<<cdiv(cap, 256), 256, 0, c->cur>>>(id, d_nsurv, nb, emit);
@@ -1491,19 +1560,42 @@ static int run_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, int W
     return TSD_OK;
 }
 
+// The chain's mode (tsd_b200.h, TSD_REC_*): TSD_E_INVALID for an unknown combination of bits.
+static int check_mode(int mode) {
+    const int rec = mode & (TSD_REC_GRAY | TSD_REC_KNN), base = mode & ~(TSD_REC_GRAY | TSD_REC_KNN);
+    if ((base != TSD_RUN_DETECT && base != TSD_RUN_RECOGNIZE) || (base == TSD_RUN_DETECT && rec)) return fail(TSD_E_INVALID, "bad mode %d", mode);
+    return TSD_OK;
+}
+
+// The state a valid mode needs: TSD_E_STATE, naming what is missing.  Both checks run before any device work.
+static int check_mode_state(const tsd_ctx* c, int mode) {
+    const int D = c->cfg.window;
+    if (mode == TSD_RUN_DETECT) return (!c->have_templates || c->tmpl_D != D) ? fail(TSD_E_STATE, "templates not set for D=%d", D) : TSD_OK;
+    const bool gray = mode & TSD_REC_GRAY;
+    const int nfeat = gray ? kMaxPx : TSD_HOG_LEN;
+    const char* desc = gray ? "GRAY" : "HOG";
+    if (D != 32) return fail(TSD_E_STATE, "recognition needs D=32 (the context has D=%d)", D);
+    if (mode & TSD_REC_KNN) {
+        if (!c->d_Zt || c->knn_nfeat != nfeat)
+            return fail(TSD_E_STATE, "%s + KNN recognition needs a %d-feature KNN model (tsd_set_knn)%s", desc, nfeat, c->d_Zt ? ": the one set has another size" : "");
+    } else if (!c->d_ldaW || c->lda_nfeat != nfeat) {
+        return fail(TSD_E_STATE, "recognition needs D=32 and %d-feature LDA weights for %s descriptors (tsd_set_lda)%s", nfeat, desc, c->d_ldaW ? ": the ones set have another size" : "");
+    }
+    return TSD_OK;
+}
+
 // host_src != NULL: d_frames is ignored, the frames are page-locked host memory (host_src = their device pointer) and are staged
 // ROI sector by ROI sector into the context's mirror, which the chain then reads.
 static int enqueue_impl(tsd_ctx* c, int mode, const uint8_t* d_frames, int nframes, int H, int W, int64_t row_stride, int64_t frame_stride,
                         const int32_t* d_boxes, const int32_t* d_box_offsets, int nb, int max_boxes_per_frame, const uint8_t* host_src) {
     if (host_src) d_frames = host_src;                       // (argument checks below)
     if (!c || !d_frames || !d_box_offsets || nframes < 1 || nb < 0 || H < 1 || W < 1) return fail(TSD_E_INVALID, "bad argument");
-    if (mode != TSD_RUN_DETECT && mode != TSD_RUN_RECOGNIZE) return fail(TSD_E_INVALID, "bad mode %d", mode);
+    TRY(check_mode(mode));
     if (row_stride < (int64_t)W * 3 || frame_stride < row_stride * (H - 1) + (int64_t)W * 3) return fail(TSD_E_INVALID, "bad strides");
     if (nframes >= kMaxBatchFrames) return fail(TSD_E_INVALID, "%d frames: a batch holds fewer than 2^23 (the K5 work lists keep frame << 8 in an int32)", nframes);
     const int D = c->cfg.window, npx = D * D, ws = win_stride(npx, 3), es = ent_stride(npx);
     const int ms = (npx + 15) & ~15, NW = (npx + 31) >> 5;
-    if (mode == TSD_RUN_DETECT && (!c->have_templates || c->tmpl_D != D)) return fail(TSD_E_STATE, "templates not set for D=%d", D);
-    if (mode == TSD_RUN_RECOGNIZE && (!c->d_ldaW || D != 32 || c->lda_nfeat != TSD_HOG_LEN)) return fail(TSD_E_STATE, "recognition needs D=32 and 324-feature LDA weights");
+    TRY(check_mode_state(c, mode));
     CU(cudaSetDevice(c->device));
     if (max_boxes_per_frame <= 0) {                          // not given: one small D2H of the CSR offsets (synchronises)
         std::vector<int32_t> ho(nframes + 1);
@@ -1576,7 +1668,12 @@ static int enqueue_impl(tsd_ctx* c, int mode, const uint8_t* d_frames, int nfram
         TRY(ensure(c, c->b_bits, cap * 2 * NW * 4));
     } else {
         TRY(ensure(c, c->b_gray, cap * npx));
-        TRY(ensure(c, c->b_hog, cap * TSD_HOG_LEN * 4));
+        if (!(mode & TSD_REC_GRAY)) TRY(ensure(c, c->b_hog, cap * TSD_HOG_LEN * 4));
+        if (mode & TSD_REC_KNN) {                            // Z per window; the split's partial lists, one region per scratch slot
+            TRY(ensure(c, c->b_knnz, cap * 6 * 8));
+            TRY(ensure(c, c->b_knnpd, 2 * knn_part_entries(c) * 8));
+            TRY(ensure(c, c->b_knnpi, 2 * knn_part_entries(c) * 4));
+        }
     }
     TRY(ensure(c, c->b_pairs, mwords * sizeof(uint32_t)));
     if (host_src) {
@@ -1716,6 +1813,8 @@ int tsd_detect_frames(tsd_ctx* c, int mode, const uint8_t* frames, int nframes, 
                       const int32_t* boxes, const int32_t* box_offsets, tsd_detection* det, int det_cap, int32_t* ndet, int32_t* counts, int mem) {
     if (!c || !frames || !box_offsets || nframes < 1 || H < 1 || W < 1) return fail(TSD_E_INVALID, "bad argument");
     if (row_stride < (int64_t)W * 3 || frame_stride < row_stride * (H - 1) + (int64_t)W * 3) return fail(TSD_E_INVALID, "bad strides");
+    TRY(check_mode(mode));
+    TRY(check_mode_state(c, mode));
     CU(cudaSetDevice(c->device));
     if (mem == TSD_MEM_DEVICE) {
         int32_t nb = 0;

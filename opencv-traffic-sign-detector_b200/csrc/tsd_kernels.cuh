@@ -1467,7 +1467,8 @@ __device__ __forceinline__ int lda_decide(const double z[6], double tol) {
     return lab;
 }
 
-__global__ void __launch_bounds__(256) k8_lda_kernel(const float* __restrict__ X, const int32_t* __restrict__ n_ptr, int n_max,
+template <typename T>    // float: descriptors; uint8_t: the chain's grey windows ((double) of a byte is exact)
+__global__ void __launch_bounds__(256) k8_lda_kernel(const T* __restrict__ X, const int32_t* __restrict__ n_ptr, int n_max,
                                                      int nfeat, const double* __restrict__ W, const double* __restrict__ b,
                                                      double tol, double* __restrict__ logits, int32_t* __restrict__ labels) {
     extern __shared__ double s_W[];                         // [nfeat][6]
@@ -1476,7 +1477,7 @@ __global__ void __launch_bounds__(256) k8_lda_kernel(const float* __restrict__ X
     const int lane = threadIdx.x & 31, nwarps = (gridDim.x * blockDim.x) >> 5;
     const int n = n_ptr ? min(*n_ptr, n_max) : n_max;
     for (int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < n; w += nwarps) {
-        const float* x = X + (int64_t)w * nfeat;
+        const T* x = X + (int64_t)w * nfeat;
         double z[6] = {0, 0, 0, 0, 0, 0};
         for (int f = lane; f < nfeat; f += 32) {
             double xv = (double)x[f];
@@ -1561,61 +1562,137 @@ __global__ void __launch_bounds__(128) k8_lda_tf32_kernel(const float* __restric
     }
 }
 
-// K8b  reducer.transform + KNeighborsClassifier(k).predict  (REC:592-596).  One warp per query: Z = (x - xbar) S in
-// f64, then every lane keeps its k best of the training rows it visits; the warp merges by (distance, index).
+// K8b  reducer.transform + KNeighborsClassifier(k).predict  (REC:592-596), SURVEY A.8, as two kernels.
+// Projection: Z = (x - xbar) S in f64, one warp per window (lane-strided terms, then warp_sum).  T = float (HOG descriptors, the
+// tsd_knn_predict entry point) or uint8_t (the chain's grey windows: (double) of a byte is exact).
 constexpr int kKnnMaxK = 8;
 constexpr int kKnnMaxLabels = 16;                   // training labels 0..15 (tsd_set_knn checks)
-__global__ void __launch_bounds__(128) k8_knn_kernel(const float* __restrict__ X, int n, int nfeat, const double* __restrict__ xbar,
-                                                     const double* __restrict__ S, const double* __restrict__ Zt,
-                                                     const int32_t* __restrict__ yt, int ntrain, int k,
-                                                     double* __restrict__ Zout, int32_t* __restrict__ labels) {
-    const int lane = threadIdx.x & 31;
-    const int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (w >= n) return;
-    const float* x = X + (int64_t)w * nfeat;
-    double z[6] = {0, 0, 0, 0, 0, 0};
-    for (int f = lane; f < nfeat; f += 32) {
-        double xc = (double)x[f] - xbar[f];
+constexpr int kKnnThreads = 128;                    // queries per CTA of the top-k kernel (one thread each)
+constexpr int kKnnTile = 256;                       // training rows per shared-memory tile (48 B each, two tiles: 24 KB)
+template <typename T>
+__global__ void __launch_bounds__(256) k8_knn_project_kernel(const T* __restrict__ X, const int32_t* __restrict__ n_ptr, int n_max, int nfeat,
+                                                             const double* __restrict__ xbar, const double* __restrict__ S, double* __restrict__ Zout) {
+    const int lane = threadIdx.x & 31, nwarps = (gridDim.x * blockDim.x) >> 5;
+    const int n = n_ptr ? min(*n_ptr, n_max) : n_max;
+    for (int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < n; w += nwarps) {
+        const T* x = X + (int64_t)w * nfeat;
+        double z[6] = {0, 0, 0, 0, 0, 0};
+        for (int f = lane; f < nfeat; f += 32) {
+            double xc = (double)x[f] - xbar[f];
 #pragma unroll
-        for (int c = 0; c < 6; c++) z[c] += xc * S[f * 6 + c];
+            for (int c = 0; c < 6; c++) z[c] += xc * S[f * 6 + c];
+        }
+#pragma unroll
+        for (int c = 0; c < 6; c++) z[c] = warp_sum(z[c]);
+        if (lane == 0) for (int c = 0; c < 6; c++) Zout[(int64_t)w * 6 + c] = z[c];
     }
+}
+
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait_group() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+
+// Sorted insert into a register list of the K best (distance, index): a strictly smaller distance moves ahead, an equal one stays
+// behind.  Candidates arrive in increasing index order, so equal distances keep the smaller index first.
+template <int K>
+__device__ __forceinline__ void knn_insert(double (&bd)[K], int (&bi)[K], double d, int t) {
+    if (!(d < bd[K - 1])) return;
+    bd[K - 1] = d; bi[K - 1] = t;
 #pragma unroll
-    for (int c = 0; c < 6; c++) z[c] = warp_sum(z[c]);
-    if (lane == 0 && Zout) for (int c = 0; c < 6; c++) Zout[(int64_t)w * 6 + c] = z[c];
-    double bd[kKnnMaxK]; int bi[kKnnMaxK];
+    for (int j = K - 1; j > 0; j--)
+        if (bd[j] < bd[j - 1]) {
+            const double td = bd[j]; bd[j] = bd[j - 1]; bd[j - 1] = td;
+            const int ti = bi[j]; bi[j] = bi[j - 1]; bi[j - 1] = ti;
+        }
+}
+
+// Uniform vote of the (up to K) neighbours found: 16 four-bit counters in one register, ties to the smallest label.
+template <int K>
+__device__ __forceinline__ int knn_vote(const int (&bi)[K], const int32_t* __restrict__ yt) {
+    uint64_t votes = 0;
 #pragma unroll
-    for (int j = 0; j < kKnnMaxK; j++) { bd[j] = INFINITY; bi[j] = 0x7fffffff; }
-    for (int t = lane; t < ntrain; t += 32) {
-        double d = 0;
+    for (int j = 0; j < K; j++)
+        if (bi[j] != 0x7fffffff) { const int y = yt[bi[j]]; if (y >= 0 && y < kKnnMaxLabels) votes += 1ull << (4 * y); }
+    int lab = 0, bv = -1;
 #pragma unroll
-        for (int c = 0; c < 6; c++) { double e = z[c] - Zt[(int64_t)t * 6 + c]; d += e * e; }
-        if (d < bd[k - 1]) {                                // per-lane indices increase, so ties keep the smaller index
-            int pos = k - 1;
-            while (pos > 0 && bd[pos - 1] > d) { bd[pos] = bd[pos - 1]; bi[pos] = bi[pos - 1]; pos--; }
-            bd[pos] = d; bi[pos] = t;
+    for (int y = 0; y < kKnnMaxLabels; y++) { const int v = (int)((votes >> (4 * y)) & 15); if (v > bv) { bv = v; lab = y; } }
+    return lab;
+}
+
+// Top-k: one thread per query, kKnnThreads queries per CTA.  The training rows [blockIdx.y * rows_per_split, + rows_per_split) stream
+// through shared memory in double-buffered cp.async tiles; every thread reads the same row (broadcast).  gridDim.y == 1: the thread
+// votes and writes its label.  gridDim.y > 1 (training set split across CTAs for small batches): it writes its partial list to
+// part_d / part_i [split][K][n_max] and k8_knn_merge_kernel finishes the query.
+template <int K>
+__global__ void __launch_bounds__(kKnnThreads) k8_knn_topk_kernel(const double* __restrict__ Z, const int32_t* __restrict__ n_ptr, int n_max,
+                                                                  const double* __restrict__ Zt, const int32_t* __restrict__ yt, int ntrain,
+                                                                  int rows_per_split, double* __restrict__ part_d, int32_t* __restrict__ part_i,
+                                                                  int32_t* __restrict__ labels) {
+    __shared__ __align__(16) double s_t[2][kKnnTile * 6];
+    const int n = n_ptr ? min(*n_ptr, n_max) : n_max;
+    if ((int)(blockIdx.x * kKnnThreads) >= n) return;                  // (uniform per CTA)
+    const int q = blockIdx.x * kKnnThreads + threadIdx.x;
+    const bool live = q < n;
+    double z[6];
+#pragma unroll
+    for (int c = 0; c < 6; c++) z[c] = live ? Z[(int64_t)q * 6 + c] : 0.0;
+    double bd[K]; int bi[K];
+#pragma unroll
+    for (int j = 0; j < K; j++) { bd[j] = INFINITY; bi[j] = 0x7fffffff; }
+    const int r0 = blockIdx.y * rows_per_split, r1 = min(ntrain, r0 + rows_per_split);
+    auto load = [&](int buf, int t0) {                                 // rows t0 .. t0 + kKnnTile - 1 (clipped), 3 x 16 B per row
+        const int chunks = min(kKnnTile, r1 - t0) * 3;
+        const char* src = (const char*)(Zt + (int64_t)t0 * 6);
+        for (int i = threadIdx.x; i < chunks; i += kKnnThreads) cp_async16(&s_t[buf][i * 2], src + (int64_t)i * 16);
+        cp_async_commit();
+    };
+    if (r0 < r1) load(0, r0);
+    int buf = 0;
+    for (int t0 = r0; t0 < r1; t0 += kKnnTile, buf ^= 1) {
+        if (t0 + kKnnTile < r1) { load(buf ^ 1, t0 + kKnnTile); cp_async_wait_group<1>(); }
+        else cp_async_wait_group<0>();
+        __syncthreads();
+        const int rows = min(kKnnTile, r1 - t0);
+        const double* tile = s_t[buf];
+#pragma unroll 2
+        for (int r = 0; r < rows; r++) {
+            double d = 0;
+#pragma unroll
+            for (int c = 0; c < 6; c++) { double e = z[c] - tile[r * 6 + c]; d += e * e; }
+            knn_insert<K>(bd, bi, d, t0 + r);
+        }
+        __syncthreads();                                               // the next iteration's prefetch overwrites this tile
+    }
+    if (!live) return;
+    if (gridDim.y == 1) { labels[q] = knn_vote<K>(bi, yt); return; }
+#pragma unroll
+    for (int j = 0; j < K; j++) {
+        part_d[((int64_t)blockIdx.y * K + j) * n_max + q] = bd[j];
+        part_i[((int64_t)blockIdx.y * K + j) * n_max + q] = bi[j];
+    }
+}
+
+// The k smallest (distance, index) over the splits' partial lists, then the vote.  Split s holds smaller indices than split s + 1 and
+// its list is sorted by (distance, index), so the candidates of an equal distance arrive in increasing index order.
+template <int K>
+__global__ void __launch_bounds__(256) k8_knn_merge_kernel(const double* __restrict__ part_d, const int32_t* __restrict__ part_i, int nsplit,
+                                                           const int32_t* __restrict__ n_ptr, int n_max, const int32_t* __restrict__ yt,
+                                                           int32_t* __restrict__ labels) {
+    const int n = n_ptr ? min(*n_ptr, n_max) : n_max;
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n) return;
+    double bd[K]; int bi[K];
+#pragma unroll
+    for (int j = 0; j < K; j++) { bd[j] = INFINITY; bi[j] = 0x7fffffff; }
+    for (int s = 0; s < nsplit; s++) {
+#pragma unroll
+        for (int j = 0; j < K; j++) {
+            const int i = part_i[((int64_t)s * K + j) * n_max + q];
+            if (i == 0x7fffffff) break;                                // (the rest of this split's list is empty too)
+            knn_insert<K>(bd, bi, part_d[((int64_t)s * K + j) * n_max + q], i);
         }
     }
-    // k rounds of warp arg-min over the lanes' current heads
-    int votes[kKnnMaxLabels];
-#pragma unroll
-    for (int j = 0; j < kKnnMaxLabels; j++) votes[j] = 0;
-    int head = 0;
-    for (int r = 0; r < k; r++) {
-        double d = head < k ? bd[head] : INFINITY; int idx = head < k ? bi[head] : 0x7fffffff;
-        double bdv = d; int bidx = idx;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            double od = __shfl_xor_sync(0xffffffffu, bdv, o); int oi = __shfl_xor_sync(0xffffffffu, bidx, o);
-            if (od < bdv || (od == bdv && oi < bidx)) { bdv = od; bidx = oi; }
-        }
-        if (idx == bidx && d == bdv) head++;
-        if (bidx != 0x7fffffff) { int y = yt[bidx]; if (y >= 0 && y < kKnnMaxLabels) votes[y]++; }
-    }
-    if (lane == 0) {
-        int lab = 0, bv = -1;
-        for (int y = 0; y < kKnnMaxLabels; y++) if (votes[y] > bv) { bv = votes[y]; lab = y; }   // ties -> smallest label
-        labels[w] = lab;
-    }
+    labels[q] = knn_vote<K>(bi, yt);
 }
 
 // =====================================================================================================

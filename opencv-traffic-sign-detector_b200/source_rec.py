@@ -10,7 +10,7 @@ import numpy as np
 
 from . import engine
 from . import source_det as _det
-from ._capi import TsdError
+from ._capi import REC_GRAY, REC_KNN, RUN_RECOGNIZE, TsdError
 
 _ctx = None
 _lda_key = None
@@ -200,10 +200,8 @@ def predictProbabilityLDAClassifiers(LDAClassifiers, detectionsDescriptors, tole
     return [int(v) for v in labels], true
 
 
-def predictProbabilityKNNClassifiers(KNNClassifier, reducer, detectionDescriptors):
-    """REC:592-596 -> (predicted labels ndarray, true labels list)."""
+def _use_knn(KNNClassifier, reducer):
     global _knn_key
-    X, true = extractDescriptorsAndRealSignTypes(detectionDescriptors)
     lda = reducer[0]
     Zt = np.asarray(KNNClassifier._fit_X, np.float64)
     yt = np.asarray(KNNClassifier.classes_)[np.asarray(KNNClassifier._y)].astype(np.int32)
@@ -214,6 +212,12 @@ def predictProbabilityKNNClassifiers(KNNClassifier, reducer, detectionDescriptor
             raise TsdError("KNN path expects the 6-component LDA reducer of REC:586-589")
         context().set_knn(lda.xbar_, lda.scalings_[:, :ncomp], Zt, yt, KNNClassifier.n_neighbors)
         _knn_key = key
+
+
+def predictProbabilityKNNClassifiers(KNNClassifier, reducer, detectionDescriptors):
+    """REC:592-596 -> (predicted labels ndarray, true labels list)."""
+    X, true = extractDescriptorsAndRealSignTypes(detectionDescriptors)
+    _use_knn(KNNClassifier, reducer)
     if not X:
         return np.zeros(0, np.int64), true
     _, labels = context().knn_predict(np.stack(X).astype(np.float32), want_Z=False)
@@ -226,6 +230,28 @@ def predictProbability(classifiers, reducer, testDataDescriptors, tolerance):
         return predictProbabilityLDAClassifiers(classifiers[0], testDataDescriptors, tolerance)
     elif classifiers[1] == 'KNN':
         return predictProbabilityKNNClassifiers(classifiers[0], reducer, testDataDescriptors)
+
+
+def recognizeBatch(frames, boxes, box_offsets, files, classifiers, reducer, featureDescriptor):
+    """Whole recognition chain for a batch of frames in ONE library call, the counterpart of source_det.detectBatch: per frame
+    MSERTrafficSignDetector (REC:47-64) -> windowsToGray -> calculateDescriptors (featureDescriptor[1] = 'HOG' or 'GRAY') ->
+    predictProbability (classifiers[1] = 'LDABAYES' with the context's proba_tol, 0.5 as at REC:760, or 'KNN' with `reducer`).
+    -> list of (file, x1, y1, x2, y2, label) for every survivor whose label is not 0, in frame order then list order, and the
+    stage counts (raw boxes, aspect-passing windows, survivors, records)."""
+    mode = RUN_RECOGNIZE
+    if featureDescriptor[1] == 'GRAY':
+        mode |= REC_GRAY
+    elif featureDescriptor[1] != 'HOG':
+        raise TsdError("featureDescriptor must be (_, 'HOG') or (_, 'GRAY'), not %r" % (featureDescriptor[1],))
+    if classifiers[1] == 'KNN':
+        mode |= REC_KNN
+        _use_knn(classifiers[0], reducer)
+    elif classifiers[1] == 'LDABAYES':
+        _use_lda(classifiers[0])
+    else:
+        raise TsdError("classifiers must be (_, 'LDABAYES') or (_, 'KNN'), not %r" % (classifiers[1],))
+    det, counts = context().detect_frames(frames, boxes, box_offsets, mode=mode)
+    return [(files[int(d["frame"])], int(d["x1"]), int(d["y1"]), int(d["x2"]), int(d["y2"]), int(d["id"])) for d in det], counts
 
 
 _PATCHED = ("grayAndEnhanceContrast", "makeWindowBiggerOrDiscardFakeDetections", "cleanDuplicatedDetections", "MSERTrafficSignDetector",
