@@ -69,7 +69,9 @@ typedef struct tsd_config {
     uint8_t blue_hi[3];        /* DET/source.py:86 */
     uint8_t pad_[6];
     double proba_tol;          /* 0.5 REC/source.py:761 */
-    int32_t knn_k;             /* 4 REC/source.py:607 */
+    int32_t knn_k;             /* 4 REC/source.py:607; 1..8 (tsd_create: TSD_E_INVALID otherwise).  The k a caller passes to
+                                  tsd_set_knn when it has no other (the Python Context.set_knn default); the k-NN kernels use
+                                  the k of the last tsd_set_knn call. */
     int32_t reserved;
 } tsd_config;
 
@@ -230,7 +232,8 @@ TSD_API int tsd_lda_predict_tf32(tsd_ctx *ctx, const float *X, int n, double tol
 
 /* K8b predictProbabilityKNNClassifiers (REC/source.py:592-596): Z f64 [n][6] (may be NULL), labels int32 [n].
  * Brute force over the training set (tiles of it in shared memory, one thread per query; below about one 128-query block per SM the
- * training set is also split across blocks and the partial lists merged); training rows at equal distance are ranked by index
+ * training set is also split across blocks and the partial lists merged; the chain decides this from the batch's box count, not from
+ * how many windows survive, and the labels are the same either way); training rows at equal distance are ranked by index
  * (the smaller one is nearer), then a uniform vote with ties to the smallest label.  scikit-learn's kd-tree orders exact distance ties its own way, so labels can
  * differ from it when a tie straddles the k-th neighbour (SURVEY A.8). */
 TSD_API int tsd_knn_predict(tsd_ctx *ctx, const float *X, int n, double *Z, int32_t *labels, int mem);

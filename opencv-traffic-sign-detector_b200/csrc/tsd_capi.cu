@@ -338,6 +338,8 @@ int tsd_create(tsd_ctx** out, int device, const tsd_config* cfg) {
     c->device = device;
     if (cfg) c->cfg = *cfg; else tsd_config_default(&c->cfg, 0);
     if (c->cfg.window < 2 || c->cfg.window > kMaxD) { delete c; return fail(TSD_E_INVALID, "window %d not in [2,%d]", c->cfg.window, kMaxD); }
+    if (c->cfg.knn_k < 1 || c->cfg.knn_k > kKnnMaxK) { const int k = c->cfg.knn_k; delete c; return fail(TSD_E_INVALID, "knn_k %d not in [1,%d]", k, kKnnMaxK); }
+    c->knn_k = c->cfg.knn_k;                                 // (no k-NN model before tsd_set_knn, which sets its own k)
     const int rc = create_impl(c, device);
     if (rc != TSD_OK) { tsd_destroy(c); return rc; }         // one cleanup path: whatever was created so far is released (g_err is kept)
     *out = c;

@@ -115,8 +115,10 @@ class Context:
         check(self._L.tsd_set_lda(self._h, ptr(W), ptr(b), W.shape[0]))
         self._lda_nfeat = W.shape[0]
 
-    def set_knn(self, xbar, scalings, Ztrain, ytrain, k=4):
-        """7-class LDA reducer (xbar_, scalings_[:, :6]) + KNN training set (REC:586-589)."""
+    def set_knn(self, xbar, scalings, Ztrain, ytrain, k=None):
+        """7-class LDA reducer (xbar_, scalings_[:, :6]) + KNN training set (REC:586-589); k = 1..8, by default the
+        context's config knn_k (4, REC:607)."""
+        k = self.cfg.knn_k if k is None else k
         xbar = np.ascontiguousarray(xbar, np.float64); S = np.ascontiguousarray(scalings, np.float64)
         Z = np.ascontiguousarray(Ztrain, np.float64); y = _i32(ytrain)
         if S.shape != (len(xbar), 6) or Z.ndim != 2 or Z.shape[1] != 6 or len(y) != len(Z):
