@@ -24,6 +24,9 @@
  *     must span less than 2 GiB (row_stride * H < 2^31; TSD_E_INVALID otherwise).  A batch of tsd_detect_frames /
  *     tsd_enqueue_frames / tsd_dedup has fewer than 2^23 frames (TSD_E_INVALID otherwise, before any device work; pageable host
  *     frames run in chunks, so only each chunk counts).  tsd_bgr2gray and tsd_bgr2hsv take any int64 pixel count.
+ *   - frames of different sizes: the *_ragged entry points take one base pointer and a tsd_frame_desc table (below) instead of
+ *     (frames, nframes, H, W, row_stride, frame_stride).  The table is ALWAYS a host pointer, whatever `mem` says; the buffer
+ *     behind `base` spans every entry's bytes, from base up to the largest offset + (H-1) * row_stride + W * channels.
  */
 #ifndef TSD_B200_H
 #define TSD_B200_H
@@ -49,6 +52,17 @@ extern "C" {
 #define TSD_NCLASS 6         /* DET/constants.py:1 SIGNALLIST */
 
 typedef struct tsd_ctx tsd_ctx;
+
+/* One frame of a batch whose frames differ in size (the *_ragged entry points): the frame is uint8 [H][W][channels] at
+ * base + offset with row_stride bytes between rows.  Entries may alias (the same frame twice, or a sub-rectangle view of
+ * another entry: an offset inside it with the parent's row stride); frames are only read.  Every entry is checked before
+ * any device work (TSD_E_INVALID otherwise, the context stays usable): H, W >= 1, row_stride >= W * channels, offset >= 0
+ * and row_stride * H < 2^31; a table has 1 .. 2^23 - 1 entries.  A record's `frame` is its entry's index in the table. */
+typedef struct tsd_frame_desc {   /* 24 bytes */
+    int64_t offset;               /* byte offset of the frame's pixel (0,0) from the call's base pointer */
+    int64_t row_stride;           /* bytes between rows */
+    int32_t H, W;
+} tsd_frame_desc;
 
 /* All hard-coded constants of the reference path, one POD (SURVEY.md section 5 "config / flags").  tsd_create refuses (TSD_E_INVALID)
  * a window outside 2..32 and a coord_tol * merge_factor that is not above sqrt(f(65535)) = 0.3913: pairs whose corners are further
@@ -103,7 +117,8 @@ TSD_API int tsd_flush(tsd_ctx *ctx);
  * device-resident mirror of the frames; batches of 512 frames or more run as up to four chunks whose transfers overlap the
  * previous chunk's kernels, TSD_STAGE_CHUNK=0 turns the chunking off); pageable frames are copied whole, in chunks that overlap
  * the kernels.  Buffers from cudaHostAlloc / torch pin_memory() are already page-locked.
- * Staging needs a 16-byte aligned frames pointer, row_stride and frame_stride multiples of 16 and 3 * W a multiple of 16; any other
+ * Staging needs a 16-byte aligned frames pointer, row_stride and frame_stride multiples of 16 and 3 * W a multiple of 16 (a
+ * tsd_frame_desc table: every entry's offset, row_stride and 3 * W); any other
  * page-locked layout is read by K2 itself, tap by tap over PCIe (as with TSD_STAGE=0).  Either way the records are the same. */
 TSD_API int tsd_host_register(void *p, int64_t bytes);
 TSD_API int tsd_host_unregister(void *p);
@@ -152,6 +167,15 @@ TSD_API int tsd_crop_resize(tsd_ctx *ctx, const uint8_t *frames, int nframes, in
 TSD_API int tsd_windows(tsd_ctx *ctx, const uint8_t *frames, int nframes, int H, int W, int64_t row_stride,
                         int64_t frame_stride, const int32_t *boxes, const int32_t *box_offsets, double enlarge, int D,
                         uint8_t *windows, int32_t *coords, int32_t *win_offsets, int32_t *total, int mem);
+
+/* tsd_crop_resize / tsd_windows on frames of different sizes: frame f of the call is table[f] over `base` (host table, see
+ * tsd_frame_desc).  Same rules and outputs as the uniform calls; a table whose entries share H, W and row_stride at offsets
+ * f * frame_stride gives what the uniform call gives. */
+TSD_API int tsd_crop_resize_ragged(tsd_ctx *ctx, const uint8_t *base, const tsd_frame_desc *table, int nframes, int channels,
+                                   const int32_t *coords, const int32_t *win_frame, int n, int D, uint8_t *windows, int mem);
+TSD_API int tsd_windows_ragged(tsd_ctx *ctx, const uint8_t *base, const tsd_frame_desc *table, int nframes, const int32_t *boxes,
+                               const int32_t *box_offsets, double enlarge, int D, uint8_t *windows, int32_t *coords,
+                               int32_t *win_offsets, int32_t *total, int mem);
 
 /* K5  cleanDuplicatedDetections(list, by_coords, tol) per frame (DET/source.py:177-223; helpers :459-477,575-586).
  * In: windows/coords/offsets (CSR per frame).  Out: survivors, compacted per frame in the fold's list order.
@@ -283,6 +307,19 @@ TSD_API int tsd_enqueue_frames(tsd_ctx *ctx, int mode, const uint8_t *d_frames, 
                                int64_t row_stride, int64_t frame_stride, const int32_t *d_boxes,
                                const int32_t *d_box_offsets, int nboxes_total, int max_boxes_per_frame);
 TSD_API int tsd_fetch_detections(tsd_ctx *ctx, tsd_detection *det, int det_cap, int32_t *ndet, int32_t *counts);
+
+/* The chain on frames of different sizes (table: host tsd_frame_desc [nframes], 3 channels): every mode and, for
+ * tsd_detect_frames_ragged, every host route of tsd_detect_frames (page-locked staged when base, every offset, row stride and 3 W
+ * are multiples of 16, else gathered by K2; pageable frames copied frame by frame in chunks).  Records come out in table order,
+ * then list order; `frame` is the table index.  tsd_enqueue_frames_ragged is tsd_enqueue_frames with the table: the library copies
+ * it, in stream order, into a per-slot device buffer of the context (the caller may reuse its table as soon as the call returns),
+ * and the batch works with tsd_fetch_detections / tsd_fetch_previous, the two-slot overlap and the CUDA graphs like any other. */
+TSD_API int tsd_detect_frames_ragged(tsd_ctx *ctx, int mode, const uint8_t *base, const tsd_frame_desc *table, int nframes,
+                                     const int32_t *boxes, const int32_t *box_offsets, tsd_detection *det, int det_cap,
+                                     int32_t *ndet, int32_t *counts, int mem);
+TSD_API int tsd_enqueue_frames_ragged(tsd_ctx *ctx, int mode, const uint8_t *d_base, const tsd_frame_desc *table, int nframes,
+                                      const int32_t *d_boxes, const int32_t *d_box_offsets, int nboxes_total,
+                                      int max_boxes_per_frame);
 /* Streaming use of the two slots: after  enqueue(batch k); enqueue(batch k+1);  tsd_fetch_previous returns batch k's records
  * (same arguments as tsd_fetch_detections) while batch k+1 keeps running -- e.g. its K2 pulling ROIs out of page-locked host
  * frames over PCIe under batch k's GPU-bound kernels.  TSD_E_STATE if there is no such batch. */

@@ -11,7 +11,7 @@ Layout
   evaluate.py      the two evaluators (generateStatistics, precision_recall_curve / AP) with their matching loops on the GPU
 """
 from . import _capi, synth  # noqa: F401
-from ._capi import DET_DTYPE, HOG_LEN, MEM_DEVICE, MEM_HOST, REC_GRAY, REC_KNN, RUN_DETECT, RUN_RECOGNIZE, TsdError, build  # noqa: F401
+from ._capi import DET_DTYPE, FRAME_DESC_DTYPE, HOG_LEN, MEM_DEVICE, MEM_HOST, REC_GRAY, REC_KNN, RUN_DETECT, RUN_RECOGNIZE, TsdError, build  # noqa: F401
 from .engine import Context, default_config, similarity_table  # noqa: F401
 from . import evaluate, sharding, source_det, source_rec  # noqa: F401,E402
 

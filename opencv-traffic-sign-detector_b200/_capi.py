@@ -38,6 +38,13 @@ class Detection(C.Structure):
                 ("id", C.c_int32), ("hundredths", C.c_int32), ("reserved", C.c_int32)]
 
 
+class FrameDesc(C.Structure):
+    """tsd_frame_desc: one frame of a batch of frames of different sizes (the *_ragged entry points)."""
+    _fields_ = [("offset", C.c_int64), ("row_stride", C.c_int64), ("H", C.c_int32), ("W", C.c_int32)]
+
+
+FRAME_DESC_DTYPE = np.dtype([("offset", "<i8"), ("row_stride", "<i8"), ("H", "<i4"), ("W", "<i4")])
+
 DET_DTYPE = np.dtype([("frame", "<i4"), ("x1", "<i4"), ("y1", "<i4"), ("x2", "<i4"), ("y2", "<i4"),
                       ("id", "<i4"), ("hundredths", "<i4"), ("reserved", "<i4")])
 
@@ -75,6 +82,10 @@ _SIGNATURES = {
     "tsd_expand_boxes": (_i, [_vp, _vp, _i, _d, _vp, _vp, _i]),
     "tsd_crop_resize": (_i, [_vp, _vp, _i, _i, _i, _i64, _i64, _i, _vp, _vp, _i, _i, _vp, _i]),
     "tsd_windows": (_i, [_vp, _vp, _i, _i, _i, _i64, _i64, _vp, _vp, _d, _i, _vp, _vp, _vp, _vp, _i]),
+    "tsd_crop_resize_ragged": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _i, _i, _vp, _i]),
+    "tsd_windows_ragged": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _d, _i, _vp, _vp, _vp, _vp, _i]),
+    "tsd_detect_frames_ragged": (_i, [_vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _i, _vp, _vp, _i]),
+    "tsd_enqueue_frames_ragged": (_i, [_vp, _i, _vp, _vp, _i, _vp, _vp, _i, _i]),
     "tsd_dedup": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _d, _vp, _vp, _vp, _vp, _i]),
     "tsd_hist": (_i, [_vp, _vp, _i, _i, _vp, _i]),
     "tsd_color_masks": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i]),

@@ -72,6 +72,7 @@ struct tsd_ctx {
     int stage_rois = 1;                      // ... by the mark + copy kernels, each touched 32-byte sector once, into a device mirror K2 reads
                                              // (TSD_STAGE=0: K2 itself gathers from host memory, round 1's path)
     DevBuf b_mirror[2], b_stagemap[2];       // per scratch slot (consecutive batches of a chunked tsd_detect_frames call overlap)
+    DevBuf b_geom[2];                        // per scratch slot: the device copy of a *_ragged batch's frame table
     int stage_chunk = 256;                   // TSD_STAGE_CHUNK: frames per chunk of tsd_detect_frames on page-locked host frames (0 = one batch)
     int stage_ctas = 2;                      // TSD_STAGE_CTAS: CTAs per SM of the staging copy (PCIe-bound: 2 keep the link as busy as 8 and leave the SMs to the other chunk's chain)
     unsigned long long* d_staged = nullptr;  // bytes the staging copy moved over PCIe (tsd_stat_staged_bytes)
@@ -354,7 +355,7 @@ int tsd_destroy(tsd_ctx* c) {
     DevBuf* bufs[] = {&c->b_coords, &c->b_winframe, &c->b_windows, &c->b_entries, &c->b_meta, &c->b_list, &c->b_flags, &c->b_cnt,
                       &c->b_winoff, &c->b_survcnt, &c->b_survoff, &c->b_slots, &c->b_pairs, &c->b_energy, &c->b_red, &c->b_blue, &c->b_bits, &c->b_id, &c->b_hund,
                       &c->b_emit, &c->b_detcnt, &c->b_detoff, &c->b_det, &c->b_gray, &c->b_hog, &c->b_labels, &c->b_scores, &c->b_knnz, &c->b_knnpd, &c->b_knnpi,
-                      &c->b_stage[0], &c->b_stage[1], &c->b_hboxes, &c->b_hoff, &c->b_summary, &c->b_order, &c->b_gramdone, &c->b_mirror[0], &c->b_mirror[1], &c->b_stagemap[0], &c->b_stagemap[1], &c->b_pgray, &c->b_pluts, &c->b_pin, &c->b_pout};
+                      &c->b_stage[0], &c->b_stage[1], &c->b_hboxes, &c->b_hoff, &c->b_summary, &c->b_order, &c->b_gramdone, &c->b_mirror[0], &c->b_mirror[1], &c->b_stagemap[0], &c->b_stagemap[1], &c->b_geom[0], &c->b_geom[1], &c->b_pgray, &c->b_pluts, &c->b_pin, &c->b_pout};
     for (DevBuf* b : bufs) if (b->p) cudaFree(b->p);
     for (int i = 0; i < 2; i++) {
         if (c->ev_slot_fork[i]) cudaEventDestroy(c->ev_slot_fork[i]);
@@ -591,6 +592,55 @@ struct Stage {                                               // stream-ordered t
     }
 };
 
+// ---- frames of different sizes: the host side of a tsd_frame_desc table ------------------------------------------------------------
+// Everything the library needs from a table, derived on the host before any device work: the kernels' per-frame geometry, the
+// bytes the frames span from the base, the staging bitmap's size and the batch-wide choices (wide K2 loads, staging eligibility).
+struct Ragged {
+    std::vector<FrameGeom> geom;
+    int nframes = 0;
+    int64_t extent = 0;                      // largest offset + (H-1) * row_stride + W * channels
+    int64_t min_offset = 0;
+    int64_t words = 0;                       // staging-bitmap words (sum of H * stage_words_per_row(W))
+    bool wide4 = true;                       // every offset and row stride a multiple of 4 (K2's wide loads, with a 4-byte aligned base)
+    bool stage16 = true;                     // every offset, row stride and 3 W a multiple of 16 (ROI staging, with a 16-byte aligned base)
+    const FrameGeom* d = nullptr;            // the device copy the kernels of this call read
+};
+
+// Validates table[0 .. n) (TSD_E_INVALID, nothing touched) and fills R.  rebase: offsets are made relative to the smallest one
+// (R->min_offset keeps it), for a chunk of a table that starts at base + min_offset.
+static int make_ragged(const tsd_frame_desc* t, int n, int ch, Ragged* R, bool rebase = false) {
+    if (!t) return fail(TSD_E_INVALID, "table is NULL");
+    if (n < 1 || n >= kMaxBatchFrames) return fail(TSD_E_INVALID, "%d table entries: a table holds 1 .. 2^23 - 1 (the K5 work lists keep frame << 8 in an int32)", n);
+    int64_t mo = INT64_MAX;
+    for (int f = 0; f < n; f++) {
+        const tsd_frame_desc& e = t[f];
+        if (e.H < 1 || e.W < 1) return fail(TSD_E_INVALID, "table entry %d: H = %d, W = %d (both must be >= 1)", f, e.H, e.W);
+        if (e.row_stride < (int64_t)e.W * ch) return fail(TSD_E_INVALID, "table entry %d: row stride %lld below W * channels = %lld", f, (long long)e.row_stride, (long long)e.W * ch);
+        if (e.offset < 0 || e.offset > (INT64_MAX >> 2)) return fail(TSD_E_INVALID, "table entry %d: offset %lld out of range", f, (long long)e.offset);
+        if (e.row_stride * (int64_t)e.H >= ((int64_t)1 << 31)) return fail(TSD_E_INVALID, "table entry %d: a frame must span less than 2 GiB (row offsets are 32-bit)", f);
+        mo = std::min(mo, (int64_t)e.offset);
+    }
+    R->geom.resize(n);
+    R->nframes = n;
+    R->min_offset = rebase ? mo : 0;
+    R->extent = 0; R->words = 0; R->wide4 = R->stage16 = true;
+    for (int f = 0; f < n; f++) {
+        const tsd_frame_desc& e = t[f];
+        FrameGeom& g = R->geom[f];
+        g.offset = e.offset - R->min_offset;
+        g.row_stride = (int32_t)e.row_stride; g.H = e.H; g.W = e.W;
+        g.word0 = R->words;
+        R->words += (int64_t)e.H * stage_words_per_row(e.W);
+        R->extent = std::max(R->extent, g.offset + (int64_t)g.row_stride * (g.H - 1) + (int64_t)g.W * ch);
+        R->wide4 = R->wide4 && g.offset % 4 == 0 && g.row_stride % 4 == 0;
+        R->stage16 = R->stage16 && g.offset % 16 == 0 && g.row_stride % 16 == 0 && ((int64_t)g.W * 3) % 16 == 0;
+    }
+    // A wide K2 load reads aligned words up to 6 bytes past the last byte a row needs: frames whose last row ends that close to the
+    // extent (the end of what the caller vouches for) keep byte loads on it, whichever table entry they are.
+    for (auto& g : R->geom) g.guard = g.offset + (int64_t)g.row_stride * (g.H - 1) + (int64_t)g.W * ch + 8 > R->extent;
+    return TSD_OK;
+}
+
 static HsvBounds bounds_of(const tsd_config& cfg) {
     HsvBounds hb;
     memcpy(hb.red_lo, cfg.red_lo, 6); memcpy(hb.red_hi, cfg.red_hi, 6);
@@ -607,23 +657,36 @@ static int dev_expand(tsd_ctx* c, const int32_t* boxes, int n, double enlarge, i
 
 // out_stride = bytes between output windows: D*D*ch (public packed layout) or win_stride() (internal, zero padded).
 // nframes = frames behind `frames` (0 = unknown: byte loads throughout).
+template <bool TAB>
+static void launch_k2(tsd_ctx* c, int g4, int g4_all, const uint8_t* frames, int H, int W, int64_t rs, int64_t fs, int ch, const int32_t* coords,
+                      const int32_t* win_frame, const int32_t* n_ptr, int n_max, int D, uint8_t* windows, int out_stride, int wide_last, const FrameGeom* geom) {
+#define K2_ARGS frames, H, W, rs, fs, (const int4*)coords, win_frame, n_ptr, n_max
+    if (ch == 3 && D == 25) k2_crop_resize_v2_kernel<3, 25, TAB><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, wide_last, geom);
+    else if (ch == 3 && D == 32) k2_crop_resize_v2_kernel<3, 32, TAB><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, wide_last, geom);
+    else if (ch == 1 && D == 25) k2_crop_resize_v2_kernel<1, 25, TAB><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, -2, geom);
+    else if (ch == 1 && D == 32) k2_crop_resize_v2_kernel<1, 32, TAB><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, -2, geom);
+    else if (ch == 3) k2_crop_resize_kernel<3, TAB><<<g4_all, 128, 0, c->cur>>>(K2_ARGS, D, windows, out_stride, geom);      // other window sizes: generic kernel
+    else k2_crop_resize_kernel<1, TAB><<<g4_all, 128, 0, c->cur>>>(K2_ARGS, D, windows, out_stride, geom);
+#undef K2_ARGS
+}
+
+// R (frames of different sizes): frame f is R->d[f] over `frames`; H, W, rs, fs and nframes are not used.
 static int dev_crop_resize(tsd_ctx* c, const uint8_t* frames, int H, int W, int64_t rs, int64_t fs, int ch, const int32_t* coords,
-                           const int32_t* win_frame, const int32_t* n_ptr, int n_max, int D, uint8_t* windows, int out_stride, int nframes = 0) {
+                           const int32_t* win_frame, const int32_t* n_ptr, int n_max, int D, uint8_t* windows, int out_stride, int nframes = 0,
+                           const Ragged* R = nullptr) {
     if (n_max == 0) return TSD_OK;
-    if (rs * (int64_t)H >= ((int64_t)1 << 31)) return fail(TSD_E_INVALID, "a frame must span less than 2 GiB (row offsets are 32-bit)");
+    if (!R && rs * (int64_t)H >= ((int64_t)1 << 31)) return fail(TSD_E_INVALID, "a frame must span less than 2 GiB (row offsets are 32-bit)");
     const int g4_all = cdiv(n_max, 4);                       // one window per warp (the generic kernel does not loop)
     int g4 = g4_all;
     if (c->k2_grid > 0 && g4 > c->k2_grid * c->sm_count) g4 = c->k2_grid * c->sm_count;     // persistent warps (the v2 kernel strides over the windows)
-#define K2_ARGS frames, H, W, rs, fs, (const int4*)coords, win_frame, n_ptr, n_max
+    if (R) {   // wide loads for the whole batch when every frame is 4-byte aligned; the entries' guard flags protect the extent's end
+        launch_k2<true>(c, g4, g4_all, frames, 0, 0, 0, 0, ch, coords, win_frame, n_ptr, n_max, D, windows, out_stride,
+                        (R->wide4 && ((uintptr_t)frames % 4) == 0) ? -1 : -2, R->d);
+        return check_launch(c, "k2_crop_resize");
+    }
     // aligned 32-bit tap loads need 4-byte aligned frames and strides and the number of frames (the last row of the last frame keeps byte loads)
     const int wide_last = (nframes > 0 && ((uintptr_t)frames % 4) == 0 && rs % 4 == 0 && fs % 4 == 0) ? nframes - 1 : -2;
-    if (ch == 3 && D == 25) k2_crop_resize_v2_kernel<3, 25><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, wide_last);
-    else if (ch == 3 && D == 32) k2_crop_resize_v2_kernel<3, 32><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, wide_last);
-    else if (ch == 1 && D == 25) k2_crop_resize_v2_kernel<1, 25><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, -2);
-    else if (ch == 1 && D == 32) k2_crop_resize_v2_kernel<1, 32><<<g4, 128, 0, c->cur>>>(K2_ARGS, windows, out_stride, -2);
-    else if (ch == 3) k2_crop_resize_kernel<3><<<g4_all, 128, 0, c->cur>>>(K2_ARGS, D, windows, out_stride);      // other window sizes: generic kernel
-    else k2_crop_resize_kernel<1><<<g4_all, 128, 0, c->cur>>>(K2_ARGS, D, windows, out_stride);
-#undef K2_ARGS
+    launch_k2<false>(c, g4, g4_all, frames, H, W, rs, fs, ch, coords, win_frame, n_ptr, n_max, D, windows, out_stride, wide_last, nullptr);
     return check_launch(c, "k2_crop_resize");
 }
 
@@ -634,13 +697,19 @@ static inline int pair_row_words(int max_n) {
 }
 
 // K1 count (+ scan by its last CTA) + compact -> coords/win_frame/win_offsets in context scratch or caller buffers
+// geom != NULL: each frame's own H and W for the crop test (frames of different sizes)
 static int dev_windows_index(tsd_ctx* c, const int32_t* boxes, const int32_t* box_offsets, int nframes, int H, int W, double enlarge,
-                             int32_t* counts, int32_t* win_offsets, int32_t* coords, int32_t* win_frame) {
+                             int32_t* counts, int32_t* win_offsets, int32_t* coords, int32_t* win_frame, const FrameGeom* geom = nullptr) {
     const double pm1 = enlarge - 1.0;
-    k1_count_kernel<<<cdiv((int64_t)nframes * 32, 128), 128, 0, c->cur>>>((const int4*)boxes, box_offsets, nframes, H, W, pm1, c->cfg.aspect_lo, c->cfg.aspect_hi, counts,
-                                                                           win_offsets, c->d_tickets + c->ticket_base);
+    const int g = cdiv((int64_t)nframes * 32, 128);
+    if (geom) k1_count_kernel<true><<<g, 128, 0, c->cur>>>((const int4*)boxes, box_offsets, nframes, 0, 0, pm1, c->cfg.aspect_lo, c->cfg.aspect_hi, counts,
+                                                           win_offsets, c->d_tickets + c->ticket_base, geom);
+    else k1_count_kernel<<<g, 128, 0, c->cur>>>((const int4*)boxes, box_offsets, nframes, H, W, pm1, c->cfg.aspect_lo, c->cfg.aspect_hi, counts,
+                                                win_offsets, c->d_tickets + c->ticket_base);
     TRY(check_launch(c, "k1_count"));
-    k1_compact_kernel<<<cdiv((int64_t)nframes * 32, 128), 128, 0, c->cur>>>((const int4*)boxes, box_offsets, nframes, H, W, pm1, c->cfg.aspect_lo, c->cfg.aspect_hi, win_offsets, (int4*)coords, win_frame);
+    if (geom) k1_compact_kernel<true><<<g, 128, 0, c->cur>>>((const int4*)boxes, box_offsets, nframes, 0, 0, pm1, c->cfg.aspect_lo, c->cfg.aspect_hi, win_offsets,
+                                                             (int4*)coords, win_frame, geom);
+    else k1_compact_kernel<<<g, 128, 0, c->cur>>>((const int4*)boxes, box_offsets, nframes, H, W, pm1, c->cfg.aspect_lo, c->cfg.aspect_hi, win_offsets, (int4*)coords, win_frame);
     return check_launch(c, "k1_compact");
 }
 
@@ -860,6 +929,79 @@ int tsd_windows(tsd_ctx* c, const uint8_t* frames, int nframes, int H, int W, in
     TRY(s.alloc(&dw, (size_t)nb * D * D * 3));
     TRY(dev_windows_index(c, (int32_t*)db, (int32_t*)dbo, nframes, H, W, enlarge, (int32_t*)dcnt, (int32_t*)dwo, (int32_t*)dc, (int32_t*)dwf));
     TRY(dev_crop_resize(c, (uint8_t*)df, H, W, row_stride, frame_stride, 3, (int32_t*)dc, (int32_t*)dwf, (int32_t*)dwo + nframes, nb, D, (uint8_t*)dw, D * D * 3, nframes));
+    TRY(s.out(win_offsets, dwo, (size_t)(nframes + 1) * 4));
+    CU(cudaStreamSynchronize(c->stream));
+    const int tot = win_offsets[nframes];
+    if (total) *total = tot;
+    if (tot) {
+        if (!windows || !coords) return fail(TSD_E_INVALID, "NULL output");
+        TRY(s.out(windows, dw, (size_t)tot * D * D * 3));
+        TRY(s.out(coords, dc, (size_t)tot * 16));
+        CU(cudaStreamSynchronize(c->stream));
+    }
+    return TSD_OK;
+}
+
+int tsd_crop_resize_ragged(tsd_ctx* c, const uint8_t* base, const tsd_frame_desc* table, int nframes, int channels, const int32_t* coords,
+                           const int32_t* win_frame, int n, int D, uint8_t* windows, int mem) {
+    if (!c || !base || n < 0 || (channels != 1 && channels != 3) || D < 2 || D > kMaxD) return fail(TSD_E_INVALID, "bad argument");
+    Ragged R;
+    TRY(make_ragged(table, nframes, channels, &R));
+    if (n && (!coords || !win_frame || !windows)) return fail(TSD_E_INVALID, "NULL argument");
+    CU(cudaSetDevice(c->device));
+    if (mem == TSD_MEM_DEVICE) {                             // (empty crops: all-zero windows, as tsd_crop_resize)
+        Stage s(c);
+        void* dg;
+        TRY(s.in(R.geom.data(), R.geom.size() * sizeof(FrameGeom), &dg));
+        R.d = (const FrameGeom*)dg;
+        return dev_crop_resize(c, base, 0, 0, 0, 0, channels, coords, win_frame, nullptr, n, D, windows, D * D * channels, nframes, &R);
+    }
+    for (int i = 0; i < n; i++) {
+        const int32_t* q = coords + 4 * (size_t)i;
+        if (win_frame[i] < 0 || win_frame[i] >= nframes) return fail(TSD_E_INVALID, "window %d: frame %d not in [0,%d)", i, win_frame[i], nframes);
+        const int H = table[win_frame[i]].H, W = table[win_frame[i]].W;
+        if (q[0] < 0 || q[1] < 0 || q[2] < 0 || q[3] < 0) return fail(TSD_E_INVALID, "window %d: negative coordinate (numpy slicing would wrap around)", i);
+        if (std::min(q[2], W) <= std::min(q[0], W) || std::min(q[3], H) <= std::min(q[1], H))
+            return fail(TSD_E_INVALID, "window %d: empty crop after clipping to the frame (cv2.resize would raise)", i);
+    }
+    Stage s(c);
+    void *df, *dg, *dc, *dwf, *dw;
+    TRY(s.in(base, (size_t)R.extent, &df));
+    TRY(s.in(R.geom.data(), R.geom.size() * sizeof(FrameGeom), &dg));
+    TRY(s.in(coords, (size_t)n * 16, &dc));
+    TRY(s.in(win_frame, (size_t)n * 4, &dwf));
+    TRY(s.alloc(&dw, (size_t)n * D * D * channels));
+    R.d = (const FrameGeom*)dg;
+    TRY(dev_crop_resize(c, (uint8_t*)df, 0, 0, 0, 0, channels, (int32_t*)dc, (int32_t*)dwf, nullptr, n, D, (uint8_t*)dw, D * D * channels, nframes, &R));
+    TRY(s.out(windows, dw, (size_t)n * D * D * channels));
+    CU(cudaStreamSynchronize(c->stream));
+    return TSD_OK;
+}
+
+int tsd_windows_ragged(tsd_ctx* c, const uint8_t* base, const tsd_frame_desc* table, int nframes, const int32_t* boxes, const int32_t* box_offsets,
+                       double enlarge, int D, uint8_t* windows, int32_t* coords, int32_t* win_offsets, int32_t* total, int mem) {
+    if (!c || !base || !box_offsets || !win_offsets || D < 2 || D > kMaxD) return fail(TSD_E_INVALID, "bad argument");
+    Ragged R;
+    TRY(make_ragged(table, nframes, 3, &R));
+    if (mem != TSD_MEM_HOST) return fail(TSD_E_INVALID, "tsd_windows_ragged takes host pointers; use tsd_enqueue_frames_ragged for device-resident batches");
+    CU(cudaSetDevice(c->device));
+    const int nb = box_offsets[nframes];
+    if (nb < 0 || (nb && !boxes)) return fail(TSD_E_INVALID, "bad boxes");
+    for (int f = 0; f < nframes; f++) if (box_offsets[f + 1] < box_offsets[f]) return fail(TSD_E_INVALID, "box_offsets must not decrease (frame %d)", f);
+    Stage s(c);
+    void *df, *dg, *db, *dbo, *dcnt, *dwo, *dc, *dwf, *dw;
+    TRY(s.in(base, (size_t)R.extent, &df));
+    TRY(s.in(R.geom.data(), R.geom.size() * sizeof(FrameGeom), &dg));
+    TRY(s.in(boxes, (size_t)nb * 16, &db));
+    TRY(s.in(box_offsets, (size_t)(nframes + 1) * 4, &dbo));
+    TRY(s.alloc(&dcnt, (size_t)nframes * 4));
+    TRY(s.alloc(&dwo, (size_t)(nframes + 1) * 4));
+    TRY(s.alloc(&dc, (size_t)nb * 16));
+    TRY(s.alloc(&dwf, (size_t)nb * 4));
+    TRY(s.alloc(&dw, (size_t)nb * D * D * 3));
+    R.d = (const FrameGeom*)dg;
+    TRY(dev_windows_index(c, (int32_t*)db, (int32_t*)dbo, nframes, 0, 0, enlarge, (int32_t*)dcnt, (int32_t*)dwo, (int32_t*)dc, (int32_t*)dwf, R.d));
+    TRY(dev_crop_resize(c, (uint8_t*)df, 0, 0, 0, 0, 3, (int32_t*)dc, (int32_t*)dwf, (int32_t*)dwo + nframes, nb, D, (uint8_t*)dw, D * D * 3, nframes, &R));
     TRY(s.out(win_offsets, dwo, (size_t)(nframes + 1) * 4));
     CU(cudaStreamSynchronize(c->stream));
     const int tot = win_offsets[nframes];
@@ -1385,7 +1527,8 @@ int tsd_knn_predict(tsd_ctx* c, const float* X, int n, double* Z, int32_t* label
 // M = the batch's rows of the pair-class bit matrix.
 static int enqueue_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, int W, int64_t row_stride, int64_t frame_stride,
                          const int32_t* d_boxes, const int32_t* d_box_offsets, int maxb, const tsd_ctx::Batch& B, uint32_t* M, int32_t* todo,
-                         const uint8_t* host_src = nullptr /* page-locked host frames (device pointer): staged into d_frames (the mirror) after K1 */) {
+                         const uint8_t* host_src = nullptr /* page-locked host frames (device pointer): staged into d_frames (the mirror) after K1 */,
+                         const Ragged* R = nullptr /* frames of different sizes (R->d on the device); H .. frame_stride unused */) {
     const int D = c->cfg.window, npx = D * D, nbytes = npx * 3, ws = win_stride(npx, 3), es = ent_stride(npx);
     const int ms = (npx + 15) & ~15, NW = (npx + 31) >> 5;     // mask byte stride (padded), mask words
     const int cf = B.nframes, nb = B.nbcap, fo = B.fo;
@@ -1411,20 +1554,23 @@ static int enqueue_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, i
     const bool stagger = B.in_slot && c->stagger;
     mark(c, "start");
     // K1: candidate loop of MSERTrafficSignDetector (DET:116-120)
-    TRY(dev_windows_index(c, d_boxes, d_box_offsets, cf, H, W, c->cfg.enlarge, cnt, winoff, coords, winframe));
+    TRY(dev_windows_index(c, d_boxes, d_box_offsets, cf, H, W, c->cfg.enlarge, cnt, winoff, coords, winframe, R ? R->d : nullptr));
     mark(c, "k1_expand_filter");
     if (host_src) {                                          // every 32-byte sector the ROIs touch crosses PCIe once, into the mirror
-        const int wpr = (cdiv((int64_t)W * 3, 32) + 31) / 32;
-        const int64_t nwords = (int64_t)cf * H * wpr;
+        const int wpr = R ? 0 : (cdiv((int64_t)W * 3, 32) + 31) / 32;
+        const int64_t nwords = R ? R->words : (int64_t)cf * H * wpr;
         uint32_t* stagemap = (uint32_t*)c->b_stagemap[B.sidx].p;
         CU(cudaMemsetAsync(stagemap, 0, (size_t)nwords * 4, c->cur));
         if (nb > 0) {
-            stage_mark_kernel<<<cdiv((int64_t)nb * 32, 128), 128, 0, c->cur>>>((const int4*)coords, winframe, d_nwin, nb, H, W, D, wpr, stagemap);
+            const int gm = cdiv((int64_t)nb * 32, 128);
+            if (R) stage_mark_kernel<true><<<gm, 128, 0, c->cur>>>((const int4*)coords, winframe, d_nwin, nb, 0, 0, D, 0, stagemap, R->d);
+            else stage_mark_kernel<<<gm, 128, 0, c->cur>>>((const int4*)coords, winframe, d_nwin, nb, H, W, D, wpr, stagemap);
             TRY(check_launch(c, "stage_mark"));
             int g = cdiv(nwords, 256);
             if (g > c->sm_count * c->stage_ctas) g = c->sm_count * c->stage_ctas;
-            stage_copy_kernel<<<g, 256, 0, c->cur>>>(host_src, row_stride, frame_stride, H, W * 3, wpr, nwords, stagemap,
-                                                     (uint8_t*)d_frames, c->d_staged);
+            if (R) stage_copy_kernel<true><<<g, 256, 0, c->cur>>>(host_src, 0, 0, 0, 0, 0, nwords, stagemap, (uint8_t*)d_frames, c->d_staged, R->d, cf);
+            else stage_copy_kernel<<<g, 256, 0, c->cur>>>(host_src, row_stride, frame_stride, H, W * 3, wpr, nwords, stagemap,
+                                                          (uint8_t*)d_frames, c->d_staged);
             TRY(check_launch(c, "stage_copy"));
         }
         // PCIe is the serial resource of a host-staged batch: the next batch's staging may start as soon as this one's has ended
@@ -1432,7 +1578,7 @@ static int enqueue_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, i
         mark(c, "stage_h2d");
     }
     // K2 (DET:123-124)
-    TRY(dev_crop_resize(c, d_frames, H, W, row_stride, frame_stride, 3, coords, winframe, d_nwin, nb, D, windows, ws, cf));
+    TRY(dev_crop_resize(c, d_frames, H, W, row_stride, frame_stride, 3, coords, winframe, d_nwin, nb, D, windows, ws, cf, R));
     mark(c, "k2_crop_resize");
     // K5 (DET:127-129)
     TRY(dev_hist(c, windows, d_nwin, nb, npx, ws, entries, meta, energy, (int64_t)cap));
@@ -1515,13 +1661,17 @@ static int enqueue_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, i
 // used goes first).  A cycle of more than kGraphCap keys therefore always runs eagerly instead of capturing on every call.
 static int run_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, int W, int64_t row_stride, int64_t frame_stride,
                      const int32_t* d_boxes, const int32_t* d_box_offsets, int maxb, const tsd_ctx::Batch& B, uint32_t* M, int32_t* todo,
-                     const uint8_t* host_src) {
+                     const uint8_t* host_src, const Ragged* R) {
     if (!c->use_graph || c->profiling)
-        return enqueue_chain(c, mode, d_frames, H, W, row_stride, frame_stride, d_boxes, d_box_offsets, maxb, B, M, todo, host_src);
+        return enqueue_chain(c, mode, d_frames, H, W, row_stride, frame_stride, d_boxes, d_box_offsets, maxb, B, M, todo, host_src, R);
     const std::vector<uint64_t> key = {(uint64_t)mode, (uint64_t)(uintptr_t)d_frames, (uint64_t)B.nframes, (uint64_t)H, (uint64_t)W, (uint64_t)row_stride,
                                        (uint64_t)frame_stride, (uint64_t)(uintptr_t)d_boxes, (uint64_t)(uintptr_t)d_box_offsets, (uint64_t)B.nbcap, (uint64_t)maxb,
                                        (uint64_t)B.wo, (uint64_t)B.fo, (uint64_t)B.sidx, (uint64_t)(uintptr_t)M, (uint64_t)(uintptr_t)todo,
-                                       (uint64_t)c->ticket_base, c->gen, (uint64_t)c->keep_masks, (uint64_t)c->use_gram, (uint64_t)(uintptr_t)host_src, (uint64_t)c->fold_per_sm_cap, (uint64_t)c->k2_grid, (uint64_t)c->stagger, (uint64_t)c->stage_ctas};
+                                       (uint64_t)c->ticket_base, c->gen, (uint64_t)c->keep_masks, (uint64_t)c->use_gram, (uint64_t)(uintptr_t)host_src, (uint64_t)c->fold_per_sm_cap, (uint64_t)c->k2_grid, (uint64_t)c->stagger, (uint64_t)c->stage_ctas,
+                                       // a table batch: its slot's table buffer, bitmap size, mirror extent and wide / bytes choice (the
+                                       // table's contents are read by the kernels at run time and may change between replays)
+                                       (uint64_t)(uintptr_t)(R ? R->d : nullptr), (uint64_t)(R ? R->words : 0), (uint64_t)(R ? R->extent : 0),
+                                       (uint64_t)(R && R->wide4 && ((uintptr_t)d_frames % 4) == 0)};
     c->graph_clock++;
     for (auto& g : c->graphs)
         if (g.key == key) {
@@ -1535,12 +1685,12 @@ static int run_chain(tsd_ctx* c, int mode, const uint8_t* d_frames, int H, int W
     if (seen == c->seen_keys.end()) {                        // first sighting: run it eagerly (one-off calls never pay for an instantiation)
         if (c->seen_keys.size() >= tsd_ctx::kGraphCap) c->seen_keys.erase(c->seen_keys.begin());
         c->seen_keys.push_back(key);
-        return enqueue_chain(c, mode, d_frames, H, W, row_stride, frame_stride, d_boxes, d_box_offsets, maxb, B, M, todo, host_src);
+        return enqueue_chain(c, mode, d_frames, H, W, row_stride, frame_stride, d_boxes, d_box_offsets, maxb, B, M, todo, host_src, R);
     }
     c->seen_keys.erase(seen);
     const int64_t l0 = c->launches;
     CU(cudaStreamBeginCapture(c->cur, cudaStreamCaptureModeThreadLocal));
-    const int rc = enqueue_chain(c, mode, d_frames, H, W, row_stride, frame_stride, d_boxes, d_box_offsets, maxb, B, M, todo, host_src);
+    const int rc = enqueue_chain(c, mode, d_frames, H, W, row_stride, frame_stride, d_boxes, d_box_offsets, maxb, B, M, todo, host_src, R);
     cudaGraph_t graph = nullptr;
     const cudaError_t ee = cudaStreamEndCapture(c->cur, &graph);
     if (rc != TSD_OK) { if (graph) cudaGraphDestroy(graph); return rc; }
@@ -1588,12 +1738,15 @@ static int check_mode_state(const tsd_ctx* c, int mode) {
 
 // host_src != NULL: d_frames is ignored, the frames are page-locked host memory (host_src = their device pointer) and are staged
 // ROI sector by ROI sector into the context's mirror, which the chain then reads.
+// R != NULL: frames of different sizes (a validated table, nframes = R->nframes); H, W, row_stride and frame_stride are not used.  The
+// table is copied into the batch's slot buffer on the batch's stream, outside any graph capture.
 static int enqueue_impl(tsd_ctx* c, int mode, const uint8_t* d_frames, int nframes, int H, int W, int64_t row_stride, int64_t frame_stride,
-                        const int32_t* d_boxes, const int32_t* d_box_offsets, int nb, int max_boxes_per_frame, const uint8_t* host_src) {
+                        const int32_t* d_boxes, const int32_t* d_box_offsets, int nb, int max_boxes_per_frame, const uint8_t* host_src,
+                        Ragged* R = nullptr) {
     if (host_src) d_frames = host_src;                       // (argument checks below)
-    if (!c || !d_frames || !d_box_offsets || nframes < 1 || nb < 0 || H < 1 || W < 1) return fail(TSD_E_INVALID, "bad argument");
+    if (!c || !d_frames || !d_box_offsets || nframes < 1 || nb < 0 || (!R && (H < 1 || W < 1))) return fail(TSD_E_INVALID, "bad argument");
     TRY(check_mode(mode));
-    if (row_stride < (int64_t)W * 3 || frame_stride < row_stride * (H - 1) + (int64_t)W * 3) return fail(TSD_E_INVALID, "bad strides");
+    if (!R && (row_stride < (int64_t)W * 3 || frame_stride < row_stride * (H - 1) + (int64_t)W * 3)) return fail(TSD_E_INVALID, "bad strides");
     if (nframes >= kMaxBatchFrames) return fail(TSD_E_INVALID, "%d frames: a batch holds fewer than 2^23 (the K5 work lists keep frame << 8 in an int32)", nframes);
     const int D = c->cfg.window, npx = D * D, ws = win_stride(npx, 3), es = ent_stride(npx);
     const int ms = (npx + 15) & ~15, NW = (npx + 31) >> 5;
@@ -1681,10 +1834,21 @@ static int enqueue_impl(tsd_ctx* c, int mode, const uint8_t* d_frames, int nfram
     if (host_src) {
         const int wpr = (cdiv((int64_t)W * 3, 32) + 31) / 32;
         const int ms_slot = ov ? c->slot : 0;                // (a grow frees + reallocates: cudaFree waits for the device)
-        TRY(ensure(c, c->b_mirror[ms_slot], (size_t)frame_stride * (nframes - 1) + (size_t)row_stride * (H - 1) + (size_t)W * 3 + 64));
-        TRY(ensure(c, c->b_stagemap[ms_slot], (size_t)nframes * H * wpr * 4));
+        TRY(ensure(c, c->b_mirror[ms_slot], (R ? (size_t)R->extent : (size_t)frame_stride * (nframes - 1) + (size_t)row_stride * (H - 1) + (size_t)W * 3) + 64));
+        TRY(ensure(c, c->b_stagemap[ms_slot], (R ? (size_t)R->words : (size_t)nframes * H * wpr) * 4));
         d_frames = (const uint8_t*)c->b_mirror[ms_slot].p;
     }
+    const int gslot = ov ? c->slot : 0;                      // the table's buffer: one per scratch slot, like the mirrors
+    if (R) {
+        TRY(ensure(c, c->b_geom[gslot], R->geom.size() * sizeof(FrameGeom)));
+        R->d = (const FrameGeom*)c->b_geom[gslot].p;
+    }
+    // (pageable source: cudaMemcpyAsync has copied the table out of R->geom when it returns; the previous batch of the slot ran on the
+    // same stream, or the batch's stream waits for it, so the buffer is rewritten only after that batch has read it)
+    auto copy_table = [&]() -> int {
+        if (R) CU(cudaMemcpyAsync((void*)R->d, R->geom.data(), R->geom.size() * sizeof(FrameGeom), cudaMemcpyHostToDevice, c->cur));
+        return TSD_OK;
+    };
     uint32_t* M = (uint32_t*)c->b_pairs.p + m_off;
     int32_t* todo = (int32_t*)c->b_gramdone.p + todo_off;
     int rc = TSD_OK;
@@ -1698,12 +1862,14 @@ static int enqueue_impl(tsd_ctx* c, int mode, const uint8_t* d_frames, int nfram
         // TSD_STAGGER: the front half of this batch starts when the previous batch's has ended (the event enqueue_chain records).
         // Waited here, on the stream, for a captured graph as well: the graph then holds only the record, as an external event node.
         if (c->stagger) CU(cudaStreamWaitEvent(c->cur, c->ev_w1[sl ^ 1], 0));
-        rc = run_chain(c, mode, d_frames, H, W, row_stride, frame_stride, d_boxes, d_box_offsets, max_boxes_per_frame, B, M, todo, host_src);
+        rc = copy_table();
+        if (rc == TSD_OK) rc = run_chain(c, mode, d_frames, H, W, row_stride, frame_stride, d_boxes, d_box_offsets, max_boxes_per_frame, B, M, todo, host_src, R);
         CU(cudaEventRecord(c->ev_join[sl], c->os[sl]));
         c->pending_join = sl;
     } else {
         c->cur = c->stream;
-        rc = run_chain(c, mode, d_frames, H, W, row_stride, frame_stride, d_boxes, d_box_offsets, max_boxes_per_frame, B, M, todo, host_src);
+        rc = copy_table();
+        if (rc == TSD_OK) rc = run_chain(c, mode, d_frames, H, W, row_stride, frame_stride, d_boxes, d_box_offsets, max_boxes_per_frame, B, M, todo, host_src, R);
     }
     c->cur = c->stream;
     c->ticket_base = 16;
@@ -1811,10 +1977,19 @@ int tsd_fetch_previous(tsd_ctx* c, tsd_detection* det, int det_cap, int32_t* nde
     return rc;
 }
 
-int tsd_detect_frames(tsd_ctx* c, int mode, const uint8_t* frames, int nframes, int H, int W, int64_t row_stride, int64_t frame_stride,
-                      const int32_t* boxes, const int32_t* box_offsets, tsd_detection* det, int det_cap, int32_t* ndet, int32_t* counts, int mem) {
-    if (!c || !frames || !box_offsets || nframes < 1 || H < 1 || W < 1) return fail(TSD_E_INVALID, "bad argument");
-    if (row_stride < (int64_t)W * 3 || frame_stride < row_stride * (H - 1) + (int64_t)W * 3) return fail(TSD_E_INVALID, "bad strides");
+int tsd_enqueue_frames_ragged(tsd_ctx* c, int mode, const uint8_t* d_base, const tsd_frame_desc* table, int nframes, const int32_t* d_boxes,
+                              const int32_t* d_box_offsets, int nb, int max_boxes_per_frame) {
+    if (!c) return fail(TSD_E_INVALID, "ctx is NULL");
+    Ragged R;
+    TRY(make_ragged(table, nframes, 3, &R));
+    return enqueue_impl(c, mode, d_base, nframes, 0, 0, 0, 0, d_boxes, d_box_offsets, nb, max_boxes_per_frame, nullptr, &R);
+}
+
+// The body of tsd_detect_frames and tsd_detect_frames_ragged.  table != NULL: frames of different sizes over `frames` (R = the whole
+// table, validated by the caller); H, W, row_stride and frame_stride are then not used.
+static int detect_impl(tsd_ctx* c, int mode, const uint8_t* frames, int nframes, int H, int W, int64_t row_stride, int64_t frame_stride,
+                       const tsd_frame_desc* table, Ragged* R, const int32_t* boxes, const int32_t* box_offsets, tsd_detection* det, int det_cap,
+                       int32_t* ndet, int32_t* counts, int mem) {
     TRY(check_mode(mode));
     TRY(check_mode_state(c, mode));
     CU(cudaSetDevice(c->device));
@@ -1822,7 +1997,7 @@ int tsd_detect_frames(tsd_ctx* c, int mode, const uint8_t* frames, int nframes, 
         int32_t nb = 0;
         CU(cudaMemcpyAsync(&nb, box_offsets + nframes, 4, cudaMemcpyDeviceToHost, c->stream));
         CU(cudaStreamSynchronize(c->stream));
-        TRY(tsd_enqueue_frames(c, mode, frames, nframes, H, W, row_stride, frame_stride, boxes, box_offsets, nb, 0));
+        TRY(enqueue_impl(c, mode, frames, nframes, H, W, row_stride, frame_stride, boxes, box_offsets, nb, 0, nullptr, R));
         return tsd_fetch_detections(c, det, det_cap, ndet, counts);
     }
     const int nb = box_offsets[nframes];
@@ -1839,11 +2014,12 @@ int tsd_detect_frames(tsd_ctx* c, int mode, const uint8_t* frames, int nframes, 
     const int32_t* d_off = (const int32_t*)c->b_hoff.p;
     int32_t tot[4] = {0, 0, 0, 0};
     int nd_total = 0;
-    auto run_chunk = [&](const uint8_t* d_frames, int f0, int cf, const uint8_t* host_src = nullptr) -> int {
+    auto run_chunk = [&](const uint8_t* d_frames, int f0, int cf, const uint8_t* host_src = nullptr, Ragged* Rc = nullptr) -> int {
         int max_n = 0;
         for (int f = f0; f < f0 + cf; f++) max_n = box_offsets[f + 1] - box_offsets[f] > max_n ? box_offsets[f + 1] - box_offsets[f] : max_n;
         // offsets stay absolute: the kernels index `boxes` with them, so the base pointer is the whole box array
-        return enqueue_impl(c, mode, d_frames, cf, H, W, row_stride, frame_stride, d_boxes, d_off + f0, box_offsets[f0 + cf] - box_offsets[f0], max_n > 0 ? max_n : 1, host_src);
+        return enqueue_impl(c, mode, d_frames, cf, H, W, row_stride, frame_stride, d_boxes, d_off + f0, box_offsets[f0 + cf] - box_offsets[f0], max_n > 0 ? max_n : 1,
+                            host_src, Rc);
     };
     auto fetch_chunk = [&](int f0) -> int {
         int32_t nd = 0, cnt[4];
@@ -1864,7 +2040,8 @@ int tsd_detect_frames(tsd_ctx* c, int mode, const uint8_t* frames, int nframes, 
         cudaPointerAttributes at;
         if (cudaPointerGetAttributes(&at, frames) == cudaSuccess && at.type == cudaMemoryTypeHost && at.devicePointer) {
             const uint8_t* hp = (const uint8_t*)at.devicePointer;
-            const bool stage = c->stage_rois && ((uintptr_t)hp % 16 == 0) && row_stride % 16 == 0 && frame_stride % 16 == 0 && ((int64_t)W * 3) % 16 == 0;
+            const bool layout16 = table ? R->stage16 : (row_stride % 16 == 0 && frame_stride % 16 == 0 && ((int64_t)W * 3) % 16 == 0);
+            const bool stage = c->stage_rois && ((uintptr_t)hp % 16 == 0) && layout16;
             const int SC = c->stage_chunk;
             if (stage && c->overlap && c->profiling != 1 && SC > 0 && nframes >= 2 * SC) {
                 // Chunks of SC frames through the two scratch slots: the staging copy of chunk k+1 (PCIe-bound, a few resident warps)
@@ -1874,7 +2051,13 @@ int tsd_detect_frames(tsd_ctx* c, int mode, const uint8_t* frames, int nframes, 
                 const int CFc = (nframes + nchunks - 1) / nchunks;
                 for (int f0 = 0; f0 < nframes; f0 += CFc) {
                     const int cf = nframes - f0 < CFc ? nframes - f0 : CFc;
-                    TRY(run_chunk(nullptr, f0, cf, hp + (size_t)f0 * frame_stride));
+                    if (table) {                             // the chunk's entries, relative to its lowest offset: its mirror spans only them
+                        Ragged sub;
+                        TRY(make_ragged(table + f0, cf, 3, &sub, true));
+                        TRY(run_chunk(nullptr, f0, cf, hp + sub.min_offset, &sub));
+                    } else {
+                        TRY(run_chunk(nullptr, f0, cf, hp + (size_t)f0 * frame_stride));
+                    }
                     if (f_prev >= 0) {
                         int32_t nd = 0, cnt[4];
                         const int room = det_cap - nd_total;
@@ -1894,7 +2077,7 @@ int tsd_detect_frames(tsd_ctx* c, int mode, const uint8_t* frames, int nframes, 
                 if (rc_chunks != TSD_OK) return fail(TSD_E_NOMEM, "det_cap %d < %d detections", det_cap, nd_total);
                 return TSD_OK;
             }
-            TRY(stage ? run_chunk(nullptr, 0, nframes, hp) : run_chunk(hp, 0, nframes));
+            TRY(stage ? run_chunk(nullptr, 0, nframes, hp, R) : run_chunk(hp, 0, nframes, nullptr, R));
             const int rc = fetch_chunk(0);
             *ndet = nd_total;
             if (counts) for (int i = 0; i < 4; i++) counts[i] = tot[i];
@@ -1902,16 +2085,40 @@ int tsd_detect_frames(tsd_ctx* c, int mode, const uint8_t* frames, int nframes, 
         }
         cudaGetLastError();
     }
-    // pageable frames: chunked, double-buffered whole-frame copies; the H2D copy of chunk k+1 (copy stream) overlaps the chain of chunk k
+    // pageable frames: chunked, double-buffered copies; the H2D copy of chunk k+1 (copy stream) overlaps the chain of chunk k.  Uniform
+    // frames are copied whole (one copy per chunk); a table's frames row by row (one 2D copy per entry) into the chunk's staging
+    // buffer, packed at 16-byte aligned offsets with rows of 3 W rounded up to 16 bytes, and the chunk runs with that packed table.
     const int CF = c->chunk_frames < nframes ? c->chunk_frames : nframes;
     const int nchunks = (nframes + CF - 1) / CF;
     const size_t frame_bytes = (size_t)row_stride * (H - 1) + (size_t)W * 3;
     auto chunk_bytes = [&](int cf) { return ((size_t)frame_stride * (cf - 1) + frame_bytes + 15) & ~(size_t)15; };
-    for (int i = 0; i < (nchunks > 1 ? 2 : 1); i++) TRY(ensure(c, c->b_stage[i], chunk_bytes(CF)));
+    std::vector<tsd_frame_desc> packed;
+    if (table) {
+        packed.resize(nframes);
+        size_t need[2] = {0, 0};
+        for (int k = 0; k < nchunks; k++) {
+            size_t o = 0;
+            for (int f = k * CF; f < nframes && f < (k + 1) * CF; f++) {
+                const int64_t prs = ((int64_t)table[f].W * 3 + 15) & ~(int64_t)15;
+                packed[f] = {(int64_t)o, prs, table[f].H, table[f].W};
+                o += ((size_t)prs * table[f].H + 15) & ~(size_t)15;
+            }
+            need[k & 1] = std::max(need[k & 1], o);
+        }
+        for (int i = 0; i < (nchunks > 1 ? 2 : 1); i++) TRY(ensure(c, c->b_stage[i], need[i]));
+    } else {
+        for (int i = 0; i < (nchunks > 1 ? 2 : 1); i++) TRY(ensure(c, c->b_stage[i], chunk_bytes(CF)));
+    }
     auto issue_copy = [&](int k) -> int {
         const int slot = k & 1, f0 = k * CF, cf = nframes - f0 < CF ? nframes - f0 : CF;
         if (k >= 2) CU(cudaStreamWaitEvent(c->copy_stream, c->ev_consumed[slot], 0));
-        CU(cudaMemcpyAsync(c->b_stage[slot].p, frames + (size_t)f0 * frame_stride, (size_t)frame_stride * (cf - 1) + frame_bytes, cudaMemcpyHostToDevice, c->copy_stream));
+        if (table) {
+            for (int f = f0; f < f0 + cf; f++)
+                CU(cudaMemcpy2DAsync((uint8_t*)c->b_stage[slot].p + packed[f].offset, (size_t)packed[f].row_stride, frames + table[f].offset,
+                                     (size_t)table[f].row_stride, (size_t)table[f].W * 3, (size_t)table[f].H, cudaMemcpyHostToDevice, c->copy_stream));
+        } else {
+            CU(cudaMemcpyAsync(c->b_stage[slot].p, frames + (size_t)f0 * frame_stride, (size_t)frame_stride * (cf - 1) + frame_bytes, cudaMemcpyHostToDevice, c->copy_stream));
+        }
         CU(cudaEventRecord(c->ev_copied[slot], c->copy_stream));
         return TSD_OK;
     };
@@ -1920,7 +2127,13 @@ int tsd_detect_frames(tsd_ctx* c, int mode, const uint8_t* frames, int nframes, 
         const int slot = k & 1, f0 = k * CF, cf = nframes - f0 < CF ? nframes - f0 : CF;
         if (k + 1 < nchunks) TRY(issue_copy(k + 1));
         CU(cudaStreamWaitEvent(c->stream, c->ev_copied[slot], 0));
-        TRY(run_chunk((const uint8_t*)c->b_stage[slot].p, f0, cf));
+        if (table) {
+            Ragged sub;
+            TRY(make_ragged(packed.data() + f0, cf, 3, &sub));
+            TRY(run_chunk((const uint8_t*)c->b_stage[slot].p, f0, cf, nullptr, &sub));
+        } else {
+            TRY(run_chunk((const uint8_t*)c->b_stage[slot].p, f0, cf));
+        }
         int rc = fetch_chunk(f0);                            // joins + synchronises the chunk's streams; the next copy is already in flight
         CU(cudaEventRecord(c->ev_consumed[slot], c->stream)); // (after the join: the batch ran on an internal stream)
         if (rc == TSD_E_NOMEM) rc_all = rc; else TRY(rc);
@@ -1930,6 +2143,21 @@ int tsd_detect_frames(tsd_ctx* c, int mode, const uint8_t* frames, int nframes, 
     if (counts) for (int i = 0; i < 4; i++) counts[i] = tot[i];
     if (rc_all != TSD_OK) return fail(TSD_E_NOMEM, "det_cap %d < %d detections", det_cap, nd_total);
     return TSD_OK;
+}
+
+int tsd_detect_frames(tsd_ctx* c, int mode, const uint8_t* frames, int nframes, int H, int W, int64_t row_stride, int64_t frame_stride,
+                      const int32_t* boxes, const int32_t* box_offsets, tsd_detection* det, int det_cap, int32_t* ndet, int32_t* counts, int mem) {
+    if (!c || !frames || !box_offsets || nframes < 1 || H < 1 || W < 1) return fail(TSD_E_INVALID, "bad argument");
+    if (row_stride < (int64_t)W * 3 || frame_stride < row_stride * (H - 1) + (int64_t)W * 3) return fail(TSD_E_INVALID, "bad strides");
+    return detect_impl(c, mode, frames, nframes, H, W, row_stride, frame_stride, nullptr, nullptr, boxes, box_offsets, det, det_cap, ndet, counts, mem);
+}
+
+int tsd_detect_frames_ragged(tsd_ctx* c, int mode, const uint8_t* base, const tsd_frame_desc* table, int nframes, const int32_t* boxes,
+                             const int32_t* box_offsets, tsd_detection* det, int det_cap, int32_t* ndet, int32_t* counts, int mem) {
+    if (!c || !base || !box_offsets) return fail(TSD_E_INVALID, "bad argument");
+    Ragged R;
+    TRY(make_ragged(table, nframes, 3, &R));
+    return detect_impl(c, mode, base, nframes, 0, 0, 0, 0, table, &R, boxes, box_offsets, det, det_cap, ndet, counts, mem);
 }
 
 }  // extern "C"

@@ -148,6 +148,21 @@ __device__ __forceinline__ void scan_by_last_block(const int32_t* counts, int n,
     if (threadIdx.x == 0) *ticket = 0;
 }
 
+// ---- frames of different sizes in one batch (the *_ragged entry points) ----------------------------------------------------------
+// The kernels that read frames (K1's crop test, K2, stage_mark, stage_copy) are templated on where the geometry comes from: TAB = false
+// reads the batch's one (H, W, row_stride, frame_stride) from kernel arguments, TAB = true reads frame f's own entry of this table
+// (the host validates every caller entry and derives the rest).  The uniform instantiations do not touch the table.
+struct FrameGeom {
+    int64_t offset;          // bytes from the batch's base to the frame's pixel (0, 0)
+    int64_t word0;           // first word of the frame in the staging bitmap (prefix sum of H * words_per_row over the table)
+    int32_t row_stride, H, W;
+    int32_t guard;           // 1: a wide K2 load on the frame's last row could reach past the table's extent (byte loads there)
+};
+static_assert(sizeof(FrameGeom) == 32, "FrameGeom layout");
+
+// words per bitmap row of the staging map for a BGR row of W pixels: one bit per 32-byte sector
+__host__ __device__ __forceinline__ int stage_words_per_row(int W) { return (((3 * W + 31) >> 5) + 31) >> 5; }
+
 // =====================================================================================================
 // K1  makeWindowBiggerOrDiscardFakeDetections  (DET:155-174 = REC:88-107), SURVEY A.1.  f64, no FMA.
 // =====================================================================================================
@@ -176,11 +191,13 @@ __global__ void k1_expand_kernel(const int4* __restrict__ boxes, int n, double p
 
 // per frame: count of aspect-passing boxes whose (frame-clipped) crop is not empty.  One warp per frame.
 // The last CTA to finish turns the counts into the CSR offsets of the windows (win_offsets [nframes + 1]).
+template <bool TAB = false>
 __global__ void k1_count_kernel(const int4* __restrict__ boxes, const int32_t* __restrict__ box_offsets, int nframes,
                                 int H, int W, double pm1, double alo, double ahi, int32_t* __restrict__ counts,
-                                int32_t* __restrict__ win_offsets, unsigned* __restrict__ ticket) {
+                                int32_t* __restrict__ win_offsets, unsigned* __restrict__ ticket, const FrameGeom* __restrict__ geom = nullptr) {
     int f = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (f < nframes) {
+        if constexpr (TAB) { H = geom[f].H; W = geom[f].W; }
         int b0 = box_offsets[f], b1 = box_offsets[f + 1], cnt = 0;
         for (int i = b0 + lane; i < b1; i += 32) {
             int4 c;
@@ -193,12 +210,14 @@ __global__ void k1_count_kernel(const int4* __restrict__ boxes, const int32_t* _
 }
 
 // order-preserving compaction: coords of passing boxes -> coords[win_offsets[f] + rank], win_frame[...] = f.
+template <bool TAB = false>
 __global__ void k1_compact_kernel(const int4* __restrict__ boxes, const int32_t* __restrict__ box_offsets, int nframes,
                                   int H, int W, double pm1, double alo, double ahi,
                                   const int32_t* __restrict__ win_offsets, int4* __restrict__ coords,
-                                  int32_t* __restrict__ win_frame) {
+                                  int32_t* __restrict__ win_frame, const FrameGeom* __restrict__ geom = nullptr) {
     int f = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (f >= nframes) return;
+    if constexpr (TAB) { H = geom[f].H; W = geom[f].W; }
     int b0 = box_offsets[f], b1 = box_offsets[f + 1], out = win_offsets[f];
     for (int base = b0; base < b1; base += 32) {
         int i = base + lane;
@@ -221,11 +240,11 @@ __global__ void k1_compact_kernel(const int4* __restrict__ boxes, const int32_t*
 // same-size copy, exact 2x2 INTER_AREA, general two-pass 11-bit fixed point (x coefficient clamp, y row clip).
 // v1: taps are gathered straight from global memory through L1 (a window's ROI is ~5 KB and stays L1-resident).
 // =====================================================================================================
-template <int C>
+template <int C, bool TAB = false>
 __global__ void __launch_bounds__(128) k2_crop_resize_kernel(
     const uint8_t* __restrict__ frames, int H, int W, int64_t row_stride, int64_t frame_stride,
     const int4* __restrict__ coords, const int32_t* __restrict__ win_frame, const int32_t* __restrict__ n_ptr, int n_max,
-    int D, uint8_t* __restrict__ windows, int out_stride) {
+    int D, uint8_t* __restrict__ windows, int out_stride, const FrameGeom* __restrict__ geom = nullptr) {
     __shared__ int16_t s_xo[4][kMaxD], s_xa0[4][kMaxD], s_xa1[4][kMaxD];
     __shared__ int16_t s_y0[4][kMaxD], s_y1[4][kMaxD], s_yb0[4][kMaxD], s_yb1[4][kMaxD];
     const int wl = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -233,9 +252,16 @@ __global__ void __launch_bounds__(128) k2_crop_resize_kernel(
     const int n = n_ptr ? min(*n_ptr, n_max) : n_max;
     if (w >= n) return;
     const int4 c = coords[w];
+    const uint8_t* fb;
+    if constexpr (TAB) {
+        const FrameGeom& g = geom[win_frame[w]];
+        fb = frames + g.offset; row_stride = g.row_stride; H = g.H; W = g.W;
+    }
     const int cx = min(c.x, W), cy = min(c.y, H);
     const int cw = min(c.z, W) - cx, ch = min(c.w, H) - cy;
-    const uint8_t* __restrict__ src = frames + (int64_t)win_frame[w] * frame_stride + (int64_t)cy * row_stride + (int64_t)cx * C;
+    const uint8_t* __restrict__ src;
+    if constexpr (TAB) src = fb + (int64_t)cy * row_stride + (int64_t)cx * C;
+    else src = frames + (int64_t)win_frame[w] * frame_stride + (int64_t)cy * row_stride + (int64_t)cx * C;
     uint8_t* __restrict__ dst = windows + (int64_t)w * out_stride;
     const int rowlen = D * C, total = D * rowlen;
     if (cw <= 0 || ch <= 0) {                                // empty crop (cv2.resize would raise; K1 never emits one): a defined, all-zero window
@@ -381,19 +407,30 @@ __device__ __forceinline__ void k2_rows_wide(const uint8_t* __restrict__ px, con
 }
 
 // One window by one warp, taps gathered straight from the frame (the body of k2_crop_resize_v2).  s_y = the warp's 32 x int4 scratch.
-template <int C, int D>
+// TAB: frame geometry from geom[win_frame[w]]; wide_last >= -1 then allows wide loads for the whole batch and the entry's guard flag
+// keeps its last row on byte loads.
+template <int C, int D, bool TAB = false>
 __device__ __forceinline__ void k2_window_gather(const uint8_t* __restrict__ frames, int H, int W, int64_t row_stride, int64_t frame_stride,
                                                  const int4* __restrict__ coords, const int32_t* __restrict__ win_frame, int w,
-                                                 uint8_t* __restrict__ windows, int out_stride, int4* s_y, int wide_last = -2) {
+                                                 uint8_t* __restrict__ windows, int out_stride, int4* s_y, int wide_last = -2,
+                                                 const FrameGeom* __restrict__ geom = nullptr) {
     const int lane = threadIdx.x & 31;
     const int4 c = coords[w];
+    const uint8_t* fb;
+    int guard;
+    if constexpr (TAB) {
+        const FrameGeom& g = geom[win_frame[w]];
+        fb = frames + g.offset; row_stride = g.row_stride; H = g.H; W = g.W; guard = g.guard;
+    }
     const int cx = min(c.x, W), cy = min(c.y, H);
     const int cw = min(c.z, W) - cx, ch = min(c.w, H) - cy;
     if (cw <= 0 || ch <= 0) {                                // empty crop (cv2.resize would raise; K1 never emits one): a defined, all-zero window
         for (int i = lane; i < out_stride; i += 32) windows[(int64_t)w * out_stride + i] = 0;
         return;
     }
-    const uint8_t* __restrict__ src = frames + (int64_t)win_frame[w] * frame_stride + (int64_t)cy * row_stride + (int64_t)cx * C;
+    const uint8_t* __restrict__ src;
+    if constexpr (TAB) src = fb + (int64_t)cy * row_stride + (int64_t)cx * C;
+    else src = frames + (int64_t)win_frame[w] * frame_stride + (int64_t)cy * row_stride + (int64_t)cx * C;
     uint8_t* __restrict__ dst = windows + (int64_t)w * out_stride + lane * C;
     if (D * D * C + lane < out_stride) windows[(int64_t)w * out_stride + D * D * C + lane] = 0;    // zero pad (< 16 bytes)
     const bool act = lane < D;
@@ -457,22 +494,25 @@ __device__ __forceinline__ void k2_window_gather(const uint8_t* __restrict__ fra
     s_y[lane] = make_int4(yr0 * (int)row_stride, yr1 * (int)row_stride, yb0, yb1);
     __syncwarp();
     // every down-scale (cw > D) has its second tap exactly one pixel to the right in every column: the tap offsets are immediates
-    if (C == 3 && wide_last >= -1 && !(win_frame[w] == wide_last && cy + ch == H)) k2_rows_wide<D>(px, s_y, xa0, xa1, dst, act);
+    bool wide;
+    if constexpr (TAB) wide = C == 3 && wide_last >= -1 && !(guard && cy + ch == H);
+    else wide = C == 3 && wide_last >= -1 && !(win_frame[w] == wide_last && cy + ch == H);
+    if (wide) k2_rows_wide<D>(px, s_y, xa0, xa1, dst, act);
     else if (__all_sync(0xffffffffu, xd1 == C)) k2_rows<C, D, true>(px, s_y, C, xa0, xa1, dst, act);
     else k2_rows<C, D, false>(px, s_y, xd1, xa0, xa1, dst, act);
 }
 
-template <int C, int D>
+template <int C, int D, bool TAB = false>
 __global__ void __launch_bounds__(128, TSD_K2_MINB) k2_crop_resize_v2_kernel(
     const uint8_t* __restrict__ frames, int H, int W, int64_t row_stride, int64_t frame_stride,
     const int4* __restrict__ coords, const int32_t* __restrict__ win_frame, const int32_t* __restrict__ n_ptr, int n_max,
-    uint8_t* __restrict__ windows, int out_stride, int wide_last) {
+    uint8_t* __restrict__ windows, int out_stride, int wide_last, const FrameGeom* __restrict__ geom = nullptr) {
     __shared__ int4 s_y[4][32];                              // per warp: (row0, row1, weight0, weight1) of every destination row
     const int wl = threadIdx.x >> 5;
     const int n = n_ptr ? min(*n_ptr, n_max) : n_max;
     const int nwarps = (gridDim.x * blockDim.x) >> 5;
     for (int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < n; w += nwarps)     // (the grid normally covers all windows: one trip)
-        k2_window_gather<C, D>(frames, H, W, row_stride, frame_stride, coords, win_frame, w, windows, out_stride, s_y[wl], wide_last);
+        k2_window_gather<C, D, TAB>(frames, H, W, row_stride, frame_stride, coords, win_frame, w, windows, out_stride, s_y[wl], wide_last, geom);
 }
 
 // =====================================================================================================
@@ -487,18 +527,27 @@ __global__ void __launch_bounds__(128, TSD_K2_MINB) k2_crop_resize_v2_kernel(
 //                device-resident mirror with the frame's own layout, which K2 then reads at HBM speed.
 // The mirror is never cleared: K2 only reads sectors that were marked (and therefore copied) in the same batch.
 // =====================================================================================================
+// TAB: frame f's bitmap starts at geom[f].word0 and has stage_words_per_row(W_f) words per row.
+template <bool TAB = false>
 __global__ void __launch_bounds__(128) stage_mark_kernel(const int4* __restrict__ coords, const int32_t* __restrict__ win_frame,
                                                          const int32_t* __restrict__ n_ptr, int n_max, int H, int W, int D, int wpr,
-                                                         uint32_t* __restrict__ bitmap) {
+                                                         uint32_t* __restrict__ bitmap, const FrameGeom* __restrict__ geom = nullptr) {
     const int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     const int n = n_ptr ? min(*n_ptr, n_max) : n_max;
     if (w >= n) return;
     const int4 c = coords[w];
+    int64_t word0;
+    if constexpr (TAB) {
+        const FrameGeom& g = geom[win_frame[w]];
+        H = g.H; W = g.W; word0 = g.word0; wpr = stage_words_per_row(W);
+    }
     const int cx = min(c.x, W), cy = min(c.y, H);
     const int cw = min(c.z, W) - cx, ch = min(c.w, H) - cy;
     if (cw <= 0 || ch <= 0) return;
     const int s0 = (3 * cx) >> 5, s1 = (3 * (cx + cw) - 1) >> 5;          // first / last 32-byte sector of the row span
-    uint32_t* fb = bitmap + (int64_t)win_frame[w] * H * wpr;
+    uint32_t* fb;
+    if constexpr (TAB) fb = bitmap + word0;
+    else fb = bitmap + (int64_t)win_frame[w] * H * wpr;
     int rows[2], nrows = 0;
     if (ch <= 2 * D) {                                       // every row of the crop (copy / 2x2 AREA / down-scales up to 2)
         if (lane < ch) rows[nrows++] = cy + lane;
@@ -524,9 +573,13 @@ __global__ void __launch_bounds__(128) stage_mark_kernel(const int4* __restrict_
 // Four non-empty bitmap words per trip: all their loads are issued before the first store, so a warp keeps up to 8 x 16 bytes per
 // lane in flight over PCIe (the copy is bound by the number of outstanding read requests, not by their size: a 128-byte L2 fetch
 // hint and spans widened to whole 128-byte lines both measured slower, DESIGN.md section 8).
+// TAB: the bitmap is the concatenation of the frames' own bitmaps (geom[f].word0, nframes entries); each lane finds the frame of
+// its word by binary search once per group of 32 words that has a set bit, and the warp reads it from the lane that owns a word.
+template <bool TAB = false>
 __global__ void __launch_bounds__(256) stage_copy_kernel(const uint8_t* __restrict__ src, int64_t row_stride, int64_t frame_stride, int H, int row_bytes,
                                                          int wpr, int64_t nwords, const uint32_t* __restrict__ bitmap, uint8_t* __restrict__ mirror,
-                                                         unsigned long long* __restrict__ bytes_out) {
+                                                         unsigned long long* __restrict__ bytes_out, const FrameGeom* __restrict__ geom = nullptr,
+                                                         int nframes = 0) {
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
     unsigned long long copied = 0;
@@ -534,6 +587,21 @@ __global__ void __launch_bounds__(256) stage_copy_kernel(const uint8_t* __restri
         const int64_t wi = base + lane;
         const uint32_t mine = wi < nwords ? __ldg(bitmap + wi) : 0u;
         unsigned nz = __ballot_sync(0xffffffffu, mine != 0u);
+        int64_t my_row = 0;                                  // TAB: byte offset of this lane's bitmap row; its length and word in the row
+        int my_rb = 0, my_wd = 0;
+        if constexpr (TAB) {
+            if (nz && wi < nwords) {
+                int lo = 0, hi = nframes - 1;                // last frame with word0 <= wi
+                while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (__ldg(&geom[mid].word0) <= wi) lo = mid; else hi = mid - 1; }
+                const FrameGeom& g = geom[lo];
+                const int wpf = stage_words_per_row(g.W);
+                const int64_t r = wi - g.word0;
+                const int row = (int)(r / wpf);
+                my_wd = (int)(r - (int64_t)row * wpf);
+                my_row = g.offset + (int64_t)row * g.row_stride;
+                my_rb = 3 * g.W;
+            }
+        }
         while (nz) {
             int64_t o[4];
             int nb[4];                                       // bytes this lane copies for word u: 0, 16 or 32
@@ -544,15 +612,25 @@ __global__ void __launch_bounds__(256) stage_copy_kernel(const uint8_t* __restri
                     const int k = __ffs(nz) - 1;
                     nz &= nz - 1;
                     const uint32_t wv = __shfl_sync(0xffffffffu, mine, k);
-                    const int64_t g = base + k;              // global word index -> (frame, row, word of the row)
-                    const int64_t fr = g / wpr;
-                    const int wd = (int)(g - fr * wpr);
-                    const int64_t f = fr / H;
-                    const int row = (int)(fr - f * H);
-                    const int off = (32 * wd + lane) * 32;   // byte offset of this lane's sector inside the row
-                    if (((wv >> lane) & 1u) && off < row_bytes) {
-                        o[u] = f * frame_stride + (int64_t)row * row_stride + off;
-                        nb[u] = min(32, row_bytes - off);
+                    if constexpr (TAB) {
+                        const int64_t rowo = __shfl_sync(0xffffffffu, my_row, k);
+                        const int rb = __shfl_sync(0xffffffffu, my_rb, k), wd = __shfl_sync(0xffffffffu, my_wd, k);
+                        const int off = (32 * wd + lane) * 32;
+                        if (((wv >> lane) & 1u) && off < rb) {
+                            o[u] = rowo + off;
+                            nb[u] = min(32, rb - off);
+                        }
+                    } else {
+                        const int64_t g = base + k;          // global word index -> (frame, row, word of the row)
+                        const int64_t fr = g / wpr;
+                        const int wd = (int)(g - fr * wpr);
+                        const int64_t f = fr / H;
+                        const int row = (int)(fr - f * H);
+                        const int off = (32 * wd + lane) * 32;   // byte offset of this lane's sector inside the row
+                        if (((wv >> lane) & 1u) && off < row_bytes) {
+                            o[u] = f * frame_stride + (int64_t)row * row_stride + off;
+                            nb[u] = min(32, row_bytes - off);
+                        }
                     }
                 }
             }

@@ -9,7 +9,7 @@ import ctypes as C
 import numpy as np
 
 from . import _capi
-from ._capi import DET_DTYPE, HOG_LEN, MEM_DEVICE, MEM_HOST, RUN_DETECT, RUN_RECOGNIZE, Config, TsdError, check, ptr
+from ._capi import DET_DTYPE, FRAME_DESC_DTYPE, HOG_LEN, MEM_DEVICE, MEM_HOST, RUN_DETECT, RUN_RECOGNIZE, Config, TsdError, check, ptr
 
 _SIMTAB = None
 
@@ -42,6 +42,36 @@ def _i32(a):
     return np.ascontiguousarray(a, np.int32)
 
 
+def is_mixed(frames):
+    """True for a list or tuple of frames that do not all have one shape (the *_ragged calls); an ndarray or a same-shape list
+    makes the uniform call."""
+    return isinstance(frames, (list, tuple)) and len({np.shape(f) for f in frames}) > 1
+
+
+def stack_if_uniform(frames):
+    """frames (a list of arrays) as one ndarray when they share a shape, else the list itself: what Context.windows /
+    crop_resize / detect_frames take either way."""
+    return frames if is_mixed(frames) else np.stack(frames)
+
+
+def frame_table(shapes, channels):
+    """Packing layout of frames of different sizes in one buffer: frame k at a 16-byte aligned offset, its rows of
+    W * channels bytes back to back.  -> (table FRAME_DESC_DTYPE [n], bytes the buffer needs)."""
+    table = np.zeros(len(shapes), FRAME_DESC_DTYPE)
+    o = 0
+    for k, (H, W) in enumerate(shapes):
+        table[k] = (o, W * channels, H, W)
+        o += (H * W * channels + 15) & ~15
+    return table, o
+
+
+def as_frame_table(table):
+    """A FRAME_DESC_DTYPE array or a sequence of (offset, row_stride, H, W) -> contiguous FRAME_DESC_DTYPE array."""
+    if isinstance(table, np.ndarray) and table.dtype == FRAME_DESC_DTYPE:
+        return np.ascontiguousarray(table)
+    return np.array([tuple(int(v) for v in e) for e in table], FRAME_DESC_DTYPE)
+
+
 class Context:
     """tsd_ctx wrapper.  flavour 'det' = x1.30 / 25x25 (DET:119,124); 'rec' = x1.15 / 32x32 (REC:54,57)."""
 
@@ -51,6 +81,7 @@ class Context:
         h = C.c_void_p()
         check(self._L.tsd_create(C.byref(h), int(device), C.byref(self.cfg)))
         self._h = h
+        self._pack_buf = None                 # page-locked buffer that lists of frames of different sizes are packed into
         self.device = int(device)
         self.D = int(self.cfg.window)
         if numpy_similarity:
@@ -62,6 +93,32 @@ class Context:
         if getattr(self, "_h", None):
             self._L.tsd_destroy(self._h)
             self._h = None
+        if getattr(self, "_pack_buf", None) is not None:
+            self._L.tsd_host_unregister(ptr(self._pack_buf))
+            self._pack_buf = None
+
+    def _pack(self, frames, channels):
+        """Copies frames of different sizes into the context's page-locked buffer (registered once, grown when too small: every
+        call that reads it has returned before the next one writes it) -> (buffer, table)."""
+        table, nbytes = frame_table([f.shape[:2] for f in frames], channels)
+        if self._pack_buf is None or self._pack_buf.nbytes < nbytes:
+            if self._pack_buf is not None:
+                check(self._L.tsd_host_unregister(ptr(self._pack_buf)))
+                self._pack_buf = None
+            size = nbytes + nbytes // 4 + 4096
+            raw = np.empty(size + 4096, np.uint8)
+            buf = raw[(-raw.ctypes.data) % 4096:][:size]
+            check(self._L.tsd_host_register(ptr(buf), int(buf.nbytes)))
+            self._pack_buf = buf
+        for f, e in zip(frames, table):
+            self._pack_buf[int(e["offset"]):int(e["offset"]) + f.nbytes] = f.reshape(-1)
+        return self._pack_buf, table
+
+    def _mixed_frames(self, frames, grey):
+        fl = [_u8(f) for f in frames]
+        if any(f.ndim != (2 if grey else 3) or (not grey and f.shape[2] != 3) for f in fl):
+            raise TsdError("a list of frames holds all BGR [H,W,3] or all grey [H,W] frames")
+        return fl
 
     def __del__(self):
         try:
@@ -138,7 +195,18 @@ class Context:
 
     def crop_resize(self, frames, coords, win_frame=None, D=None):
         """K2: cv2.resize(cropImageByCoords(coords, frame), (D, D)) (DET:123-124).  frames uint8 [F,H,W,3], [H,W,3],
-        [F,H,W] or [H,W] (grey, REC:253-254)."""
+        [F,H,W] or [H,W] (grey, REC:253-254), or a list of [H,W,3] (or of [H,W]) frames of different sizes."""
+        if is_mixed(frames):
+            grey = np.ndim(frames[0]) == 2
+            base, table = self._pack(self._mixed_frames(frames, grey), 1 if grey else 3)
+            coords = _i32(coords).reshape(-1, 4)
+            n = len(coords)
+            wf = np.zeros(n, np.int32) if win_frame is None else _i32(win_frame)
+            D = self.D if D is None else int(D)
+            out = np.empty((n, D, D) if grey else (n, D, D, 3), np.uint8)
+            check(self._L.tsd_crop_resize_ragged(self._h, ptr(base), ptr(table), len(table), 1 if grey else 3, ptr(coords), ptr(wf), n, D,
+                                                 ptr(out), MEM_HOST))
+            return out
         frames = np.asarray(frames)
         grey = frames.ndim == 2 or (frames.ndim == 3 and frames.shape[-1] != 3)
         if (frames.ndim == 2) or (frames.ndim == 3 and not grey):
@@ -156,7 +224,18 @@ class Context:
 
     def windows(self, frames, boxes, box_offsets):
         """K1+K2 on whole frames: the candidate loop of MSERTrafficSignDetector (DET:116-124).
+        frames: uint8 [F,H,W,3], [H,W,3] or a list of [H,W,3] frames of different sizes.
         -> (windows uint8[m,D,D,3], coords int32[m,4], win_offsets int32[F+1])."""
+        if is_mixed(frames):
+            base, table = self._pack(self._mixed_frames(frames, False), 3)
+            F = len(table)
+            boxes = _i32(boxes).reshape(-1, 4); box_offsets = _i32(box_offsets)
+            nb = int(box_offsets[-1])
+            wins = np.empty((max(nb, 1), self.D, self.D, 3), np.uint8); coords = np.empty((max(nb, 1), 4), np.int32)
+            woff = np.zeros(F + 1, np.int32); tot = C.c_int32()
+            check(self._L.tsd_windows_ragged(self._h, ptr(base), ptr(table), F, ptr(boxes), ptr(box_offsets), float(self.cfg.enlarge),
+                                             self.D, ptr(wins), ptr(coords), ptr(woff), C.byref(tot), MEM_HOST))
+            return wins[:tot.value].copy(), coords[:tot.value].copy(), woff
         frames = _u8(frames)
         if frames.ndim == 3:
             frames = frames[None]
@@ -274,7 +353,17 @@ class Context:
     # -- whole path ------------------------------------------------------------------------------------------------
     def detect_frames(self, frames, boxes, box_offsets, mode=RUN_DETECT):
         """The whole post-MSER chain on HOST frames (H2D copy inside): DET:116-131 + DET:708-716.
+        frames: uint8 [F,H,W,3], [H,W,3] or a list of [H,W,3] frames of different sizes (packed into the context's page-locked
+        buffer: the chain stages their candidate ROIs from there).
         -> (records structured array DET_DTYPE, counts int32[4] = raw / aspect-passing / survivors / detections)."""
+        if is_mixed(frames):
+            base, table = self._pack(self._mixed_frames(frames, False), 3)
+            boxes = _i32(boxes).reshape(-1, 4); box_offsets = _i32(box_offsets)
+            cap = max(int(box_offsets[-1]), 1)
+            det = np.empty(cap, DET_DTYPE); nd = C.c_int32(); counts = np.zeros(4, np.int32)
+            check(self._L.tsd_detect_frames_ragged(self._h, int(mode), ptr(base), ptr(table), len(table), ptr(boxes), ptr(box_offsets),
+                                                   ptr(det), cap, C.byref(nd), ptr(counts), MEM_HOST))
+            return det[:nd.value].copy(), counts
         frames = _u8(frames)
         if frames.ndim == 3:
             frames = frames[None]
@@ -294,6 +383,13 @@ class Context:
         fs = H * rs if frame_stride is None else int(frame_stride)
         check(self._L.tsd_enqueue_frames(self._h, int(mode), ptr(int(d_frames)), int(nframes), int(H), int(W), rs, fs,
                                          ptr(int(d_boxes)), ptr(int(d_box_offsets)), int(nboxes_total), int(max_boxes_per_frame)))
+
+    def enqueue_frames_ragged(self, d_base, table, d_boxes, d_box_offsets, nboxes_total, mode=RUN_DETECT, max_boxes_per_frame=0):
+        """enqueue_frames on device frames of different sizes: frame f is table[f] = (offset, row_stride, H, W) over the integer
+        device pointer d_base (a FRAME_DESC_DTYPE array or a sequence of 4-tuples; the library copies it before returning)."""
+        table = as_frame_table(table)
+        check(self._L.tsd_enqueue_frames_ragged(self._h, int(mode), ptr(int(d_base)), ptr(table), len(table), ptr(int(d_boxes)),
+                                                ptr(int(d_box_offsets)), int(nboxes_total), int(max_boxes_per_frame)))
 
     def fetch_detections(self, cap, previous=False):
         """Records + stage counts of the last enqueue_frames call; previous=True: of the call before it, while the last batch

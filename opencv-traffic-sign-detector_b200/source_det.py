@@ -74,7 +74,10 @@ def meanMasksFromCrops(crops_per_type):
     off = np.concatenate([[0], np.cumsum([len(t) for t in crops_per_type])]).astype(np.int32)
     Hm, Wm = max(c.shape[0] for c in crops), max(c.shape[1] for c in crops)
     Wm = (Wm + 15) // 16 * 16
-    atlas = np.zeros((len(crops), Hm, Wm, 3), np.uint8)       # one "frame" per crop; the crop is the ROI (0, 0, w, h)
+    # One "frame" per crop; the crop is the ROI (0, 0, w, h).  Context.crop_resize would take the crops as a list of frames of
+    # different sizes, but the atlas stays: the reference's driver test runs this function through an oracle-backed stand-in
+    # of the Context that takes ndarrays only.
+    atlas = np.zeros((len(crops), Hm, Wm, 3), np.uint8)
     coords = np.zeros((len(crops), 4), np.int32)
     for i, c in enumerate(crops):
         atlas[i, :c.shape[0], :c.shape[1]] = c

@@ -83,7 +83,7 @@ def orderCroppedImagesByImageFile(trainImages, trainResults):
     if not files:
         return out
     index = {f: i for i, f in enumerate(files)}
-    grey = np.stack([ctx.bgr2gray(np.asarray(trainImages[f], np.uint8)) for f in files])
+    grey = engine.stack_if_uniform([ctx.bgr2gray(np.asarray(trainImages[f], np.uint8)) for f in files])     # (frames of different sizes: a list)
     coords = np.array([r[1:5] for r in trainResults], np.int32)
     wf = np.array([index[r[0]] for r in trainResults], np.int32)
     wins = ctx.crop_resize(grey, coords, wf)
@@ -124,7 +124,7 @@ def extractMSERDetectionsGray(trainImages, mser, frames_per_call=64):
     out = dict((name, []) for name in names)
     for c0 in range(0, len(names), frames_per_call):
         chunk = names[c0:c0 + frames_per_call]
-        imgs = np.stack([np.asarray(trainImages[n], np.uint8) for n in chunk])
+        imgs = engine.stack_if_uniform([np.asarray(trainImages[n], np.uint8) for n in chunk])
         boxes = [proposals(trainImages[n], mser) for n in chunk]
         off = np.concatenate([[0], np.cumsum([len(b) for b in boxes])]).astype(np.int32)
         allb = np.concatenate(boxes) if off[-1] else np.zeros((0, 4), np.int32)
