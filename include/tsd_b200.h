@@ -187,6 +187,14 @@ TSD_API int tsd_dedup(tsd_ctx *ctx, const uint8_t *windows, const int32_t *coord
 
 /* calculateHistAndNormalize (DET/source.py:575-586): float32 [n][50][60] min-max normalised H-S histograms. */
 TSD_API int tsd_hist(tsd_ctx *ctx, const uint8_t *windows, int n, int D, float *hist, int mem);
+/* The same histograms in the sparse form the duplicate removal works on, all pointers on the device, stream-ordered on
+ * tsd_stream(ctx): windows of D x D BGR pixels window_stride bytes apart (>= 3 D^2; a multiple of 16 with a 16-byte aligned base is
+ * the chain's own padded layout); entries uint32 [n][(D*D + 3) & ~3] = bin << 16 | count in bin order, zero padded; meta [n][48 bytes]
+ * = f64 s1, s11 (sums of the normalised values and their squares), A = s11 - s1^2 / 3000, sqrt(A), f32 a = 1 / max count,
+ * i32 nnz, u32 pixel hash, u32 0; energies float [28][n]: rows 0-24 the group energy bounds, rows 25-27 the entry index where
+ * each 512-bin chunk starts (u16 pairs: chunks 1, 2 / 3, 4 / 5, then nnz). */
+TSD_API int tsd_hist_sparse(tsd_ctx *ctx, const uint8_t *windows, int n, int D, int64_t window_stride, uint32_t *entries,
+                            void *meta, float *energies);
 
 /* Proposal pre-processing (SURVEY section 8(f) N1): grayAndEnhanceContrast (DET/source.py:135-152 = REC/source.py:67-84) for a
  * batch of frames: cv2.cvtColor(BGR2GRAY) -> cv2.createCLAHE(clipLimit, (tiles_x, tiles_y)).apply -> cv2.GaussianBlur((3,3), 0) ->

@@ -88,6 +88,7 @@ _SIGNATURES = {
     "tsd_enqueue_frames_ragged": (_i, [_vp, _i, _vp, _vp, _i, _vp, _vp, _i, _i]),
     "tsd_dedup": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _d, _vp, _vp, _vp, _vp, _i]),
     "tsd_hist": (_i, [_vp, _vp, _i, _i, _vp, _i]),
+    "tsd_hist_sparse": (_i, [_vp, _vp, _i, _i, _i64, _vp, _vp, _vp]),
     "tsd_color_masks": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i]),
     "tsd_bgr2hsv": (_i, [_vp, _vp, _i64, _vp, _i]),
     "tsd_score_masks": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _i]),

@@ -1094,6 +1094,15 @@ int tsd_hist(tsd_ctx* c, const uint8_t* windows, int n, int D, float* hist, int 
     return TSD_OK;
 }
 
+int tsd_hist_sparse(tsd_ctx* c, const uint8_t* windows, int n, int D, int64_t window_stride, uint32_t* entries, void* meta, float* energies) {
+    if (!c || n < 0 || D < 2 || D > kMaxD || window_stride < 3 * D * D || window_stride > (1 << 20) ||
+        (n && (!windows || !entries || !meta || !energies)))
+        return fail(TSD_E_INVALID, "bad argument");
+    CU(cudaSetDevice(c->device));
+    TRY(join_pending(c));
+    return dev_hist(c, windows, nullptr, n, D * D, (int)window_stride, entries, (WinMeta*)meta, energies, n);
+}
+
 int tsd_color_masks(tsd_ctx* c, const uint8_t* windows, int n, int D, uint8_t* red, uint8_t* blue, int mem) {
     if (!c || n < 0 || D < 1 || (n && (!windows || !red || !blue))) return fail(TSD_E_INVALID, "bad argument");
     CU(cudaSetDevice(c->device));

@@ -96,19 +96,28 @@ __device__ __forceinline__ WinMeta load_meta_cg(const WinMeta* p) {      // 3 x 
 
 // =====================================================================================================================
 // Histogram of one window by one warp.  Scratch (per warp, shared memory):
-//   bitmap[96]  occupancy of the 3000 bins; prefix[96] exclusive popcounts -> rank(bin) = perfect hash into cnt[]
-//   binbuf[p]   bin of pixel p;  cnt[r] count of the r-th occupied bin;  binof[r] that bin.
+//   occ[w]    .x occupancy bits of bins 32w .. 32w+31, .y occupied bins before word w -> rank(bin) = perfect hash into cnt[]
+//             (one 64-bit load gives both halves of the rank)
+//   cnt[r]    count of the r-th occupied bin;  binof[r] that bin;  binbuf[p] bin of pixel p
+// The occupancy is first marked as one BYTE per bin with plain stores (no atomics: lanes whose bins share a word do not queue on it)
+// in the space of cnt and binof, dead until pass B, and each lane then packs its 96 bytes into its three bit words.
+// A lane owns groups of four consecutive pixels, g = lane + 32 k.
 // CAP = capacity in pixels (640 for D=25, 1024 for D=32).
 // =====================================================================================================================
 template <int CAP>
 struct __align__(16) HistScratch {
     uint32_t gsum[32];           // sum of count^2 per bin group (exact integers -> deterministic energies)
-    uint32_t bitmap[96];
-    uint32_t cnt[CAP];           // (k5_hist stages the window's pixels here during pass A: cnt is first written after it)
-    uint16_t prefix[96];
-    uint16_t binbuf[CAP];
+    uint2 occ[96];
+    uint32_t cnt[CAP];           // (k5_hist stages the window's pixels here during pass A; the bin marks follow it)
     uint16_t binof[CAP];
+    uint16_t binbuf[CAP];
+    __device__ __forceinline__ uint8_t* mark() { return reinterpret_cast<uint8_t*>(cnt); }     // [96 * 32] over cnt + binof
+    static_assert(sizeof(uint32_t) * CAP + sizeof(uint16_t) * CAP >= 96 * 32, "the bin marks must fit into cnt + binof");
 };
+// The pixels of the last group past npx (npx % 4 != 0) are marked in this bin: bit 31 of occupancy word 95, above the 3000 bins.
+// It is left out of the ranks, so those pixels count into cnt[nnz], past the entries.
+constexpr int kPadBin = 96 * 32 - 1;
+static_assert(kPadBin >= kHistBins, "pad bin");
 
 // calcHist's hue bin floor(H * 50 / 180.0) for H in [0, 180) without a table: (H * 5) / 18 == (H * 18205) >> 16 (checked below for
 // every H; tsd_create checks the same expression against the host-built Tables::hbin and fails loudly if they ever differ)
@@ -139,7 +148,24 @@ __device__ __forceinline__ int hs_bin(int b, int g, int r, const LUT& lut, int l
     return hue_bin(H) * kHistS + ((S * kHistS) >> 8);        // floor(S*60/256.0) exactly (60/256 is a dyadic rational)
 }
 
-__device__ __forceinline__ void mark_bin(uint32_t* bitmap, int bin) { atomicOr(&bitmap[bin >> 5], 1u << (bin & 31)); }
+// Pass A over group g (pixels 4g .. 4g+3), given as the three little-endian words that hold its 12 bytes: bins (pixels past npx ->
+// kPadBin) stored with one 64-bit store, and the pixel hash.
+template <int CAP, class LUT>
+__device__ __forceinline__ void hist_group(uint32_t q0, uint32_t q1, uint32_t q2, int g, int npx, const LUT& lut, HistScratch<CAP>& sw,
+                                           int lane, uint32_t& hsh) {
+    const int p0 = 4 * g;
+    const uint32_t col[4] = {q0 & 0xffffffu, __funnelshift_r(q0, q1, 24) & 0xffffffu, __funnelshift_r(q1, q2, 16) & 0xffffffu, q2 >> 8};
+    uint32_t bins[4];
+#pragma unroll
+    for (int j = 0; j < 4; j++) {
+        int bin = hs_bin((int)(col[j] & 255u), (int)((col[j] >> 8) & 255u), (int)(col[j] >> 16), lut, lane);
+        const uint32_t hv = pix_hash32(p0 + j, col[j]);
+        if (j == 0 || p0 + j < npx) hsh += hv;               // (p0 < npx for every group a lane processes)
+        else bin = kPadBin;
+        bins[j] = (uint32_t)bin;
+    }
+    *reinterpret_cast<uint2*>(&sw.binbuf[p0]) = make_uint2(bins[0] | (bins[1] << 16), bins[2] | (bins[3] << 16));
+}
 
 // px: window pixels (global; may have been rewritten by this warp -> plain loads), e: entries out (global, es words,
 // zero-padded to a multiple of 4), meta out, Eg: optional group energies (E_T + w, stride e_stride).
@@ -148,82 +174,78 @@ template <int CAP, class LUT>
 __device__ __forceinline__ int hist_build_warp(const uint8_t* px, int npx, const LUT& lut, HistScratch<CAP>& sw,
                                                uint32_t* __restrict__ e, WinMeta* meta, float* Eg, int64_t e_stride, bool gram_aux = false) {
     const int lane = threadIdx.x & 31;
-    for (int i = lane; i < 96; i += 32) sw.bitmap[i] = 0;
     sw.gsum[lane] = 0;
-    __syncwarp();
-    // pass A: bin of every pixel + occupancy bitmap + pixel hash.  The kernel is bound by shared-memory wavefronts: with a 4-byte
-    // aligned window (internal layout) a lane takes FOUR consecutive pixels from three aligned words (3 conflict-free LDS.32
-    // instead of 12 byte loads) and stores their bins with one 64-bit store.
+    // pass A: bin of every pixel + pixel hash.  A 4-byte aligned window (internal layout) is read as three words per group
+    // (conflict-free LDS.32 when staged), the packed public layout byte by byte.  Two groups per lane in flight.
     uint32_t hsh = 0;
-    const bool aligned = (reinterpret_cast<uintptr_t>(px) & 3) == 0 && 4 * ((npx + 3) >> 2) <= CAP;
     const int ngroups = (npx + 3) >> 2;
-    if (aligned) {
+    if ((reinterpret_cast<uintptr_t>(px) & 3) == 0) {
         const uint32_t* pw = reinterpret_cast<const uint32_t*>(px);
-#pragma unroll kHistGroupUnroll
-        for (int g = lane; g < ngroups; g += 32) {
-            const uint32_t q0 = pw[3 * g], q1 = pw[3 * g + 1], q2 = pw[3 * g + 2];
-            const uint32_t col[4] = {q0 & 0xffffffu, (q0 >> 24) | ((q1 & 0xffffu) << 8), (q1 >> 16) | ((q2 & 0xffu) << 16), q2 >> 8};
-            uint32_t bins[4];
-#pragma unroll
-            for (int j = 0; j < 4; j++) {
-                const int p = 4 * g + j;
-                const int bin = hs_bin((int)(col[j] & 255u), (int)((col[j] >> 8) & 255u), (int)(col[j] >> 16), lut, lane);
-                bins[j] = (uint32_t)bin;
-                if (p < npx) {
-                    mark_bin(sw.bitmap, bin);
-                    hsh += pix_hash32(p, col[j]);
-                }
-            }
-            *reinterpret_cast<uint2*>(&sw.binbuf[4 * g]) = make_uint2(bins[0] | (bins[1] << 16), bins[2] | (bins[3] << 16));
-        }
+#pragma unroll 2
+        for (int g = lane; g < ngroups; g += 32) hist_group(pw[3 * g], pw[3 * g + 1], pw[3 * g + 2], g, npx, lut, sw, lane, hsh);
     } else {
-#pragma unroll kHistUnroll
-    for (int p = lane; p < npx; p += 32) {
-        const int b = px[3 * p], g = px[3 * p + 1], r = px[3 * p + 2];
-        const int bin = hs_bin(b, g, r, lut, lane);
-        sw.binbuf[p] = (uint16_t)bin;
-        mark_bin(sw.bitmap, bin);
-        hsh += pix_hash32(p, (uint32_t)(b | (g << 8) | (r << 16)));
+#pragma unroll 2
+        for (int g = lane; g < ngroups; g += 32) {
+            uint32_t q[3] = {0, 0, 0};
+#pragma unroll
+            for (int i = 0; i < 12; i++) if (12 * g + i < 3 * npx) q[i >> 2] |= (uint32_t)px[12 * g + i] << (8 * (i & 3));
+            hist_group(q[0], q[1], q[2], g, npx, lut, sw, lane, hsh);
+        }
     }
+    __syncwarp();                                            // (the pixels, staged in cnt by k5_hist, are dead from here)
+    uint8_t* const mark = sw.mark();
+#pragma unroll
+    for (int i = lane; i < 96 * 32 / 16; i += 32) reinterpret_cast<uint4*>(mark)[i] = make_uint4(0, 0, 0, 0);
+    __syncwarp();
+#pragma unroll 2
+    for (int g = lane; g < ngroups; g += 32) {
+        const uint2 bb = *reinterpret_cast<const uint2*>(&sw.binbuf[4 * g]);
+        mark[bb.x & 0xffffu] = 1; mark[bb.x >> 16] = 1; mark[bb.y & 0xffffu] = 1; mark[bb.y >> 16] = 1;
     }
     __syncwarp();
+    // the lane's 96 marks (bins 96 lane .. 96 lane + 95) -> its three occupancy words: (x * 0x01020408) >> 24 gathers the four 0/1
+    // bytes of x into bits 0..3 (every other partial product falls below bit 24 or past bit 31)
+    uint32_t wd[3] = {0, 0, 0};
+    {
+        const uint4* m4 = reinterpret_cast<const uint4*>(mark) + 6 * lane;
+#pragma unroll
+        for (int k = 0; k < 6; k++) {
+            const uint4 q = m4[k];
+            const uint32_t x[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+            for (int t = 0; t < 4; t++) wd[k >> 1] |= ((x[t] * 0x01020408u) >> 24) << (4 * (4 * (k & 1) + t));
+        }
+    }
+    if (lane == 31) wd[2] &= 0x7fffffffu;                   // the pad bin is no rank
     // per-word exclusive prefix popcounts (lane owns words 3*lane .. 3*lane+2)
-    const uint32_t w0 = sw.bitmap[3 * lane], w1 = sw.bitmap[3 * lane + 1], w2 = sw.bitmap[3 * lane + 2];
-    const int c0 = __popc(w0), c1 = __popc(w1), c2 = __popc(w2);
+    const int c0 = __popc(wd[0]), c1 = __popc(wd[1]), c2 = __popc(wd[2]);
     int incl = c0 + c1 + c2;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) { int y = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += y; }
     const int excl = incl - (c0 + c1 + c2);
     const int nnz = __shfl_sync(0xffffffffu, incl, 31);
-    sw.prefix[3 * lane] = (uint16_t)excl; sw.prefix[3 * lane + 1] = (uint16_t)(excl + c0); sw.prefix[3 * lane + 2] = (uint16_t)(excl + c0 + c1);
+    sw.occ[3 * lane] = make_uint2(wd[0], (uint32_t)excl);
+    sw.occ[3 * lane + 1] = make_uint2(wd[1], (uint32_t)(excl + c0));
+    sw.occ[3 * lane + 2] = make_uint2(wd[2], (uint32_t)(excl + c0 + c1));
     const int nnz4 = (nnz + 3) & ~3;
-    for (int i = lane; i < nnz4; i += 32) sw.cnt[i] = 0;
+    {                                                        // zero cnt[0 .. nnz] (cnt[nnz] takes the pad pixels) in 16-byte stores
+        const int nz4 = (nnz + ((npx & 3) ? 4 : 3)) >> 2;    // <= CAP / 4 (pad pixels: npx % 4 != 0 and nnz <= npx)
+        uint4* c4 = reinterpret_cast<uint4*>(sw.cnt);
+        for (int i = lane; i < nz4; i += 32) c4[i] = make_uint4(0, 0, 0, 0);
+    }
     __syncwarp();
     // pass B: counts through the rank hash; binof[rank] = bin (all writers of a rank store the same value)
-    if (aligned) {
-#pragma unroll kHistGroupUnroll
-        for (int g = lane; g < ngroups; g += 32) {
-            const uint2 bb = *reinterpret_cast<const uint2*>(&sw.binbuf[4 * g]);
+#pragma unroll 2
+    for (int g = lane; g < ngroups; g += 32) {
+        const uint2 bb = *reinterpret_cast<const uint2*>(&sw.binbuf[4 * g]);
 #pragma unroll
-            for (int j = 0; j < 4; j++) {
-                if (4 * g + j < npx) {
-                    const int bin = (int)(((j < 2 ? bb.x : bb.y) >> (16 * (j & 1))) & 0xffffu);
-                    const uint32_t word = sw.bitmap[bin >> 5];
-                    const int r = (int)sw.prefix[bin >> 5] + __popc(word & ((1u << (bin & 31)) - 1));
-                    atomicAdd(&sw.cnt[r], 1u);
-                    sw.binof[r] = (uint16_t)bin;
-                }
-            }
+        for (int j = 0; j < 4; j++) {
+            const int bin = (int)(((j < 2 ? bb.x : bb.y) >> (16 * (j & 1))) & 0xffffu);
+            const uint2 o = sw.occ[bin >> 5];
+            const int r = (int)o.y + __popc(o.x & ((1u << (bin & 31)) - 1));
+            atomicAdd(&sw.cnt[r], 1u);
+            sw.binof[r] = (uint16_t)bin;
         }
-    } else {
-#pragma unroll kHistUnroll
-    for (int p = lane; p < npx; p += 32) {
-        const int bin = sw.binbuf[p];
-        const uint32_t word = sw.bitmap[bin >> 5];
-        const int r = (int)sw.prefix[bin >> 5] + __popc(word & ((1u << (bin & 31)) - 1));
-        atomicAdd(&sw.cnt[r], 1u);
-        sw.binof[r] = (uint16_t)bin;
-    }
     }
     __syncwarp();
     unsigned mx = 0;
@@ -255,8 +277,8 @@ __device__ __forceinline__ int hist_build_warp(const uint8_t* px, int npx, const
         if (lane < kHistGroups) Eg[(int64_t)lane * e_stride] = a * sqrtf((float)sw.gsum[lane]) * 1.00001f;
         else if (gram_aux && lane < kEnergyRows) {           // entry index where chunk c starts = occupied bins before bitmap word c * kGramKC / 32
             const int c1 = 2 * (lane - kHistGroups) + 1, c2 = c1 + 1;
-            const uint32_t p1 = c1 < kGramChunks ? sw.prefix[c1 * (kGramKC / 32)] : (uint32_t)nnz;
-            const uint32_t p2 = c2 < kGramChunks ? sw.prefix[c2 * (kGramKC / 32)] : (uint32_t)nnz;
+            const uint32_t p1 = c1 < kGramChunks ? sw.occ[c1 * (kGramKC / 32)].y : (uint32_t)nnz;
+            const uint32_t p2 = c2 < kGramChunks ? sw.occ[c2 * (kGramKC / 32)].y : (uint32_t)nnz;
             reinterpret_cast<uint32_t*>(Eg)[(int64_t)lane * e_stride] = p1 | (p2 << 16);
         }
     }

@@ -28,9 +28,6 @@
 #ifndef TSD_FOLD_MINB
 #define TSD_FOLD_MINB 1          // min resident CTAs per SM of the warp-per-frame fold (register budget: 1 -> as many as it likes, 128)
 #endif
-#ifndef TSD_HIST_UNROLL
-#define TSD_HIST_UNROLL 8        // pixels per lane in flight in the two histogram passes (measured: 2: .266, 4: .274, 5: .283, 7-8: .259, 10: .310, 20: .369 ms)
-#endif
 
 #ifndef TSD_HIST_MINB
 #define TSD_HIST_MINB 8          // min resident CTAs per SM of k5_hist (register budget: 8 -> 64 registers)
@@ -38,13 +35,9 @@
 #ifndef TSD_K2_MINB
 #define TSD_K2_MINB 12           // min resident CTAs per SM of k2_crop_resize_v2 (12 -> 40 registers)
 #endif
-#ifndef TSD_HIST_GROUP_UNROLL
-#define TSD_HIST_GROUP_UNROLL 2  // groups of 4 pixels per lane in flight in the aligned histogram passes (measured at 4096 frames: 1: .922, 2: .921, 3: .934, 4: .953 ms)
-#endif
 
 namespace tsd {
-constexpr int kHistGroupUnroll = TSD_HIST_GROUP_UNROLL;
-constexpr int kK2Unroll = TSD_K2_UNROLL, kHistUnroll = TSD_HIST_UNROLL, kK3Unroll = TSD_K3_UNROLL;     // (#pragma unroll takes a constant expression, not a macro)
+constexpr int kK2Unroll = TSD_K2_UNROLL, kK3Unroll = TSD_K3_UNROLL;     // (#pragma unroll takes a constant expression, not a macro)
 
 constexpr int kHistH = 50, kHistS = 60, kHistBins = kHistH * kHistS;   // DET:578
 constexpr int kMaxD = 32;

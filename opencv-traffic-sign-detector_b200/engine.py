@@ -267,6 +267,10 @@ class Context:
         check(self._L.tsd_hist(self._h, ptr(windows), n, D, ptr(out), MEM_HOST))
         return out
 
+    def hist_sparse(self, windows_ptr, n, D, window_stride, entries_ptr, meta_ptr, energies_ptr):
+        """The sparse histograms of n device-resident windows (device pointers; layouts in tsd_hist_sparse), stream-ordered."""
+        check(self._L.tsd_hist_sparse(self._h, windows_ptr, n, D, window_stride, entries_ptr, meta_ptr, energies_ptr))
+
     def color_masks(self, windows):
         """K3: getColorMaskRedOrBlue(img,'r'), (img,'b') (DET:63-89) -> (red, blue) uint8 [n,D,D]."""
         windows = _u8(windows)
